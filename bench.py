@@ -2,7 +2,7 @@
 """Headline benchmark: SVGP-Gibbs ELBO steps/s at BASELINE.json config 2 (sparse multivariate Gibbs SVGP, synthetic 3-D
 inputs, N = 2^20, M = 1024 inducing points, global minibatch 65536, fp64), rows of each minibatch sharded over the ranks.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--variant full|diag] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--variant full|diag] [--impl reference] [--dump-outputs DIR]
   N > 1:  python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py ...
 
 One step = field interpolation -> K(X_B,Z) -> Kzz Cholesky -> whitened predictive mean/variance -> Gaussian E[log-lik] +
@@ -184,6 +184,21 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
+def dump_outputs(dirname, model, loss):
+    """What a caller of the timed step holds after its last step, one float64 DIR/<name>.npy per array: the loss, every
+    parameter after the Adam update and every gradient of that step (about 17 MB at M = 1024).  The inputs are seeded, so
+    two builds run with the same arguments can be compared array for array.  The kernels accumulate with FP64 atomics and
+    Adam carries the rounding differences into later steps, so even two runs of one build agree to a tolerance, not bit for
+    bit (on a B200 at its 1000 W limit, after 10 + 37 steps: loss to 5e-6 relative)."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    arrays = {"loss": loss.reshape(1)}
+    arrays.update({"param_" + k: v for k, v in model.p.items()})
+    arrays.update({"grad_" + k: v for k, v in model.g.items()})
+    for name, t in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), t.detach().cpu().numpy())
+
+
 def workload_config(args):
     return {"workload": "BASELINE config 2: sparse multivariate Gibbs SVGP, synthetic 3-D inputs, N=2^20, M=1024, "
                         "global minibatch 65536, fp64" + ("" if args.variant == "full" else " [diagonal-Gibbs variant]"),
@@ -283,6 +298,8 @@ def run_ours(args):
     launches = lib().npgp_launch_count() - l0 + launches_per_replay * args.steps
     clocks = sampler.stop() if rank == 0 else None
     final_loss = loss.item()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, model, loss)
 
     # ---- end to end: minibatch from pinned host memory every step, loss read back every step
     xp, yp = x_h.pin_memory(), y_h.pin_memory()
@@ -555,7 +572,13 @@ def main():
     ap.add_argument("--ref-rows", type=int, default=16384, help="minibatch rows the CPU reference processes per step")
     ap.add_argument("--legs", default="c5,c4,c3", help="extra legs reported under \"configs\" (comma list of c5,c4,c3; none)")
     ap.add_argument("--legs-timeout", type=int, default=240, help="seconds after which the legs are abandoned")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the loss, parameters and gradients of the last one to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU step computed; --impl reference has no such step")
     if args.impl == "reference":
         run_reference(args)
     else:
