@@ -251,9 +251,11 @@ int npgp_gibbs_full_fwd_digits(int d, int n1, int n2, const double* x1, const do
                                double jitter, const double* scale, void* digits, const double* u, double* Ku_part,
                                long ku_stride, npgp_stream_t stream);
 /* T = K C from planes.  a_expo NULL: matrix-wide exponent from *a_scale.  Kmat (optional): FP64 K for the row dot, else K is
- * rebuilt from the planes.  q (optional): q_stride == 0 -> q[i] += rowdot (atomics); q_stride >= n -> q[cb * q_stride + i] =
- * partial of column block cb (M / 64 blocks; deterministic).  gvec / du_part (optional): du_part[rb * M + j] = sum over the
- * rows of row block rb (128 rows) of gvec_i K_ij -- K^T g_mu of the ELBO backward from the K tiles the kernel holds anyway. */
+ * rebuilt from the planes.  T may be NULL when q is given: only the row dot is formed (bitwise the q of the same call with T),
+ * T is not stored; T and q both NULL is NPGP_EINVAL.  q (optional): q_stride == 0 -> q[i] += rowdot (atomics);
+ * q_stride >= n -> q[cb * q_stride + i] = partial of column block cb (M / 64 blocks; deterministic).  gvec / du_part
+ * (optional): du_part[rb * M + j] = sum over the rows of row block rb (128 rows) of gvec_i K_ij -- K^T g_mu of the ELBO
+ * backward from the K tiles the kernel holds anyway. */
 int npgp_o8_rowquad_digits(int n, int M, const void* a_digits, const int* a_expo, const double* a_scale,
                            const void* c_digits, const int* c_expo, const double* Kmat, long ldk, double* T, long ldt,
                            double* q, long q_stride, const double* gvec, double* du_part, npgp_stream_t stream);
@@ -325,6 +327,27 @@ int npgp_svgp_elbo_bwd(npgp_svgp_plan* plan, const double* x, const double* thet
 int npgp_svgp_step(npgp_svgp_plan* plan, const double* x, const double* y, double* theta, double* grad, double* adam_m,
                    double* adam_v, const double* mask, double* step_dev, int* status, double lr, double beta1, double beta2,
                    double eps, void* comm, npgp_stream_t stream);
+/* Posterior prediction with a fitted theta (SVGPGibbs.predict semantics, the reference's model.predict through GPyTorch's
+ * whitened VariationalStrategy).  Both calls reuse the plan's workspace (no allocation) and are capturable.
+ * prepare: Z-side factors of the posterior for this theta: Kzz -> Cholesky + inverse, u = P^T m, C = P^T (Ls Ls^T - I) P and
+ * its digit planes, the field's prior-kernel factorisations and interpolation weights (alpha / W).  status (optional,
+ * sticky): bit 0 on a failed factorisation, as in npgp_svgp_elbo_fwd.  Invalidates the saved forward (npgp_svgp_elbo_bwd then
+ * returns NPGP_EINVAL until the next npgp_svgp_elbo_fwd). */
+int npgp_svgp_predict_prepare(npgp_svgp_plan* plan, const double* theta, int* status, npgp_stream_t stream);
+/* Posterior marginals at n rows xs (n,d), in chunks of B_local rows, with the theta of the last prepare on this plan (theta:
+ * the same buffer, read for Z and D):
+ *   mean (n), var_f (n) = max(s + jitter_xx + k^T C k, min_var)                 required
+ *   var_y (n) = var_f + noise, noise = 1e-4 + softplus(raw_noise)               optional (NULL)
+ *   field: variant 0 (d,n) dim-major ell(x) = exp(c + K^p alpha); variant 1 (n, d(d+1)/2) Sigma(x) packed as
+ *          npgp_sigma_from_h_fwd                                                optional
+ *   lpd (n) = log N(y_i | mean_i, var_y_i)                                      optional, needs ys
+ *   sums (3), ACCUMULATED: += [sum (y-mean)^2, sum -lpd, n]                     optional, needs ys
+ * Every reduction of this call has a fixed order: bitwise reproducible for a fixed plan, n and prepared factors (prepare, like
+ * the step's forward, splits its M x M products over K with FP64 atomics from M = 512 on).  Rows may be sharded across ranks
+ * with no collective; one npgp_allreduce_f64 of the 3 sums gives the global RMSE / NLPD.  NPGP_EINVAL without a prepare since the
+ * last fwd / step / set_extra_jitter on this plan.  Invalidates the saved forward like prepare. */
+int npgp_svgp_predict(npgp_svgp_plan* plan, long n, const double* xs, const double* ys, const double* theta, double* mean,
+                      double* var_f, double* var_y, double* field, double* lpd, double* sums, npgp_stream_t stream);
 /* device pointers into the workspace (inspection): 0 mu (B), 1 T (B,M), 2 P (M,M), 3 C (M,M), 4 u (M), 5 g_mu (B), 6 g_v (B),
  * 7 acc4, 8 info (ints: Kzz, then the prior-kernel factorisations) */
 const void* npgp_svgp_buffer(npgp_svgp_plan* plan, int which);

@@ -104,6 +104,8 @@ _SIGS = {
     "npgp_svgp_elbo_fwd": ([_p, _p, _p, _p, _p, _p, _p], _i),
     "npgp_svgp_elbo_bwd": ([_p, _p, _p, _p, _p], _i),
     "npgp_svgp_step": ([_p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _d, _d, _d, _d, _p, _p], _i),
+    "npgp_svgp_predict_prepare": ([_p, _p, _p, _p], _i),
+    "npgp_svgp_predict": ([_p, _l, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p], _i),
     "npgp_svgp_buffer": ([_p, _i], _p),
     "npgp_comm_unique_id": ([_p], _i),
     "npgp_comm_create": ([_p, _p, _i, _i], _i),

@@ -271,8 +271,9 @@ __device__ __forceinline__ double o8_scale_or_nan(int e, int shift) {
 //   Bs / eb: digit planes of the symmetric C (BR = 64) and its per-row (= per-column) exponents.
 //   Kmat:    optional FP64 K for the row dot / column sums; NULL: K is rebuilt from the A digits.
 //   q:       q_stride == 0: q[row] += (atomics);  q_stride > 0: q[cb * q_stride + row] = partial (deterministic)
+//   WT:      false: T is not stored (T unused, q required); the row dot is formed from the same products in the same order
 // ---------------------------------------------------------------------------------------------------------------------
-template <bool COLL>
+template <bool COLL, bool WT>
 __global__ void __launch_bounds__(O8_RQ_THREADS, 1)
 o8_rowquad_kernel(int n, int N, int Kd, const int8_t* __restrict__ As, const int* __restrict__ ea,
                   const double* __restrict__ a_scale, const int8_t* __restrict__ Bs, const int* __restrict__ eb,
@@ -454,11 +455,11 @@ o8_rowquad_kernel(int n, int N, int Kd, const int8_t* __restrict__ As, const int
       const double* sc = scol + half * HC;
       double qsum = 0.0;
       if (row < n) {
-        double* tp = T + (long)row * ldt + cb * O8_BN + half * HC;
+        double* tp = WT ? T + (long)row * ldt + cb * O8_BN + half * HC : nullptr;
 #pragma unroll
         for (int j = 0; j < HC; j += 2) {
           const double o0 = val[j] * rs * sc[j], o1 = val[j + 1] * rs * sc[j + 1];
-          *reinterpret_cast<double2*>(tp + j) = make_double2(o0, o1);
+          if (WT) *reinterpret_cast<double2*>(tp + j) = make_double2(o0, o1);
           if (q) {
             const double2 kk = *reinterpret_cast<const double2*>(krow + j);
             qsum = fma(o0, kk.x, qsum);
@@ -903,35 +904,44 @@ extern "C" int npgp_o8_slice_rows(int R, int Kd, const double* X, long ldx, int 
 //   a_digits / a_expo: A operand (n x M); a_expo NULL -> one matrix-wide exponent from the positive device scalar *a_scale
 //   c_digits / c_expo: symmetric C (M x M, block_rows 64)
 //   Kmat (optional): FP64 K for the row dot; NULL -> rebuilt from the digits
+//   T (optional when q is given): NULL -> only the row dot is formed (bitwise the q of a run with T), no T stores
 //   q (optional): q_stride == 0 -> q[i] += (atomics; zeroed by the caller); q_stride >= n -> q[cb * q_stride + i] = partial of
 //                 column block cb (M / 64 blocks, plain stores: deterministic)
 //   gvec / du_part (optional, both or none): du_part[rb * M + j] = sum over the rows of row block rb of gvec_i K_ij
+template <bool COLL, bool WT>
+static int o8_rowquad_launch(int grid, int n, int M, const void* a_digits, const int* a_expo, const double* a_scale,
+                             const void* c_digits, const int* c_expo, const double* Kmat, long ldk, double* T, long ldt,
+                             double* q, long q_stride, const double* gvec, double* du_part, cudaStream_t stream) {
+  NPGP_CUDA(cudaFuncSetAttribute(o8_rowquad_kernel<COLL, WT>, cudaFuncAttributeMaxDynamicSharedMemorySize, O8_RQ_SMEM));
+  o8_rowquad_kernel<COLL, WT><<<grid, O8_RQ_THREADS, O8_RQ_SMEM, stream>>>(n, M, M, (const int8_t*)a_digits, a_expo, a_scale,
+                                                                         (const int8_t*)c_digits, c_expo, Kmat, ldk, T, ldt, q,
+                                                                         q_stride, gvec, du_part, g_o8_dbg);
+  NPGP_LAUNCH_CHECK();
+  return NPGP_OK;
+}
+
 extern "C" int npgp_o8_rowquad_digits(int n, int M, const void* a_digits, const int* a_expo, const double* a_scale,
                                       const void* c_digits, const int* c_expo, const double* Kmat, long ldk, double* T,
                                       long ldt, double* q, long q_stride, const double* gvec, double* du_part,
                                       cudaStream_t stream) {
   if (n < 0 || M < 0) return NPGP_EINVAL;
   if (n == 0 || M == 0) return NPGP_OK;
-  if (!a_digits || (!a_expo && !a_scale) || !c_digits || !c_expo || !T) return NPGP_EINVAL;
+  if (!a_digits || (!a_expo && !a_scale) || !c_digits || !c_expo || (!T && !q)) return NPGP_EINVAL;
   if ((gvec == nullptr) != (du_part == nullptr)) return NPGP_EINVAL;
-  if (M % O8_BN || M > O8_MAX_KD || (ldt & 1) || (reinterpret_cast<uintptr_t>(T) & 15) ||
+  if (M % O8_BN || M > O8_MAX_KD || (T && ((ldt & 1) || (reinterpret_cast<uintptr_t>(T) & 15))) ||
       (Kmat && ((ldk & 1) || (reinterpret_cast<uintptr_t>(Kmat) & 15))) || (q_stride != 0 && q_stride < n))
     return NPGP_EUNSUPPORTED;
-  NPGP_CUDA(cudaFuncSetAttribute(o8_rowquad_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, O8_RQ_SMEM));
-  NPGP_CUDA(cudaFuncSetAttribute(o8_rowquad_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, O8_RQ_SMEM));
   const long npad = ((long)n + O8_BM - 1) / O8_BM * O8_BM;
   const int tiles = (int)(npad / O8_BM) * (M / O8_BN);
   const int grid = tiles < kNumSMs ? tiles : kNumSMs;
-  if (g_o8_collector)
-    o8_rowquad_kernel<true><<<grid, O8_RQ_THREADS, O8_RQ_SMEM, stream>>>(n, M, M, (const int8_t*)a_digits, a_expo, a_scale,
-                                                                     (const int8_t*)c_digits, c_expo, Kmat, ldk, T, ldt, q,
-                                                                     q_stride, gvec, du_part, g_o8_dbg);
-  else
-    o8_rowquad_kernel<false><<<grid, O8_RQ_THREADS, O8_RQ_SMEM, stream>>>(n, M, M, (const int8_t*)a_digits, a_expo, a_scale,
-                                                                      (const int8_t*)c_digits, c_expo, Kmat, ldk, T, ldt, q,
-                                                                      q_stride, gvec, du_part, g_o8_dbg);
-  NPGP_LAUNCH_CHECK();
-  return NPGP_OK;
+#define NPGP_RQ(COLL, WT) \
+  o8_rowquad_launch<COLL, WT>(grid, n, M, a_digits, a_expo, a_scale, c_digits, c_expo, Kmat, ldk, T, ldt, q, q_stride, gvec, \
+                              du_part, stream)
+  int rc;
+  if (T) rc = g_o8_collector ? NPGP_RQ(true, true) : NPGP_RQ(false, true);
+  else rc = g_o8_collector ? NPGP_RQ(true, false) : NPGP_RQ(false, false);
+#undef NPGP_RQ
+  return rc;
 }
 
 // out[j] = sum_b part[b * N + j], b in index order (e.g. du from the du_part of npgp_o8_rowquad_digits, nb = ceil(n / 128))

@@ -216,6 +216,58 @@ __global__ void svgp_diag_prior_vec_kernel(int M, double pw, const double* __res
   }
 }
 
+// Posterior marginals of one chunk of n rows (scal = [s, noise, ...]).  mean_i = sum_s mu_part[s n + i] and q_i = sum_c
+// q_part[c n + i], both added in index order as in the step; var_f = max(s + jitter_xx + q, min_var), var_y = var_f + noise.
+// With y: lpd_i = log N(y_i | mean_i, var_y_i) and per-block partials blk[b] = sum (y - mean)^2, blk[nblk + b] = sum -lpd.
+// var_y, lpd may be NULL.
+__global__ void __launch_bounds__(256) svgp_predict_finish_kernel(int n, const double* __restrict__ mu_part, int nsplit,
+                                                                  const double* __restrict__ q_part, int nq,
+                                                                  const double* __restrict__ scal, double jitter_xx,
+                                                                  double min_var, const double* __restrict__ y,
+                                                                  double* __restrict__ mean, double* __restrict__ var_f,
+                                                                  double* __restrict__ var_y, double* __restrict__ lpd,
+                                                                  double* __restrict__ blk) {
+  __shared__ double red[32];
+  const int i = blockIdx.x * 256 + threadIdx.x;
+  double r2 = 0.0, nl = 0.0;
+  if (i < n) {
+    double mu = 0.0, q = 0.0;
+    for (int k = 0; k < nsplit; ++k) mu += mu_part[(long)k * n + i];
+    for (int k = 0; k < nq; ++k) q += q_part[(long)k * n + i];
+    double v = scal[0] + jitter_xx + q;
+    if (v < min_var) v = min_var;
+    const double vy = v + scal[1];
+    mean[i] = mu;
+    var_f[i] = v;
+    if (var_y) var_y[i] = vy;
+    if (y) {
+      const double r = y[i] - mu;
+      const double l = -0.5 * (kLog2Pi + log(vy) + r * r / vy);
+      if (lpd) lpd[i] = l;
+      r2 = r * r;
+      nl = -l;
+    }
+  }
+  if (!y) return;  // the same for every thread: no thread leaves a barrier of block_sum that others reach
+  double t = block_sum(r2, red);
+  if (threadIdx.x == 0) blk[blockIdx.x] = t;
+  t = block_sum(nl, red);
+  if (threadIdx.x == 0) blk[gridDim.x + blockIdx.x] = t;
+}
+
+// sums += [sum_b blk[b], sum_b blk[nblk + b], n]: one CTA, fixed assignment and tree (bitwise reproducible)
+__global__ void __launch_bounds__(256) svgp_predict_sums_kernel(int nblk, int n, const double* __restrict__ blk,
+                                                                double* __restrict__ sums) {
+  __shared__ double red[32];
+  for (int k = 0; k < 2; ++k) {
+    double a = 0.0;
+    for (int b = threadIdx.x; b < nblk; b += 256) a += blk[(long)k * nblk + b];
+    const double t = block_sum(a, red);
+    if (threadIdx.x == 0) sums[k] += t;
+  }
+  if (threadIdx.x == 0) sums[2] += (double)n;
+}
+
 }  // namespace npgp
 
 using namespace npgp;
@@ -242,6 +294,7 @@ struct npgp_svgp_plan {
   int8_t *Ad, *Cd;
   int *cexp, *skip_count, *skip_rows, *info, *flags[8];  // flags[0]: Kzz, flags[1 + b]: prior-kernel factorisation b
   long flags_bytes, syrk_part_bytes, gwork_bytes;
+  bool prepared;  // the Z-side factors of npgp_svgp_predict_prepare are in the workspace (cleared by fwd / step / jitter)
 };
 
 namespace {
@@ -446,16 +499,20 @@ extern "C" int npgp_svgp_plan_destroy(npgp_svgp_plan* p) {
 extern "C" int npgp_svgp_set_extra_jitter(npgp_svgp_plan* p, double extra) {
   if (!p || !(extra >= 0.0)) return NPGP_EINVAL;
   p->c.extra_jitter = extra;
+  p->prepared = false;  // the prepared Cholesky used the old jitter
   return NPGP_OK;
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
-// forward: -ELBO share of this rank into grad[n_pad]; leaves everything the backward needs in the workspace
+// Z-side chain (independent of the rows), shared by the forward and npgp_svgp_predict_prepare: scalars, field at Z, the
+// accumulator reset and the KL / prior sums of the loss; on the side streams Kzz -> Cholesky + inverse -> u = P^T m (event
+// ev[10]) -> C = P^T (Ls Ls^T - I) P and its digit planes (event ev[3]); on `st` the prior-kernel factorisations and the
+// interpolation weights of the field (alpha / W).  The side streams are NOT joined here: the forward waits for ev[10] and
+// ev[3] at the points where it needs u and C.
 // ---------------------------------------------------------------------------------------------------------------------
-static int svgp_forward(npgp_svgp_plan* p, const double* x, const double* y, const double* theta, double* grad, int* status,
-                        cudaStream_t st) {
+static int svgp_zside(npgp_svgp_plan* p, const double* theta, int* status, cudaStream_t st) {
   const npgp_svgp_config& c = p->c;
-  const int M = c.M, d = c.d, B = c.B_local, full = c.variant == 1;
+  const int M = c.M, d = c.d, full = c.variant == 1;
   const long MM = (long)M * M;
   const double* Z = theta + p->off_Z;
   const double* F = theta + p->off_F;   // H (M,d) or log_ell_z (d,M)
@@ -463,7 +520,6 @@ static int svgp_forward(npgp_svgp_plan* p, const double* x, const double* y, con
   const double* m = theta + p->off_m;
   const double* Ls = theta + p->off_Ls;
   const double* s = p->scal;
-  const double* noise = p->scal + 1;
   cudaStream_t sd = p->side, sd2 = p->side2;
 
   svgp_scalars_kernel<<<1, 32, 0, st>>>(theta + p->off_os, theta + p->off_noise, p->scal);
@@ -542,13 +598,11 @@ static int svgp_forward(npgp_svgp_plan* p, const double* x, const double* y, con
   NPGP_TRY(stamp(p, 2 * SEC_ZZ + 1, sd));
   NPGP_CUDA(cudaEventRecord(p->ev[3], sd));
 
-  // ---- main stream: interpolation weights and the latent field at the rows (matrix free)
+  // ---- main stream: interpolation weights of the latent field
   if (full) {
     NPGP_TRY(solve_cols(p, p->Pr, F, d, d, p->R4, p->T4, p->W4, st));   // W = (K_row + 1e-5 I)^-1 H
     svgp_pad_cols_kernel<<<ceil_div(M, 256), 256, 0, st>>>(M, d, d, p->W4, p->kp, p->Wp);
     NPGP_LAUNCH_CHECK();
-    NPGP_TRY(npgp_rbf_matvec_fwd(d, 1, d, B, M, x, Z, c.row_lam, c.row_os, p->Wp, nullptr, 0, p->Hx, st));
-    NPGP_TRY(npgp_sigma_from_h_fwd(d, B, p->Hx, Dm, p->fx, st));
   } else {
     for (int b = 0; b < d; ++b) {
       const double* Pb = p->Pr + (long)b * MM;
@@ -561,17 +615,52 @@ static int svgp_forward(npgp_svgp_plan* p, const double* x, const double* y, con
         NPGP_LAUNCH_CHECK();
       }
     }
-    NPGP_TRY(npgp_rbf_matvec_fwd(d, d, 1, B, M, x, Z, c.prior_lam, c.prior_os, p->alpha, c.prior_c, 1, p->ell_x, st));
   }
+  return NPGP_OK;
+}
+
+// The latent field at n rows x (matrix free): fx (n,P) = Sigma(x) (full) or ell_x (d,n) = ell(x) (diag).  Needs svgp_zside.
+static int svgp_row_field(npgp_svgp_plan* p, int n, const double* x, const double* theta, cudaStream_t st) {
+  const npgp_svgp_config& c = p->c;
+  const int M = c.M, d = c.d;
+  const double* Z = theta + p->off_Z;
+  if (c.variant == 1) {
+    NPGP_TRY(npgp_rbf_matvec_fwd(d, 1, d, n, M, x, Z, c.row_lam, c.row_os, p->Wp, nullptr, 0, p->Hx, st));
+    return npgp_sigma_from_h_fwd(d, n, p->Hx, theta + p->off_D, p->fx, st);
+  }
+  return npgp_rbf_matvec_fwd(d, d, 1, n, M, x, Z, c.prior_lam, c.prior_os, p->alpha, c.prior_c, 1, p->ell_x, st);
+}
+
+// K(X,Z) of n rows as digit planes (p->Ad) with the per-split partials of K u (stride ku_stride).  Needs svgp_row_field and u.
+static int svgp_kxz_digits(npgp_svgp_plan* p, int n, const double* x, const double* theta, double* ku_part, long ku_stride,
+                           cudaStream_t st) {
+  const npgp_svgp_config& c = p->c;
+  const double* Z = theta + p->off_Z;
+  if (c.variant == 1)
+    return npgp_gibbs_full_fwd_digits(c.d, n, c.M, x, p->fx, Z, p->fz, c.kernel_jitter, p->scal, p->Ad, p->u, ku_part,
+                                      ku_stride, st);
+  return npgp_gibbs_diag_fwd_digits(c.d, n, c.M, x, p->ell_x, Z, p->fz, p->scal, p->Ad, p->u, ku_part, ku_stride, st);
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// forward: -ELBO share of this rank into grad[n_pad]; leaves everything the backward needs in the workspace
+// ---------------------------------------------------------------------------------------------------------------------
+static int svgp_forward(npgp_svgp_plan* p, const double* x, const double* y, const double* theta, double* grad, int* status,
+                        cudaStream_t st) {
+  const npgp_svgp_config& c = p->c;
+  const int M = c.M, d = c.d, B = c.B_local;
+  const double* s = p->scal;
+  const double* noise = p->scal + 1;
+  p->prepared = false;  // overwrites the Z-side factors, mu_part, q_part and the digit planes
+
+  NPGP_TRY(svgp_zside(p, theta, status, st));
+  NPGP_TRY(svgp_row_field(p, B, x, theta, st));
   NPGP_TRY(stamp(p, 2 * SEC_FIELD + 1, st));
   NPGP_CUDA(cudaStreamWaitEvent(st, p->ev[10], 0));
 
   // ---- data pass: K(X_B,Z) as digit planes (+ partial K u), T = K C with the row dot and K^T g_mu, E[log-lik]
   NPGP_TRY(stamp(p, 2 * SEC_KXZ, st));
-  if (full)
-    NPGP_TRY(npgp_gibbs_full_fwd_digits(d, B, M, x, p->fx, Z, p->fz, c.kernel_jitter, s, p->Ad, p->u, p->mu_part, B, st));
-  else
-    NPGP_TRY(npgp_gibbs_diag_fwd_digits(d, B, M, x, p->ell_x, Z, p->fz, s, p->Ad, p->u, p->mu_part, B, st));
+  NPGP_TRY(svgp_kxz_digits(p, B, x, theta, p->mu_part, B, st));
   NPGP_TRY(npgp_mu_gmu_parts(B, y, p->mu_part, p->nsplit, B, noise, 1.0 / c.B_global, p->mu, p->gmu0, st));
   NPGP_TRY(stamp(p, 2 * SEC_KXZ + 1, st));
   NPGP_CUDA(cudaStreamWaitEvent(st, p->ev[3], 0));  // C and its digit planes (computed under the tile kernel above)
@@ -767,6 +856,58 @@ extern "C" int npgp_svgp_step(npgp_svgp_plan* p, const double* x, const double* 
   NPGP_TRY(npgp_adam_step_guarded(p->n_pad, theta, grad, adam_m, adam_v, mask, lr, beta1, beta2, eps, step_dev, 1.0, status,
                                   stream));
   NPGP_TRY(stamp(p, 2 * SEC_ADAM + 1, stream));
+  return NPGP_OK;
+}
+
+/* Z-side factors of the posterior for theta (the forward's Z-side chain), side streams joined before the return. */
+extern "C" int npgp_svgp_predict_prepare(npgp_svgp_plan* p, const double* theta, int* status, cudaStream_t stream) {
+  if (!p || !theta) return NPGP_EINVAL;
+  p->fwd_done = false;  // the forward's Z-side factors and partial sums are overwritten
+  p->prepared = false;
+  NPGP_TRY(svgp_zside(p, theta, status, stream));
+  NPGP_CUDA(cudaStreamWaitEvent(stream, p->ev[3], 0));  // u, C, its digit planes (the side chain after both side streams)
+  p->prepared = true;
+  return NPGP_OK;
+}
+
+/* Posterior marginals at n rows, streamed through the workspace in chunks of B_local rows (one stream, no allocation). */
+extern "C" int npgp_svgp_predict(npgp_svgp_plan* p, long n, const double* xs, const double* ys, const double* theta, double* mean,
+                                 double* var_f, double* var_y, double* field, double* lpd, double* sums, cudaStream_t stream) {
+  if (!p || n < 0 || !p->prepared) return NPGP_EINVAL;
+  if (n == 0) return NPGP_OK;
+  if (!xs || !theta || !mean || !var_f || ((lpd || sums) && !ys)) return NPGP_EINVAL;
+  const npgp_svgp_config& c = p->c;
+  const int M = c.M, d = c.d, B = c.B_local, nq = M / 64;
+  p->fwd_done = false;  // mu_part, q_part, the digit planes and the row field are overwritten
+  for (long lo = 0; lo < n; lo += B) {
+    const int nc = (int)(n - lo < B ? n - lo : B);
+    const double* x = xs + lo * d;
+    const double* y = ys ? ys + lo : nullptr;
+    NPGP_TRY(svgp_row_field(p, nc, x, theta, stream));
+    if (field) {
+      if (c.variant == 1)
+        NPGP_CUDA(cudaMemcpyAsync(field + lo * p->P6, p->fx, sizeof(double) * nc * p->P6, cudaMemcpyDeviceToDevice, stream));
+      else  // (d, nc) chunk -> columns [lo, lo + nc) of the caller's (d, n)
+        NPGP_CUDA(cudaMemcpy2DAsync(field + lo, sizeof(double) * n, p->ell_x, sizeof(double) * nc, sizeof(double) * nc, d,
+                                    cudaMemcpyDeviceToDevice, stream));
+    }
+    // The K u partials of a chunk take nsplit(nc) x nc doubles, and nsplit is not monotone in the row count: a short last
+    // chunk can need more than mu_part holds.  Then they go to the T buffer (B x M >= (M / 64) x nc), unused by prediction.
+    const int nsplit = npgp_gibbs_digits_splits(nc, M);
+    double* mu_part = (long)nsplit * nc <= (long)p->nsplit * B ? p->mu_part : p->T;
+    NPGP_TRY(svgp_kxz_digits(p, nc, x, theta, mu_part, nc, stream));
+    NPGP_TRY(npgp_o8_rowquad_digits(nc, M, p->Ad, nullptr, p->scal, p->Cd, p->cexp, nullptr, 0, nullptr, M, p->q_part, nc,
+                                    nullptr, nullptr, stream));
+    const int nblk = ceil_div(nc, 256);  // <= the 3 ceil(B / 256) doubles of gwork
+    svgp_predict_finish_kernel<<<nblk, 256, 0, stream>>>(nc, mu_part, nsplit, p->q_part, nq, p->scal, c.jitter_xx, c.min_var, y,
+                                                         mean + lo, var_f + lo, var_y ? var_y + lo : nullptr,
+                                                         lpd ? lpd + lo : nullptr, p->gwork);
+    NPGP_LAUNCH_CHECK();
+    if (sums) {
+      svgp_predict_sums_kernel<<<1, 256, 0, stream>>>(nblk, nc, p->gwork, sums);
+      NPGP_LAUNCH_CHECK();
+    }
+  }
   return NPGP_OK;
 }
 

@@ -311,10 +311,11 @@ def o8_rowquad_digits(n, M, a_digits, a_scale, c_digits, c_expo, T, q_part=None,
                       Kmat=None):
     """T = K C from digit planes; q_part (M/64, n) receives the per-column-block partials of rowdot(T, K); du_part
     (ceil(n/128), M) the per-row-block partials of K^T gvec.  a_scale: device scalar bounding the entries of K (matrix-wide
-    exponent) unless per-row exponents a_expo are given."""
+    exponent) unless per-row exponents a_expo are given.  T = None (with q_part): the row dot only, T is not stored."""
     check(lib().npgp_o8_rowquad_digits(n, M, ptr(a_digits), ptr(a_expo), ptr(a_scale), ptr(c_digits), ptr(c_expo), ptr(Kmat),
-                                       Kmat.stride(0) if Kmat is not None else 0, ptr(T), T.stride(0), ptr(q_part),
-                                       q_part.stride(0) if q_part is not None else 0, ptr(gvec), ptr(du_part), stream()),
+                                       Kmat.stride(0) if Kmat is not None else 0, ptr(T), T.stride(0) if T is not None else M,
+                                       ptr(q_part), q_part.stride(0) if q_part is not None else 0, ptr(gvec), ptr(du_part),
+                                       stream()),
           "npgp_o8_rowquad_digits")
     return T
 

@@ -19,7 +19,7 @@ from __future__ import annotations
 
 import contextlib
 import math
-from typing import Optional
+from typing import NamedTuple, Optional
 
 import torch
 
@@ -34,6 +34,18 @@ def _softplus(x):
 
 def _inv_softplus(v: float) -> float:
     return v + math.log(-math.expm1(-v))
+
+
+class Predictive(NamedTuple):
+    """Posterior marginals of SVGPGibbs.predictive at n rows: var of f, var_y = var + noise; field (field=True): ell(x) (d, n)
+    for 'diag', packed Sigma(x) (n, d(d+1)/2) for 'full'; with y: lpd = log N(y | mean, var_y) (n) and
+    sums = [sum (y - mean)^2, sum -lpd, n] (3), whose all-reduce over ranks gives the global RMSE / NLPD."""
+    mean: torch.Tensor
+    var: torch.Tensor
+    var_y: torch.Tensor
+    field: Optional[torch.Tensor]
+    lpd: Optional[torch.Tensor]
+    sums: Optional[torch.Tensor]
 
 
 class _Section:
@@ -761,3 +773,29 @@ class SVGPGibbs:
             mean[lo:lo + chunk] = mu
             var[lo:lo + chunk] = (s + self.jitter_xx + q).clamp_min(1e-6)
         return mean, var
+
+    @torch.no_grad()
+    def predictive(self, xs, y=None, *, field: bool = False, chunk: int = 65536) -> Predictive:
+        """Posterior marginals at xs through the C ABI (npgp_svgp_predict_prepare + npgp_svgp_predict): one call for the
+        Z-side factors, one for all rows, streamed in chunks of `chunk` rows through the plan of a single-rank C-engine run
+        with that batch size (no allocation per chunk; the row-side reductions have a fixed order).  Works whichever engine
+        trains the model; same arithmetic as predict().  Needs M % 128 == 0 (the digit-plane path)."""
+        if self.M % 128:
+            raise ValueError("the C prediction needs M % 128 == 0 (got %d)" % self.M)
+        from ._lib import check, lib, ptr, stream
+        ent = self._plan(chunk, 1, chunk)
+        xs = xs.contiguous()
+        n = xs.shape[0]
+        f64 = dict(dtype=torch.float64, device=self.dev)
+        mean, var, var_y = (torch.empty(n, **f64) for _ in range(3))
+        fld = lpd = sums = None
+        if field:
+            fld = torch.empty(self.d, n, **f64) if self.variant == "diag" else torch.empty(n, self.d * (self.d + 1) // 2, **f64)
+        if y is not None:
+            y = y.contiguous()
+            lpd, sums = torch.empty(n, **f64), torch.zeros(3, **f64)
+        check(lib().npgp_svgp_predict_prepare(ent["handle"], ptr(self.theta), ptr(self.status), stream()),
+              "npgp_svgp_predict_prepare")
+        check(lib().npgp_svgp_predict(ent["handle"], n, ptr(xs), ptr(y), ptr(self.theta), ptr(mean), ptr(var), ptr(var_y),
+                                      ptr(fld), ptr(lpd), ptr(sums), stream()), "npgp_svgp_predict")
+        return Predictive(mean, var, var_y, fld, lpd, sums)
