@@ -259,6 +259,11 @@ int npgp_gibbs_full_fwd_digits(int d, int n1, int n2, const double* x1, const do
 int npgp_o8_rowquad_digits(int n, int M, const void* a_digits, const int* a_expo, const double* a_scale,
                            const void* c_digits, const int* c_expo, const double* Kmat, long ldk, double* T, long ldt,
                            double* q, long q_stride, const double* gvec, double* du_part, npgp_stream_t stream);
+/* T (n x N) = A B^T from planes, T stored only (no row dot, no column sums): A (n x Kd, block_rows 128; a_expo NULL ->
+ * matrix-wide exponent from *a_scale), B (N x Kd, block_rows 64) with per-row exponents b_expo.  N % 64 == 0, Kd % 32 == 0,
+ * Kd <= 16384, T 16-byte aligned with even ldt >= N.  Same arithmetic and rounding bound as npgp_o8_rowquad_digits. */
+int npgp_o8_gemm_digits(int n, int N, int Kd, const void* a_digits, const int* a_expo, const double* a_scale,
+                        const void* b_digits, const int* b_expo, double* T, long ldt, npgp_stream_t stream);
 int npgp_o8_sum_partials(int nb, int N, const double* part, double* out, npgp_stream_t stream); /* out[j] = sum_b part[b*N+j] */
 /* Out (+)= alpha * w0 * (K^T K - sum_{i in skip} k_i k_i^T) from the ROW-layout planes of K (n x M, matrix-wide scale
  * *x_scale), read MN-major: no transposed copy.  skip_count / skip_rows (optional): rows of weight 0 (clamped variances).
@@ -348,6 +353,33 @@ int npgp_svgp_predict_prepare(npgp_svgp_plan* plan, const double* theta, int* st
  * last fwd / step / set_extra_jitter on this plan.  Invalidates the saved forward like prepare. */
 int npgp_svgp_predict(npgp_svgp_plan* plan, long n, const double* xs, const double* ys, const double* theta, double* mean,
                       double* var_f, double* var_y, double* field, double* lpd, double* sums, npgp_stream_t stream);
+/* Posterior sample fields at any number of rows, correlated across rows, with the factors of the last predict_prepare
+ * (L = chol(Kzz + (jitter_zz + extra) I), P = L^-1, outputscale s).  The draws are the modified predictive process under q(u)
+ * (Finley, Sang, Banerjee & Gelfand, CSDA 2009):
+ *   f_s(x) = mean(x) + k(x)^T W_s + sqrt(r(x)) xi_s(x),   W = P^T Ls E (M x S),   r(x) = max(s + jitter_xx - k^T P^T P k, 0)
+ * with E and xi independent standard normals; noise != 0 draws y instead, with sqrt(r(x) + noise) in place of sqrt(r(x)).
+ * mean(x) is bitwise the mean npgp_svgp_predict returns for the same plan and chunking.  The covariance of the draws is
+ * k^T P^T S P k' + delta_xx' r(x) (S = Ls Ls^T): each marginal equals var_f = s + jitter_xx + k^T C k wherever neither clamp
+ * is active.  The only departure from the exact SVGP posterior k(x,x') + k^T C k' is that the off-diagonal residual
+ * k(x,x') - k^T P^T P k' is set to zero.
+ * Normals: E[j, s] = normal_from_index(seed, (s << 32) + j), xi_s(row) = normal_from_index(seed, 2^63 + (s << 48) + row_offset
+ * + i) (Philox as npgp_dsvi_sample with mu = 0, var = 1): every rank draws the same E, so rows sharded over ranks with their
+ * global row_offset are parts of one joint draw, and draw s does not depend on S.
+ * workspace_bytes: size of `work` (256-byte aligned) for S draws, -1 on a bad cfg or S outside 1 .. 1024; it grows with
+ *   64 ceil(S / 64): G = P^T P and its digit planes, W^T padded to that many rows and its planes, a B_local-row chunk of K W.
+ * prepare: G, W and their planes into work.  NPGP_EINVAL unless npgp_svgp_predict_prepare has run since the last fwd / step /
+ *   set_extra_jitter (theta: that prepare's buffer).
+ * sample: out (S, n), leading dimension ldo >= n, rows xs (n, d) streamed in chunks of B_local through the plan (it overwrites
+ *   what npgp_svgp_predict overwrites; P, C and their planes stay, so npgp_svgp_predict still works).  NPGP_EINVAL unless
+ *   prepare ran on this work since the last fwd / step / set_extra_jitter / predict_prepare.
+ * Both calls run on `stream` only, allocate nothing and are capturable; both invalidate the saved forward like predict.  For a
+ * fixed plan and prepared factors the draws are bitwise reproducible (the prepares split their M x M products over K with FP64
+ * atomics from M = 512 on). */
+long npgp_svgp_sample_workspace_bytes(const npgp_svgp_config* cfg, int S);
+int npgp_svgp_sample_prepare(npgp_svgp_plan* plan, const double* theta, int S, unsigned long long seed, void* work,
+                             long work_bytes, npgp_stream_t stream);
+int npgp_svgp_sample(npgp_svgp_plan* plan, long n, const double* xs, long row_offset, const double* theta, int noise,
+                     double* out, long ldo, void* work, long work_bytes, npgp_stream_t stream);
 /* device pointers into the workspace (inspection): 0 mu (B), 1 T (B,M), 2 P (M,M), 3 C (M,M), 4 u (M), 5 g_mu (B), 6 g_v (B),
  * 7 acc4, 8 info (ints: Kzz, then the prior-kernel factorisations) */
 const void* npgp_svgp_buffer(npgp_svgp_plan* plan, int which);

@@ -57,6 +57,7 @@ _SIGS = {
     "npgp_o8_slice_rows": ([_i, _i, _p, _l, _i, _p, _p, _p], _i),
     "npgp_o8_rowquad_digits": ([_i, _i, _p, _p, _p, _p, _p, _p, _l, _p, _l, _p, _l, _p, _p, _p], _i),
     "npgp_o8_sum_partials": ([_i, _i, _p, _p, _p], _i),
+    "npgp_o8_gemm_digits": ([_i, _i, _i, _p, _p, _p, _p, _p, _p, _l, _p], _i),
     "npgp_o8_syrk_part_bytes": ([_i, _i], _l),
     "npgp_o8_syrk_digits": ([_i, _i, _p, _p, _d, _p, _p, _p, _i, _p, _l, _p, _l, _p], _i),
     "npgp_gibbs_digits_splits": ([_i, _i], _i),
@@ -106,6 +107,9 @@ _SIGS = {
     "npgp_svgp_step": ([_p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _d, _d, _d, _d, _p, _p], _i),
     "npgp_svgp_predict_prepare": ([_p, _p, _p, _p], _i),
     "npgp_svgp_predict": ([_p, _l, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p], _i),
+    "npgp_svgp_sample_workspace_bytes": ([_p, _i], _l),
+    "npgp_svgp_sample_prepare": ([_p, _p, _i, C.c_ulonglong, _p, _l, _p], _i),
+    "npgp_svgp_sample": ([_p, _l, _p, _l, _p, _i, _p, _l, _p, _l, _p], _i),
     "npgp_svgp_buffer": ([_p, _i], _p),
     "npgp_comm_unique_id": ([_p], _i),
     "npgp_comm_create": ([_p, _p, _i, _i], _i),

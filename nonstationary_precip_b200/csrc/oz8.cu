@@ -272,6 +272,8 @@ __device__ __forceinline__ double o8_scale_or_nan(int e, int shift) {
 //   Kmat:    optional FP64 K for the row dot / column sums; NULL: K is rebuilt from the A digits.
 //   q:       q_stride == 0: q[row] += (atomics);  q_stride > 0: q[cb * q_stride + row] = partial (deterministic)
 //   WT:      false: T is not stored (T unused, q required); the row dot is formed from the same products in the same order
+// The row dot and the column sums need N == Kd (they pair T with K); with q and du_part NULL the output width N (B rows) and
+// the contraction length Kd are independent: T = A B^T of npgp_o8_gemm_digits.
 // ---------------------------------------------------------------------------------------------------------------------
 template <bool COLL, bool WT>
 __global__ void __launch_bounds__(O8_RQ_THREADS, 1)
@@ -909,11 +911,14 @@ extern "C" int npgp_o8_slice_rows(int R, int Kd, const double* X, long ldx, int 
 //                 column block cb (M / 64 blocks, plain stores: deterministic)
 //   gvec / du_part (optional, both or none): du_part[rb * M + j] = sum over the rows of row block rb of gvec_i K_ij
 template <bool COLL, bool WT>
-static int o8_rowquad_launch(int grid, int n, int M, const void* a_digits, const int* a_expo, const double* a_scale,
+static int o8_rowquad_launch(int n, int N, int Kd, const void* a_digits, const int* a_expo, const double* a_scale,
                              const void* c_digits, const int* c_expo, const double* Kmat, long ldk, double* T, long ldt,
                              double* q, long q_stride, const double* gvec, double* du_part, cudaStream_t stream) {
+  const long npad = ((long)n + O8_BM - 1) / O8_BM * O8_BM;
+  const long tiles = npad / O8_BM * (N / O8_BN);
+  const int grid = (int)(tiles < kNumSMs ? tiles : kNumSMs);
   NPGP_CUDA(cudaFuncSetAttribute(o8_rowquad_kernel<COLL, WT>, cudaFuncAttributeMaxDynamicSharedMemorySize, O8_RQ_SMEM));
-  o8_rowquad_kernel<COLL, WT><<<grid, O8_RQ_THREADS, O8_RQ_SMEM, stream>>>(n, M, M, (const int8_t*)a_digits, a_expo, a_scale,
+  o8_rowquad_kernel<COLL, WT><<<grid, O8_RQ_THREADS, O8_RQ_SMEM, stream>>>(n, N, Kd, (const int8_t*)a_digits, a_expo, a_scale,
                                                                          (const int8_t*)c_digits, c_expo, Kmat, ldk, T, ldt, q,
                                                                          q_stride, gvec, du_part, g_o8_dbg);
   NPGP_LAUNCH_CHECK();
@@ -931,17 +936,31 @@ extern "C" int npgp_o8_rowquad_digits(int n, int M, const void* a_digits, const 
   if (M % O8_BN || M > O8_MAX_KD || (T && ((ldt & 1) || (reinterpret_cast<uintptr_t>(T) & 15))) ||
       (Kmat && ((ldk & 1) || (reinterpret_cast<uintptr_t>(Kmat) & 15))) || (q_stride != 0 && q_stride < n))
     return NPGP_EUNSUPPORTED;
-  const long npad = ((long)n + O8_BM - 1) / O8_BM * O8_BM;
-  const int tiles = (int)(npad / O8_BM) * (M / O8_BN);
-  const int grid = tiles < kNumSMs ? tiles : kNumSMs;
 #define NPGP_RQ(COLL, WT) \
-  o8_rowquad_launch<COLL, WT>(grid, n, M, a_digits, a_expo, a_scale, c_digits, c_expo, Kmat, ldk, T, ldt, q, q_stride, gvec, \
+  o8_rowquad_launch<COLL, WT>(n, M, M, a_digits, a_expo, a_scale, c_digits, c_expo, Kmat, ldk, T, ldt, q, q_stride, gvec, \
                               du_part, stream)
   int rc;
   if (T) rc = g_o8_collector ? NPGP_RQ(true, true) : NPGP_RQ(false, true);
   else rc = g_o8_collector ? NPGP_RQ(true, false) : NPGP_RQ(false, false);
 #undef NPGP_RQ
   return rc;
+}
+
+// T (n x N) = A B^T from planes: A (n x Kd, block_rows 128; a_expo NULL -> matrix-wide exponent from *a_scale), B (N x Kd,
+// block_rows 64, per-row exponents b_expo = per-column scales of T).  The row-quadratic kernel with T stored and neither the
+// row dot nor the column sums: its output width N and contraction length Kd are independent.
+extern "C" int npgp_o8_gemm_digits(int n, int N, int Kd, const void* a_digits, const int* a_expo, const double* a_scale,
+                                   const void* b_digits, const int* b_expo, double* T, long ldt, cudaStream_t stream) {
+  if (n < 0 || N < 0 || Kd < 0) return NPGP_EINVAL;
+  if (n == 0 || N == 0) return NPGP_OK;
+  if (!a_digits || (!a_expo && !a_scale) || !b_digits || !b_expo || !T) return NPGP_EINVAL;
+  if (N % O8_BN || Kd == 0 || Kd % O8_KS || Kd > O8_MAX_KD || ldt < N || (ldt & 1) || (reinterpret_cast<uintptr_t>(T) & 15))
+    return NPGP_EUNSUPPORTED;
+  if (g_o8_collector)
+    return o8_rowquad_launch<true, true>(n, N, Kd, a_digits, a_expo, a_scale, b_digits, b_expo, nullptr, 0, T, ldt, nullptr,
+                                         0, nullptr, nullptr, stream);
+  return o8_rowquad_launch<false, true>(n, N, Kd, a_digits, a_expo, a_scale, b_digits, b_expo, nullptr, 0, T, ldt, nullptr, 0,
+                                        nullptr, nullptr, stream);
 }
 
 // out[j] = sum_b part[b * N + j], b in index order (e.g. du from the du_part of npgp_o8_rowquad_digits, nb = ceil(n / 128))

@@ -23,6 +23,7 @@
 #include <new>
 
 #include "common.cuh"
+#include "philox.cuh"
 #include "svgp_glue.cuh"
 #include "../../include/npgp.h"
 
@@ -268,6 +269,55 @@ __global__ void __launch_bounds__(256) svgp_predict_sums_kernel(int nblk, int n,
   if (threadIdx.x == 0) sums[2] += (double)n;
 }
 
+
+// Et (Sp x M) = E^T of the sampler: Et[s][j] = E[j, s] = normal_from_index(seed, (s << 32) + j) for s < S, zero rows s >= S
+__global__ void svgp_sample_normals_kernel(int M, int S, int Sp, unsigned long long seed, double* __restrict__ Et) {
+  const long k = (long)blockIdx.x * 256 + threadIdx.x;
+  if (k >= (long)Sp * M) return;
+  const int s = (int)(k / M), j = (int)(k % M);
+  Et[k] = s < S ? normal_from_index(seed, ((unsigned long long)s << 32) + (unsigned long long)j) : 0.0;
+}
+
+// Posterior draws of one chunk of n rows (scal = [s, noise, ...]), CTA = 32 rows x 8 thread rows:
+//   out[s ldo + i] = mean_i + (F[i ldf + s] + sqrt(r_i) xi_s(row0 + i)),  r_i = max(s + jitter_xx - q_i, 0) (+ noise)
+// mean_i and q_i are the partials added in index order (mean as in svgp_predict_finish_kernel); F (n x ldf) = K W is read
+// along s and written along i through a shared-memory tile; xi_s(row) = normal_from_index(seed, 2^63 + (s << 48) + row).
+__global__ void __launch_bounds__(256) svgp_sample_finish_kernel(int n, int S, const double* __restrict__ mu_part, int nsplit,
+                                                                 const double* __restrict__ q_part, int nq,
+                                                                 const double* __restrict__ scal, double jitter_xx, int noise,
+                                                                 const double* __restrict__ F, int ldf, unsigned long long seed,
+                                                                 long row0, double* __restrict__ out, long ldo) {
+  __shared__ double tile[32][33];
+  __shared__ double smean[32], ssd[32];
+  const int tx = threadIdx.x, ty = threadIdx.y, i0 = blockIdx.x * 32, i = i0 + tx;
+  if (ty == 0) {
+    double mu = 0.0, q = 0.0;
+    if (i < n) {
+      for (int k = 0; k < nsplit; ++k) mu += mu_part[(long)k * n + i];
+      for (int k = 0; k < nq; ++k) q += q_part[(long)k * n + i];
+    }
+    double r = scal[0] + jitter_xx - q;
+    if (r < 0.0) r = 0.0;  // (a NaN stays NaN)
+    if (noise) r += scal[1];
+    smean[tx] = mu;
+    ssd[tx] = sqrt(r);
+  }
+  for (int s0 = 0; s0 < S; s0 += 32) {
+    for (int rr = ty; rr < 32; rr += 8) {
+      const int s = s0 + tx;
+      tile[rr][tx] = (i0 + rr < n && s < S) ? F[(long)(i0 + rr) * ldf + s] : 0.0;
+    }
+    __syncthreads();
+    for (int c = ty; c < 32; c += 8) {
+      const int s = s0 + c;
+      if (s < S && i < n) {
+        const double xi = normal_from_index(seed, (1ull << 63) + ((unsigned long long)s << 48) + (unsigned long long)(row0 + i));
+        out[(long)s * ldo + i] = smean[tx] + fma(ssd[tx], xi, tile[tx][c]);
+      }
+    }
+    __syncthreads();
+  }
+}
 }  // namespace npgp
 
 using namespace npgp;
@@ -295,6 +345,12 @@ struct npgp_svgp_plan {
   int *cexp, *skip_count, *skip_rows, *info, *flags[8];  // flags[0]: Kzz, flags[1 + b]: prior-kernel factorisation b
   long flags_bytes, syrk_part_bytes, gwork_bytes;
   bool prepared;  // the Z-side factors of npgp_svgp_predict_prepare are in the workspace (cleared by fwd / step / jitter)
+  // npgp_svgp_sample_prepare has filled sample_work for sample_S draws of sample_seed (cleared by fwd / step / jitter /
+  // predict_prepare)
+  bool sample_ready;
+  int sample_S;
+  unsigned long long sample_seed;
+  void* sample_work;
 };
 
 namespace {
@@ -500,6 +556,7 @@ extern "C" int npgp_svgp_set_extra_jitter(npgp_svgp_plan* p, double extra) {
   if (!p || !(extra >= 0.0)) return NPGP_EINVAL;
   p->c.extra_jitter = extra;
   p->prepared = false;  // the prepared Cholesky used the old jitter
+  p->sample_ready = false;
   return NPGP_OK;
 }
 
@@ -652,6 +709,7 @@ static int svgp_forward(npgp_svgp_plan* p, const double* x, const double* y, con
   const double* s = p->scal;
   const double* noise = p->scal + 1;
   p->prepared = false;  // overwrites the Z-side factors, mu_part, q_part and the digit planes
+  p->sample_ready = false;
 
   NPGP_TRY(svgp_zside(p, theta, status, st));
   NPGP_TRY(svgp_row_field(p, B, x, theta, st));
@@ -864,10 +922,19 @@ extern "C" int npgp_svgp_predict_prepare(npgp_svgp_plan* p, const double* theta,
   if (!p || !theta) return NPGP_EINVAL;
   p->fwd_done = false;  // the forward's Z-side factors and partial sums are overwritten
   p->prepared = false;
+  p->sample_ready = false;  // the sampler's G and W derive from the factors about to be replaced
   NPGP_TRY(svgp_zside(p, theta, status, stream));
   NPGP_CUDA(cudaStreamWaitEvent(stream, p->ev[3], 0));  // u, C, its digit planes (the side chain after both side streams)
   p->prepared = true;
   return NPGP_OK;
+}
+
+// Where the K u partials of an nc-row chunk of prediction or sampling go.  They take nsplit(nc) x nc doubles, and nsplit is not
+// monotone in the row count: a short last chunk can need more than mu_part holds.  Then they go to the T buffer
+// (B x M >= (M / 64) x nc), which neither prediction nor sampling uses.
+static double* svgp_ku_parts(npgp_svgp_plan* p, int nc, int* nsplit) {
+  *nsplit = npgp_gibbs_digits_splits(nc, p->c.M);
+  return (long)*nsplit * nc <= (long)p->nsplit * p->c.B_local ? p->mu_part : p->T;
 }
 
 /* Posterior marginals at n rows, streamed through the workspace in chunks of B_local rows (one stream, no allocation). */
@@ -891,10 +958,8 @@ extern "C" int npgp_svgp_predict(npgp_svgp_plan* p, long n, const double* xs, co
         NPGP_CUDA(cudaMemcpy2DAsync(field + lo, sizeof(double) * n, p->ell_x, sizeof(double) * nc, sizeof(double) * nc, d,
                                     cudaMemcpyDeviceToDevice, stream));
     }
-    // The K u partials of a chunk take nsplit(nc) x nc doubles, and nsplit is not monotone in the row count: a short last
-    // chunk can need more than mu_part holds.  Then they go to the T buffer (B x M >= (M / 64) x nc), unused by prediction.
-    const int nsplit = npgp_gibbs_digits_splits(nc, M);
-    double* mu_part = (long)nsplit * nc <= (long)p->nsplit * B ? p->mu_part : p->T;
+    int nsplit;
+    double* mu_part = svgp_ku_parts(p, nc, &nsplit);
     NPGP_TRY(svgp_kxz_digits(p, nc, x, theta, mu_part, nc, stream));
     NPGP_TRY(npgp_o8_rowquad_digits(nc, M, p->Ad, nullptr, p->scal, p->Cd, p->cexp, nullptr, 0, nullptr, M, p->q_part, nc,
                                     nullptr, nullptr, stream));
@@ -907,6 +972,97 @@ extern "C" int npgp_svgp_predict(npgp_svgp_plan* p, long n, const double* xs, co
       svgp_predict_sums_kernel<<<1, 256, 0, stream>>>(nblk, nc, p->gwork, sums);
       NPGP_LAUNCH_CHECK();
     }
+  }
+  return NPGP_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// posterior sample fields (modified predictive process under q(u)): with the factors of the last predict_prepare,
+//     f_s(x) = mean(x) + k(x)^T W_s + sqrt(r(x)) xi_s(x),  W = P^T Ls E,  r(x) = max(s + jitter_xx - k^T P^T P k, 0)
+// Everything beyond the plan lives in the caller's `work`: G = P^T P and its planes, W^T (Sp = 64 ceil(S / 64) rows; E^T and
+// Y = E^T Ls^T on the way) and its planes, and the B_local x Sp chunk of F = K W.
+// ---------------------------------------------------------------------------------------------------------------------
+struct SampleBufs {
+  double *G, *Y, *Wt, *F;
+  int8_t *Gd, *Wd;
+  int *gexp, *wexp;
+};
+
+static inline int sample_pad(int S) { return (S + 63) / 64 * 64; }
+
+static long sample_layout(const npgp_svgp_config& c, int S, void* work, SampleBufs* b) {
+  const int M = c.M, Sp = sample_pad(S);
+  Carver w{static_cast<char*>(work), 0};
+  b->G = w.take<double>((long)M * M);
+  b->Gd = w.take<int8_t>(npgp_o8_digits_bytes(M, M, 64)), b->gexp = w.take<int>(M);
+  b->Y = w.take<double>((long)Sp * M), b->Wt = w.take<double>((long)Sp * M);
+  b->Wd = w.take<int8_t>(npgp_o8_digits_bytes(Sp, M, 64)), b->wexp = w.take<int>(Sp);
+  b->F = w.take<double>((long)c.B_local * Sp);
+  return w.off + 256;
+}
+
+extern "C" long npgp_svgp_sample_workspace_bytes(const npgp_svgp_config* cfg, int S) {
+  if (!cfg || S < 1 || S > 1024) return -1;
+  npgp_svgp_plan tmp;
+  tmp.c = *cfg;
+  long bytes;
+  if (svgp_layout(&tmp, nullptr, &bytes)) return -1;
+  SampleBufs b;
+  return sample_layout(*cfg, S, nullptr, &b);
+}
+
+/* The row-independent part of S draws: G = P^T P, W = P^T Ls E and their digit planes into work (one stream). */
+extern "C" int npgp_svgp_sample_prepare(npgp_svgp_plan* p, const double* theta, int S, unsigned long long seed, void* work,
+                                        long work_bytes, cudaStream_t st) {
+  if (!p || !theta || !work || S < 1 || S > 1024 || !p->prepared) return NPGP_EINVAL;
+  if (reinterpret_cast<uintptr_t>(work) & 255) return NPGP_EUNSUPPORTED;
+  SampleBufs b;
+  if (work_bytes < sample_layout(p->c, S, work, &b)) return NPGP_EWORKSPACE;
+  const int M = p->c.M, Sp = sample_pad(S);
+  p->fwd_done = false;
+  p->sample_ready = false;
+  // G = P^T P: op(A) = P^T upper, op(B) = P lower; the lower tiles, mirrored
+  NPGP_TRY(npgp_dgemm(1, 0, M, M, M, 1.0, p->P, M, p->P, M, 0.0, b.G, M, 2, 1, 1, st));
+  NPGP_TRY(npgp_symmetrize(M, b.G, M, 0, st));
+  NPGP_TRY(npgp_o8_slice_rows(M, M, b.G, M, 64, b.Gd, b.gexp, st));
+  // W^T = E^T Ls^T P: E^T into Wt, Y = E^T Ls^T (Ls_t lower), then Wt = Y P (P lower)
+  svgp_sample_normals_kernel<<<(unsigned)ceil_div((long)Sp * M, 256), 256, 0, st>>>(M, S, Sp, seed, b.Wt);
+  NPGP_LAUNCH_CHECK();
+  NPGP_TRY(npgp_dgemm(0, 1, Sp, M, M, 1.0, b.Wt, M, p->Ls_t, M, 0.0, b.Y, M, 0, 2, 0, st));
+  NPGP_TRY(npgp_dgemm(0, 0, Sp, M, M, 1.0, b.Y, M, p->P, M, 0.0, b.Wt, M, 0, 1, 0, st));
+  NPGP_TRY(npgp_o8_slice_rows(Sp, M, b.Wt, M, 64, b.Wd, b.wexp, st));
+  p->sample_S = S;
+  p->sample_seed = seed;
+  p->sample_work = work;
+  p->sample_ready = true;
+  return NPGP_OK;
+}
+
+/* S draws at n rows, streamed in chunks of B_local rows: out (S, n), leading dimension ldo. */
+extern "C" int npgp_svgp_sample(npgp_svgp_plan* p, long n, const double* xs, long row_offset, const double* theta, int noise,
+                                double* out, long ldo, void* work, long work_bytes, cudaStream_t st) {
+  if (!p || n < 0 || row_offset < 0 || !p->sample_ready || work != p->sample_work) return NPGP_EINVAL;
+  SampleBufs b;
+  if (work_bytes < sample_layout(p->c, p->sample_S, work, &b)) return NPGP_EWORKSPACE;
+  if (n == 0) return NPGP_OK;
+  if (!xs || !theta || !out || ldo < n || n > (1L << 48) - row_offset) return NPGP_EINVAL;  // row index: 48 key bits
+  const npgp_svgp_config& c = p->c;
+  const int M = c.M, d = c.d, B = c.B_local, nq = M / 64, S = p->sample_S, Sp = sample_pad(S);
+  p->fwd_done = false;  // mu_part, q_part, the digit planes and the row field are overwritten
+  for (long lo = 0; lo < n; lo += B) {
+    const int nc = (int)(n - lo < B ? n - lo : B);
+    const double* x = xs + lo * d;
+    NPGP_TRY(svgp_row_field(p, nc, x, theta, st));
+    int nsplit;
+    double* mu_part = svgp_ku_parts(p, nc, &nsplit);
+    NPGP_TRY(svgp_kxz_digits(p, nc, x, theta, mu_part, nc, st));
+    NPGP_TRY(npgp_o8_rowquad_digits(nc, M, p->Ad, nullptr, p->scal, b.Gd, b.gexp, nullptr, 0, nullptr, M, p->q_part, nc,
+                                    nullptr, nullptr, st));  // k^T G k
+    NPGP_TRY(npgp_o8_gemm_digits(nc, Sp, M, p->Ad, nullptr, p->scal, b.Wd, b.wexp, b.F, Sp, st));  // F = K W
+    svgp_sample_finish_kernel<<<ceil_div(nc, 32), dim3(32, 8), 0, st>>>(nc, S, mu_part, nsplit, p->q_part, nq, p->scal,
+                                                                        c.jitter_xx, noise, b.F, Sp, p->sample_seed,
+                                                                        row_offset + lo, out + lo, ldo);
+    NPGP_LAUNCH_CHECK();
   }
   return NPGP_OK;
 }

@@ -799,3 +799,32 @@ class SVGPGibbs:
         check(lib().npgp_svgp_predict(ent["handle"], n, ptr(xs), ptr(y), ptr(self.theta), ptr(mean), ptr(var), ptr(var_y),
                                       ptr(fld), ptr(lpd), ptr(sums), stream()), "npgp_svgp_predict")
         return Predictive(mean, var, var_y, fld, lpd, sums)
+
+    @torch.no_grad()
+    def sample(self, xs, num_samples: int, *, seed: int = 0, noise: bool = False, row_offset: int = 0,
+               chunk: int = 65536) -> torch.Tensor:
+        """num_samples posterior draws of f (noise=True: of y) at xs, correlated across rows: (num_samples, n).  Goes through
+        the C ABI (npgp_svgp_predict_prepare, npgp_svgp_sample_prepare, npgp_svgp_sample) on the same plan as predictive();
+        the mean of the draws is predictive().mean.  Draw s at global row row_offset + i depends only on seed, s and that row,
+        so rows sharded over ranks with their global offsets are parts of one joint draw.  The draws are the modified
+        predictive process under q(u) (see npgp_svgp_sample in include/npgp.h).  Needs M % 128 == 0 (the digit-plane path)."""
+        if self.M % 128:
+            raise ValueError("the C sampler needs M % 128 == 0 (got %d)" % self.M)
+        from ._lib import check, lib, ptr, stream
+        import ctypes as C
+        ent = self._plan(chunk, 1, chunk)
+        xs = xs.contiguous()
+        n = xs.shape[0]
+        nbytes = lib().npgp_svgp_sample_workspace_bytes(C.byref(ent["cfg"]), int(num_samples))
+        if nbytes < 0:
+            raise ValueError("num_samples must be in 1 .. 1024 (got %d)" % num_samples)
+        work = torch.empty(nbytes + 256, dtype=torch.uint8, device=self.dev)
+        wp = work.data_ptr() + (-work.data_ptr()) % 256
+        out = torch.empty(int(num_samples), n, dtype=torch.float64, device=self.dev)
+        check(lib().npgp_svgp_predict_prepare(ent["handle"], ptr(self.theta), ptr(self.status), stream()),
+              "npgp_svgp_predict_prepare")
+        check(lib().npgp_svgp_sample_prepare(ent["handle"], ptr(self.theta), int(num_samples), int(seed), wp, nbytes, stream()),
+              "npgp_svgp_sample_prepare")
+        check(lib().npgp_svgp_sample(ent["handle"], n, ptr(xs), int(row_offset), ptr(self.theta), int(bool(noise)), ptr(out),
+                                     n, wp, nbytes, stream()), "npgp_svgp_sample")
+        return out
