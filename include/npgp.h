@@ -264,6 +264,15 @@ int npgp_o8_rowquad_digits(int n, int M, const void* a_digits, const int* a_expo
  * Kd <= 16384, T 16-byte aligned with even ldt >= N.  Same arithmetic and rounding bound as npgp_o8_rowquad_digits. */
 int npgp_o8_gemm_digits(int n, int N, int Kd, const void* a_digits, const int* a_expo, const double* a_scale,
                         const void* b_digits, const int* b_expo, double* T, long ldt, npgp_stream_t stream);
+/* Row norms of a triangular contraction from planes: q[cb * q_stride + i] = sum_{j in column block cb} (A B^T)_ij^2, T never
+ * stored.  A (n x Kd, block_rows 128; a_expo NULL -> matrix-wide exponent from *a_scale), B (N x Kd, block_rows 64, per-row
+ * exponents b_expo as npgp_o8_slice_rows writes them) lower triangular: column block cb (64 rows of B) contracts over
+ * k < 64 (cb + 1) only.  Ms > 0 splits B block-diagonally at column Ms: blocks with 64 cb >= Ms also start at k = Ms (the zero
+ * quadrant of blockdiag(P_t, P_s) costs nothing).  The skipped k-steps of B are never read.  Deterministic per-block
+ * partials (plain stores), N / 64 of them per row.  N % 64 == 0, Kd % 32 == 0, 0 < Kd <= 16384, Ms % 64 == 0, Ms == 0 or
+ * Ms < Kd, q_stride >= n; anything else (and NULL operands) is NPGP_EINVAL. */
+int npgp_o8_trinorm_digits(int n, int N, int Kd, int Ms, const void* a_digits, const int* a_expo, const double* a_scale,
+                           const void* b_digits, const int* b_expo, double* q, long q_stride, npgp_stream_t stream);
 int npgp_o8_sum_partials(int nb, int N, const double* part, double* out, npgp_stream_t stream); /* out[j] = sum_b part[b*N+j] */
 /* Out (+)= alpha * w0 * (K^T K - sum_{i in skip} k_i k_i^T) from the ROW-layout planes of K (n x M, matrix-wide scale
  * *x_scale), read MN-major: no transposed copy.  skip_count / skip_rows (optional): rows of weight 0 (clamped variances).
@@ -383,6 +392,26 @@ int npgp_svgp_sample(npgp_svgp_plan* plan, long n, const double* xs, long row_of
 /* device pointers into the workspace (inspection): 0 mu (B), 1 T (B,M), 2 P (M,M), 3 C (M,M), 4 u (M), 5 g_mu (B), 6 g_v (B),
  * 7 acc4, 8 info (ints: Kzz, then the prior-kernel factorisations) */
 const void* npgp_svgp_buffer(npgp_svgp_plan* plan, int which);
+
+/* ---- streamed SGPR posterior (sgpr.py posterior().predictive()): row-side kernels (csrc/sgpr_predict.cu) ---- */
+/* Finishing kernel of one chunk of n rows, one launch.  qn: per-column-block partials of |P k(x)|^2 (row c * qn_stride + i),
+ * the first nb_t blocks of the temporal component (0 for the diagonal model), the next nb_s of the Gibbs one; qv: the nb_v
+ * partials of |V k(x)|^2.  Each component's partials are added in index order.  Device scalars s, noise, os_t (os_t only
+ * with nb_t > 0):
+ *   var_f (n) = [nb_t > 0] max(os_t - q_t, 0) + s max(1 - q_s, 0) + q_v      required
+ *   var_y (n) = var_f + noise                                                 optional
+ *   lpd (n) = log N(y | mean, var_y)                                          optional, needs y and mean
+ *   sums (3), ACCUMULATED: += [sum (y - mean)^2, sum -lpd, n]                 optional, needs y and mean (fixed order)
+ * work: npgp_sgpr_predict_workspace_bytes(n) bytes, zeroed before its first use (the kernel leaves it so); needed with sums.
+ * Same sums contract as npgp_svgp_predict: one all-reduce of 3 doubles gives the global RMSE / NLPD. */
+long npgp_sgpr_predict_workspace_bytes(int n);
+int npgp_sgpr_predict_finish(int n, const double* qn, long qn_stride, int nb_t, int nb_s, const double* qv, long qv_stride,
+                             int nb_v, const double* mean, const double* y, const double* s, const double* noise,
+                             const double* os_t, double* var_f, double* var_y, double* lpd, double* sums, void* work,
+                             long work_bytes, npgp_stream_t stream);
+/* FP64 per-column-block row norms q[cb * q_stride + i] = sum_{j in [64 cb, min(64 cb + 64, W))} G_ij^2 (one warp per row,
+ * fixed order): the partials npgp_o8_trinorm_digits gives, for widths the digit path does not take. */
+int npgp_sgpr_rownorm_parts(int n, int W, const double* G, long ldg, double* q, long q_stride, npgp_stream_t stream);
 
 /* ---- the path's one collective (csrc/comm.cu; SURVEY.md section 8(e)): sum all-reduce of the flat fp64 gradient buffer.
  * NCCL is bound at run time (dlopen), the communicator is an opaque handle.  id128: 128-byte token made on one rank by

@@ -57,6 +57,7 @@ _SIGS = {
     "npgp_o8_slice_rows": ([_i, _i, _p, _l, _i, _p, _p, _p], _i),
     "npgp_o8_rowquad_digits": ([_i, _i, _p, _p, _p, _p, _p, _p, _l, _p, _l, _p, _l, _p, _p, _p], _i),
     "npgp_o8_sum_partials": ([_i, _i, _p, _p, _p], _i),
+    "npgp_o8_trinorm_digits": ([_i, _i, _i, _i, _p, _p, _p, _p, _p, _p, _l, _p], _i),
     "npgp_o8_gemm_digits": ([_i, _i, _i, _p, _p, _p, _p, _p, _p, _l, _p], _i),
     "npgp_o8_syrk_part_bytes": ([_i, _i], _l),
     "npgp_o8_syrk_digits": ([_i, _i, _p, _p, _d, _p, _p, _p, _i, _p, _l, _p, _l, _p], _i),
@@ -111,6 +112,9 @@ _SIGS = {
     "npgp_svgp_sample_prepare": ([_p, _p, _i, C.c_ulonglong, _p, _l, _p], _i),
     "npgp_svgp_sample": ([_p, _l, _p, _l, _p, _i, _p, _l, _p, _l, _p], _i),
     "npgp_svgp_buffer": ([_p, _i], _p),
+    "npgp_sgpr_predict_workspace_bytes": ([_i], _l),
+    "npgp_sgpr_predict_finish": ([_i, _p, _l, _i, _i, _p, _l, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _l, _p], _i),
+    "npgp_sgpr_rownorm_parts": ([_i, _i, _p, _l, _p, _l, _p], _i),
     "npgp_comm_unique_id": ([_p], _i),
     "npgp_comm_create": ([_p, _p, _i, _i], _i),
     "npgp_comm_destroy": ([_p], _i),

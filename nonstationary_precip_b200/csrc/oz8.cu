@@ -263,6 +263,15 @@ __device__ __forceinline__ double o8_scale_or_nan(int e, int shift) {
   return (e == O8_POISON) ? __longlong_as_double(0x7FF8000000000000ll) : o8_pow2(e + shift);
 }
 
+// first k-step of column block cb of a lower-triangular B operand: blocks at or past the split column start there
+__device__ __forceinline__ int o8_tri_klo(int cb, int ms_ks) { return (ms_ks > 0 && 2 * cb >= ms_ks) ? ms_ks : 0; }
+// column block of tile `tile` (row block rb): row-block-major, snake order in the TRI mode
+template <bool TRI>
+__device__ __forceinline__ int o8_rq_cb(int tile, int rb, int n_cb) {
+  if constexpr (TRI) return (rb & 1) ? n_cb - 1 - tile % n_cb : tile % n_cb;
+  else return tile % n_cb;
+}
+
 // ---------------------------------------------------------------------------------------------------------------------
 // T (n x N) = K C,  q += rowdot(T, K),  du_part[rb] = column sums of g_i K_ij over the rows of row block rb.
 // Persistent: grid = #SMs, tiles (rb, cb) in row-block-major order so that CTAs working at the same time share A through L2.
@@ -274,13 +283,18 @@ __device__ __forceinline__ double o8_scale_or_nan(int e, int shift) {
 //   WT:      false: T is not stored (T unused, q required); the row dot is formed from the same products in the same order
 // The row dot and the column sums need N == Kd (they pair T with K); with q and du_part NULL the output width N (B rows) and
 // the contraction length Kd are independent: T = A B^T of npgp_o8_gemm_digits.
+//   TRI:     B is lower triangular (npgp_o8_trinorm_digits): q[cb * q_stride + row] = sum_{j in cb} T_ij^2 (T, K never
+//            formed), column block cb contracts over k-steps [klo(cb), 2 (cb + 1)) only, klo = ms_ks for blocks at or past
+//            the split column (ms_ks k-steps; 0: no split), else 0.  The tiles of a row block run in snake order (cb
+//            descending on odd row blocks) so that the persistent CTAs, which take every gridDim.x-th tile, get even work.
 // ---------------------------------------------------------------------------------------------------------------------
-template <bool COLL, bool WT>
+template <bool COLL, bool WT, bool TRI = false>
 __global__ void __launch_bounds__(O8_RQ_THREADS, 1)
 o8_rowquad_kernel(int n, int N, int Kd, const int8_t* __restrict__ As, const int* __restrict__ ea,
                   const double* __restrict__ a_scale, const int8_t* __restrict__ Bs, const int* __restrict__ eb,
                   const double* __restrict__ Kmat, long ldk, double* __restrict__ T, long ldt, double* __restrict__ q,
-                  long q_stride, const double* __restrict__ gvec, double* __restrict__ du_part, long long* __restrict__ dbg) {
+                  long q_stride, const double* __restrict__ gvec, double* __restrict__ du_part, long long* __restrict__ dbg,
+                  int ms_ks) {
   extern __shared__ __align__(1024) uint8_t o8_sm[];
   uint8_t* sA = o8_sm;
   uint8_t* sB = o8_sm + O8_RQ_STAGES * O8_A_STAGE;
@@ -316,10 +330,11 @@ o8_rowquad_kernel(int n, int N, int Kd, const int8_t* __restrict__ As, const int
     uint32_t phase = 0;
     long long w_empty = 0;
     for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-      const int rb = tile / n_cb, cb = tile % n_cb;
+      const int rb = tile / n_cb, cb = o8_rq_cb<TRI>(tile, rb, n_cb);
       const int8_t* a = As + ((long)rb * O8_NS + lane) * nks * O8_A_PLANE;  // lane = digit
       const int8_t* b = Bs + (long)cb * nks * O8_B_STAGE;
-      for (int ks = 0; ks < nks; ++ks) {
+      const int k_lo = TRI ? o8_tri_klo(cb, ms_ks) : 0, k_hi = TRI ? min(nks, 2 * (cb + 1)) : nks;
+      for (int ks = k_lo; ks < k_hi; ++ks) {
         const long long c0 = dbg ? clock64() : 0;
         o8_mbar_wait(&empty[stage], phase ^ 1);
         if (dbg) w_empty += clock64() - c0;
@@ -347,7 +362,9 @@ o8_rowquad_kernel(int n, int N, int Kd, const int8_t* __restrict__ As, const int
       o8_mbar_wait(&acc_empty, acc_phase ^ 1);  // epilogue has drained the accumulators of the previous tile
       if (dbg) w_acc += clock64() - c0;
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      for (int ks = 0; ks < nks; ++ks) {
+      const int k_lo = TRI ? o8_tri_klo(o8_rq_cb<TRI>(tile, tile / n_cb, n_cb), ms_ks) : 0;
+      const int k_hi = TRI ? min(nks, 2 * (o8_rq_cb<TRI>(tile, tile / n_cb, n_cb) + 1)) : nks;
+      for (int ks = k_lo; ks < k_hi; ++ks) {
         c0 = dbg ? clock64() : 0;
         o8_mbar_wait(&full[stage], phase);
         if (dbg) w_full += clock64() - c0;
@@ -356,7 +373,7 @@ o8_rowquad_kernel(int n, int N, int Kd, const int8_t* __restrict__ As, const int
           // leading byte offset = distance of the two 16-byte halves of the k-step (BR * 16)
           const uint32_t a_lo = ((o8_smem(sA + stage * O8_A_STAGE) >> 4) & 0x3FFFu) | ((uint32_t)(O8_BM * 16 >> 4) << 16);
           const uint32_t b_lo = ((o8_smem(sB + stage * O8_B_STAGE) >> 4) & 0x3FFFu) | ((uint32_t)(O8_BN * 16 >> 4) << 16);
-          o8_issue_kstep<COLL>(tmem, a_lo, kHi, 2 * O8_BM * 16 >> 4, b_lo, kHi, 2 * O8_BN * 16 >> 4, idesc, ks > 0 ? 1u : 0u);
+          o8_issue_kstep<COLL>(tmem, a_lo, kHi, 2 * O8_BM * 16 >> 4, b_lo, kHi, 2 * O8_BN * 16 >> 4, idesc, ks > k_lo ? 1u : 0u);
           o8_commit(&empty[stage]);  // frees the stage when these MMAs have read it
         }
         __syncwarp();
@@ -378,12 +395,12 @@ o8_rowquad_kernel(int n, int N, int Kd, const int8_t* __restrict__ As, const int
     const int quad = warp & 3, half = (warp - 2) >> 2, et = tid - 64;  // et: 0..255
     const int rloc = quad * 32 + lane;                                 // this thread's row inside the tile (= its TMEM lane)
     constexpr int HC = O8_BN / 2;                                      // columns per thread
-    const bool need_k = (q != nullptr) || (du_part != nullptr);
+    const bool need_k = !TRI && ((q != nullptr) || (du_part != nullptr));
     const int e_all = ea ? 0 : o8_exponent_of_scale(*a_scale);
     uint32_t acc_phase = 0;
     long long w_accfull = 0;
     for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-      const int rb = tile / n_cb, cb = tile % n_cb;
+      const int rb = tile / n_cb, cb = o8_rq_cb<TRI>(tile, rb, n_cb);
       const int row = rb * O8_BM + rloc;
       const int er = ea ? ((row < n_rb * O8_BM) ? ea[row] : 0) : e_all;
       // while the MMAs of this tile run: the K tile (row dot, column sums) and the column scales
@@ -462,7 +479,10 @@ o8_rowquad_kernel(int n, int N, int Kd, const int8_t* __restrict__ As, const int
         for (int j = 0; j < HC; j += 2) {
           const double o0 = val[j] * rs * sc[j], o1 = val[j + 1] * rs * sc[j + 1];
           if (WT) *reinterpret_cast<double2*>(tp + j) = make_double2(o0, o1);
-          if (q) {
+          if (TRI) {
+            qsum = fma(o0, o0, qsum);
+            qsum = fma(o1, o1, qsum);
+          } else if (q) {
             const double2 kk = *reinterpret_cast<const double2*>(krow + j);
             qsum = fma(o0, kk.x, qsum);
             qsum = fma(o1, kk.y, qsum);
@@ -910,17 +930,18 @@ extern "C" int npgp_o8_slice_rows(int R, int Kd, const double* X, long ldx, int 
 //   q (optional): q_stride == 0 -> q[i] += (atomics; zeroed by the caller); q_stride >= n -> q[cb * q_stride + i] = partial of
 //                 column block cb (M / 64 blocks, plain stores: deterministic)
 //   gvec / du_part (optional, both or none): du_part[rb * M + j] = sum over the rows of row block rb of gvec_i K_ij
-template <bool COLL, bool WT>
+template <bool COLL, bool WT, bool TRI = false>
 static int o8_rowquad_launch(int n, int N, int Kd, const void* a_digits, const int* a_expo, const double* a_scale,
                              const void* c_digits, const int* c_expo, const double* Kmat, long ldk, double* T, long ldt,
-                             double* q, long q_stride, const double* gvec, double* du_part, cudaStream_t stream) {
+                             double* q, long q_stride, const double* gvec, double* du_part, cudaStream_t stream,
+                             int ms_ks = 0) {
   const long npad = ((long)n + O8_BM - 1) / O8_BM * O8_BM;
   const long tiles = npad / O8_BM * (N / O8_BN);
   const int grid = (int)(tiles < kNumSMs ? tiles : kNumSMs);
-  NPGP_CUDA(cudaFuncSetAttribute(o8_rowquad_kernel<COLL, WT>, cudaFuncAttributeMaxDynamicSharedMemorySize, O8_RQ_SMEM));
-  o8_rowquad_kernel<COLL, WT><<<grid, O8_RQ_THREADS, O8_RQ_SMEM, stream>>>(n, N, Kd, (const int8_t*)a_digits, a_expo, a_scale,
-                                                                         (const int8_t*)c_digits, c_expo, Kmat, ldk, T, ldt, q,
-                                                                         q_stride, gvec, du_part, g_o8_dbg);
+  NPGP_CUDA(cudaFuncSetAttribute(o8_rowquad_kernel<COLL, WT, TRI>, cudaFuncAttributeMaxDynamicSharedMemorySize, O8_RQ_SMEM));
+  o8_rowquad_kernel<COLL, WT, TRI><<<grid, O8_RQ_THREADS, O8_RQ_SMEM, stream>>>(
+      n, N, Kd, (const int8_t*)a_digits, a_expo, a_scale, (const int8_t*)c_digits, c_expo, Kmat, ldk, T, ldt, q, q_stride, gvec,
+      du_part, g_o8_dbg, ms_ks);
   NPGP_LAUNCH_CHECK();
   return NPGP_OK;
 }
@@ -961,6 +982,23 @@ extern "C" int npgp_o8_gemm_digits(int n, int N, int Kd, const void* a_digits, c
                                          0, nullptr, nullptr, stream);
   return o8_rowquad_launch<false, true>(n, N, Kd, a_digits, a_expo, a_scale, b_digits, b_expo, nullptr, 0, T, ldt, nullptr, 0,
                                         nullptr, nullptr, stream);
+}
+
+// q[cb * q_stride + i] = sum_{j in column block cb} (A B^T)_ij^2 from planes, B (N x Kd, block_rows 64, per-row exponents)
+// lower triangular: block cb contracts over k < 64 (cb + 1) only, and from k = Ms on when 64 cb >= Ms (Ms > 0: B is
+// block diagonal with its split at column Ms < Kd).  The skipped k-steps of B are never read.  T is never stored.
+extern "C" int npgp_o8_trinorm_digits(int n, int N, int Kd, int Ms, const void* a_digits, const int* a_expo,
+                                      const double* a_scale, const void* b_digits, const int* b_expo, double* q, long q_stride,
+                                      cudaStream_t stream) {
+  if (n < 0 || N < 0 || Kd <= 0 || !a_digits || (!a_expo && !a_scale) || !b_digits || !b_expo || !q) return NPGP_EINVAL;
+  if (N % O8_BN || Kd % O8_KS || Kd > O8_MAX_KD || Ms < 0 || Ms % O8_BN || (Ms > 0 && Ms >= Kd) || q_stride < n)
+    return NPGP_EINVAL;
+  if (n == 0 || N == 0) return NPGP_OK;
+  if (g_o8_collector)
+    return o8_rowquad_launch<true, false, true>(n, N, Kd, a_digits, a_expo, a_scale, b_digits, b_expo, nullptr, 0, nullptr,
+                                                0, q, q_stride, nullptr, nullptr, stream, Ms / O8_KS);
+  return o8_rowquad_launch<false, false, true>(n, N, Kd, a_digits, a_expo, a_scale, b_digits, b_expo, nullptr, 0, nullptr, 0,
+                                               q, q_stride, nullptr, nullptr, stream, Ms / O8_KS);
 }
 
 // out[j] = sum_b part[b * N + j], b in index order (e.g. du from the du_part of npgp_o8_rowquad_digits, nb = ceil(n / 128))

@@ -115,13 +115,15 @@ def sigma_from_h_bwd(H, Dm, dS, need_dD=True):
     return dH, dD
 
 
-def rbf_matvec_fwd(x, z, lam, os, V, bias=None, apply_exp=False):
+def rbf_matvec_fwd(x, z, lam, os, V, bias=None, apply_exp=False, out=None):
     """out[b,i,c] = f(bias_b + sum_j os_b exp(-0.5|(x_i-z_j)/lam_b|^2) V[b,j,c]);  lam (nb,d), V (nb,m,nv)."""
     x, z, lam, os, V, bias = map(_c, (x, z, lam, os, V, bias))
     n, d = x.shape
     nb, m, nv = V.shape
     assert lam.shape == (nb, d)
-    out = torch.empty(nb, n, nv, dtype=torch.float64, device=x.device)
+    if out is None:
+        out = torch.empty(nb, n, nv, dtype=torch.float64, device=x.device)
+    assert out.shape == (nb, n, nv) and out.is_contiguous()
     check(lib().npgp_rbf_matvec_fwd(d, nb, nv, n, m, ptr(x), ptr(z), ptr(lam), ptr(os), ptr(V), ptr(bias),
                                     int(apply_exp), ptr(out), stream()), "npgp_rbf_matvec_fwd")
     return out
@@ -328,6 +330,41 @@ def o8_sum_partials(part, out=None):
     return out
 
 
+def o8_trinorm_digits(n, N, Kd, a_digits, a_scale, b_digits, b_expo, q_part, Ms=0, a_expo=None):
+    """q_part[cb, i] = sum_{j in column block cb} (A B^T)_ij^2 with B (N x Kd) lower triangular (block diagonal with its split
+    at column Ms when Ms > 0); q_part (N/64, >= n).  a_scale: device scalar bounding A unless per-row exponents a_expo."""
+    check(lib().npgp_o8_trinorm_digits(n, N, Kd, Ms, ptr(a_digits), ptr(a_expo), ptr(a_scale), ptr(b_digits), ptr(b_expo),
+                                       ptr(q_part), q_part.stride(0), stream()), "npgp_o8_trinorm_digits")
+    return q_part
+
+
+def sgpr_rownorm_parts(G, q_part):
+    """q_part[cb, i] = sum_{j in [64 cb, 64 cb + 64)} G_ij^2 (FP64; G may be a column view)."""
+    n, W = G.shape
+    assert G.stride(1) == 1
+    check(lib().npgp_sgpr_rownorm_parts(n, W, ptr(G), G.stride(0), ptr(q_part), q_part.stride(0), stream()),
+          "npgp_sgpr_rownorm_parts")
+    return q_part
+
+
+def sgpr_predict_workspace(n, device):
+    """Zeroed workspace of sgpr_predict_finish for chunks of up to n rows (its ticket must start at 0)."""
+    return torch.zeros(lib().npgp_sgpr_predict_workspace_bytes(n), dtype=torch.uint8, device=device)
+
+
+def sgpr_predict_finish(qn, nb_t, qv, s, noise, var_f, os_t=None, mean=None, y=None, var_y=None, lpd=None, sums=None,
+                        work=None):
+    """Predictive variances (and with y: lpd, accumulated sums) of one chunk from the row-norm partials qn (nb_t temporal
+    blocks, then the Gibbs ones) and qv; see npgp_sgpr_predict_finish."""
+    n = var_f.shape[0]
+    nbn, nbv = qn.shape[0], qv.shape[0]
+    nbytes = work.numel() if work is not None else 0
+    check(lib().npgp_sgpr_predict_finish(n, ptr(qn), qn.stride(0), nb_t, nbn - nb_t, ptr(qv), qv.stride(0), nbv, ptr(mean),
+                                         ptr(y), ptr(s), ptr(noise), ptr(os_t), ptr(var_f), ptr(var_y), ptr(lpd), ptr(sums),
+                                         ptr(work), nbytes, stream()), "npgp_sgpr_predict_finish")
+    return var_f
+
+
 def o8_syrk_part_bytes(n, M):
     return lib().npgp_o8_syrk_part_bytes(n, M)
 
@@ -437,10 +474,11 @@ def colwsum(K, w=None, out=None):
     return out
 
 
-def gemv_n(A, v):
+def gemv_n(A, v, out=None):
     """A @ v (one warp per row)."""
     n, M = A.shape
-    out = torch.empty(n, dtype=torch.float64, device=A.device)
+    if out is None:
+        out = torch.empty(n, dtype=torch.float64, device=A.device)
     check(lib().npgp_gemv_n(n, M, ptr(A), A.stride(0), ptr(_c(v)), ptr(out), stream()), "npgp_gemv_n")
     return out
 

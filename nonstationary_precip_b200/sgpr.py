@@ -98,25 +98,13 @@ class SGPRGibbsStream(torch.nn.Module):
         K = ops.gibbs_diag_fwd(xc, ell_x, self.Z.detach(), ell_z, out=K_out)
         return ell_x, K
 
-    def neg_objective_and_grad(self, x, y, chunk: int = 65536, n_total: Optional[int] = None, all_reduce=None,
-                               world_size: int = 1):
-        """Fills .grad of the parameters with the gradient of MINUS the collapsed SGPR objective (divided by n, as
-        ExactMarginalLogLikelihood does) and returns its value.  `x`, `y`: this rank's rows; `n_total`: global row count;
-        `all_reduce(t)` sums a tensor over ranks (W, c, y^T y after pass 1; the data-side gradients after pass 2).
-
-        Rows are whitened chunk by chunk before they are accumulated, G = K L^-T (the reference's own root,
-        gibbs_kernels.py:225), so that B = I + (s/noise) G^T G has eigenvalues >= 1 and log det Kzz cancels: accumulating
-        the unwhitened Gram matrix K^T K instead (12 instead of 22 M^2 flop per row) was measured to move the objective by
-        4e-5 at N = 4.2e6 when K^T K changed in its last bits -- `Kzz + (s/noise) K^T K` is too ill-conditioned there."""
+    def _pass1(self, x, y, chunk, ell_zd, alphad, Pd, all_reduce):
+        """Pass 1 over this rank's rows: W = G^T G, c = G^T y, y^T y of the whitened root rows G = K P^T, summed over ranks by
+        `all_reduce`.  Also returns the chunk buffers (K, G) for the caller's second pass."""
         dev = x.device
         n_loc = x.shape[0]
-        n = n_total if n_total is not None else n_loc
-        M, D = self.Z.shape
+        M = self.Z.shape[0]
         use_i8 = getattr(self, "use_i8", True)
-        ell_z, alpha, (_, _, P), lp = self._z_side()
-        ell_zd, alphad, Pd = ell_z.detach().contiguous(), alpha.detach().contiguous(), P.detach()
-
-        # ---- pass 1: W = G^T G, c = G^T y, y^T y
         W = torch.zeros(M, M, dtype=torch.float64, device=dev)
         c = torch.zeros(M, dtype=torch.float64, device=dev)
         yy = torch.zeros((), dtype=torch.float64, device=dev)
@@ -135,6 +123,50 @@ class SGPRGibbsStream(torch.nn.Module):
             packed = torch.cat([W.reshape(-1), c, yy.reshape(1)])
             all_reduce(packed)
             W, c, yy = packed[:M * M].reshape(M, M), packed[M * M:M * M + M], packed[-1]
+        return W, c, yy, Kbuf, Gbuf
+
+    @torch.no_grad()
+    def posterior(self, x, y, *, chunk: int = 65536, n_total: Optional[int] = None, all_reduce=None) -> "SGPRPosterior":
+        """The collapsed SGPR posterior at the current parameters, from one pass over this rank's training rows (x, y) --
+        the pass 1 of neg_objective_and_grad, all-reduced the same way.  Returns a snapshot: later parameter updates do not
+        change it.  With B = I + (s/noise) W and P_B = chol(B)^-1, a test row with whitened features g = P k(x) has
+            mean = (s/noise) g^T B^-1 c = k^T u,    var_f = s max(1 - |P k|^2, 0) + |V k|^2,    V = sqrt(s) P_B P,
+        the second term being the reference's eval-time diagonal correction (gibbs_kernels.py:228-232).  `n_total` is
+        accepted for symmetry with neg_objective_and_grad; the posterior does not depend on it."""
+        del n_total
+        ell_z, alpha, (_, _, P), _ = self._z_side()
+        ell_z, alpha, P = ell_z.contiguous(), alpha.contiguous(), P.contiguous()
+        W, c, _, _, _ = self._pass1(x, y, chunk, ell_z, alpha, P, all_reduce)
+        M = self.Z.shape[0]
+        s = _softplus(self.raw_outputscale).reshape(())
+        noise = (1e-4 + _softplus(self.raw_noise)).reshape(())
+        Bm = torch.eye(M, dtype=torch.float64, device=x.device) + (s / noise) * (0.5 * (W + W.T))
+        _, PB = F.psd_safe_chol_inv(Bm)
+        u = F.matmul(P.T, F.matmul(PB.T, F.matmul(PB, c))) * (s / noise)
+        V = ops.dgemm(F._aligned(PB), F._aligned(P), tri_a=1, tri_b=1, out_tri=1, C=torch.zeros_like(P))
+        V *= torch.sqrt(s)
+        return SGPRPosterior(self, "diag", P=P, V=V, u=u, s=s, noise=noise, ell_z=ell_z, alpha=alpha,
+                             use_i8=getattr(self, "use_i8", True))
+
+    def neg_objective_and_grad(self, x, y, chunk: int = 65536, n_total: Optional[int] = None, all_reduce=None,
+                               world_size: int = 1):
+        """Fills .grad of the parameters with the gradient of MINUS the collapsed SGPR objective (divided by n, as
+        ExactMarginalLogLikelihood does) and returns its value.  `x`, `y`: this rank's rows; `n_total`: global row count;
+        `all_reduce(t)` sums a tensor over ranks (W, c, y^T y after pass 1; the data-side gradients after pass 2).
+
+        Rows are whitened chunk by chunk before they are accumulated, G = K L^-T (the reference's own root,
+        gibbs_kernels.py:225), so that B = I + (s/noise) G^T G has eigenvalues >= 1 and log det Kzz cancels: accumulating
+        the unwhitened Gram matrix K^T K instead (12 instead of 22 M^2 flop per row) was measured to move the objective by
+        4e-5 at N = 4.2e6 when K^T K changed in its last bits -- `Kzz + (s/noise) K^T K` is too ill-conditioned there."""
+        dev = x.device
+        n_loc = x.shape[0]
+        n = n_total if n_total is not None else n_loc
+        M, D = self.Z.shape
+        use_i8 = getattr(self, "use_i8", True)
+        ell_z, alpha, (_, _, P), lp = self._z_side()
+        ell_zd, alphad, Pd = ell_z.detach().contiguous(), alpha.detach().contiguous(), P.detach()
+
+        W, c, yy, Kbuf, Gbuf = self._pass1(x, y, chunk, ell_zd, alphad, Pd, all_reduce)
         W = W.clone().requires_grad_(True)
         c = c.clone().requires_grad_(True)
 
@@ -286,25 +318,12 @@ class SGPRSpatioTemporalStream(torch.nn.Module):
         ops.dgemm(Fc[:, :M], Pt, transB=True, tri_b=2, C=Gc[:, :M])
         ops.dgemm(Fc[:, M:], Ps, transB=True, tri_b=2, C=Gc[:, M:])
 
-    def neg_objective_and_grad(self, x, y, chunk: int = 32768, n_total: Optional[int] = None, all_reduce=None):
-        """As SGPRGibbsStream.neg_objective_and_grad, for x (n, 3) = (time, lon, lat).
-
-        Numerics: Kzz of the temporal kernel (M inducing times on a smooth 1-D kernel) is nearly singular, and at
-        N ~ 4e6 rows the unwhitened Gram matrix F^T F / noise has norm ~1e12, so `Kzz + F^T F / noise` cannot be
-        factored in fp64.  Rows are therefore whitened chunk by chunk BEFORE they are accumulated, G = F L^-T, exactly
-        as the reference forms its root; then B = I + D G^T G D / noise has eigenvalues >= 1 and the log-determinants of
-        Kzz cancel analytically.  Cost per row: 22 M^2 flop for both passes instead of 12 M^2."""
+    def _pass1(self, x, y, chunk, zs, zt, hypd, ell_zd, alphad, Ptd, Psd, all_reduce):
+        """Pass 1 over this rank's rows: W = G^T G, c = G^T y, y^T y of the whitened feature rows G = [F_t P_t^T, F_s P_s^T],
+        summed over ranks by `all_reduce`.  Also returns the chunk buffers (F, G) for the caller's second pass."""
         dev = x.device
         n_loc = x.shape[0]
-        n = n_total if n_total is not None else n_loc
-        M = self.Z.shape[0]
-        M2 = 2 * M
-        ell_z, alpha, hyp, zt, (_, _, Ps), (_, _, Pt), lp = self._z_side()
-        ell_zd, alphad, hypd = ell_z.detach().contiguous(), alpha.detach().contiguous(), hyp.detach().contiguous()
-        Ptd, Psd = Pt.detach(), Ps.detach()
-        zs = self.Z.detach()[:, 1:3].contiguous()
-
-        # ---- pass 1: W = G^T G, c = G^T y, y^T y
+        M2 = 2 * self.Z.shape[0]
         W = torch.zeros(M2, M2, dtype=torch.float64, device=dev)
         c = torch.zeros(M2, dtype=torch.float64, device=dev)
         yy = torch.zeros((), dtype=torch.float64, device=dev)
@@ -324,6 +343,57 @@ class SGPRSpatioTemporalStream(torch.nn.Module):
             packed = torch.cat([W.reshape(-1), c, yy.reshape(1)])
             all_reduce(packed)
             W, c, yy = packed[:M2 * M2].reshape(M2, M2), packed[M2 * M2:M2 * M2 + M2], packed[-1]
+        return W, c, yy, Fbuf, Gbuf
+
+    @torch.no_grad()
+    def posterior(self, x, y, *, chunk: int = 32768, n_total: Optional[int] = None, all_reduce=None) -> "SGPRPosterior":
+        """The collapsed posterior of the spatio-temporal model at the current parameters (the literal=False predictive of
+        the reference, spatio_temporal_exp.py's default), from pass 1 of neg_objective_and_grad over this rank's rows,
+        all-reduced the same way.  Returns a snapshot that later parameter updates do not change.  With D = diag(I_M,
+        sqrt(s) I_M), B = I + D W D / noise, P_B = chol(B)^-1, P = blockdiag(P_t, P_s) and features k = [k_t | k_s]:
+            mean = k^T u,  u = P^T D B^-1 D c / noise,
+            var_f = max(os_t - |P_t k_t|^2, 0) + s max(1 - |P_s k_s|^2, 0) + |V k|^2,   V = P_B D P (lower triangular).
+        `n_total` is accepted for symmetry with neg_objective_and_grad; the posterior does not depend on it."""
+        del n_total
+        M = self.Z.shape[0]
+        M2 = 2 * M
+        ell_z, alpha, hyp, zt, (_, _, Ps), (_, _, Pt), _ = self._z_side()
+        ell_z, alpha, hyp = ell_z.contiguous(), alpha.contiguous(), hyp.contiguous()
+        zs = self.Z[:, 1:3].contiguous()
+        W, c, _, _, _ = self._pass1(x, y, chunk, zs, zt, hyp, ell_z, alpha, Pt, Ps, all_reduce)
+        s = _softplus(self.raw_outputscale).reshape(())
+        noise = (1e-4 + _softplus(self.raw_noise)).reshape(())
+        sv = torch.cat([torch.ones(M, dtype=torch.float64, device=x.device), torch.sqrt(s).expand(M)])
+        Bm = torch.eye(M2, dtype=torch.float64, device=x.device) + 0.5 * (W + W.T) * sv[:, None] * sv[None, :] / noise
+        _, PB = F.psd_safe_chol_inv(Bm)
+        w = F.matmul(PB.T, F.matmul(PB, c * sv)) * sv / noise          # D B^-1 D c / noise
+        u = torch.cat([F.matmul(Pt.T, w[:M]), F.matmul(Ps.T, w[M:])])
+        P = torch.zeros(M2, M2, dtype=torch.float64, device=x.device)  # blockdiag(P_t, P_s)
+        P[:M, :M] = Pt
+        P[M:, M:] = Ps
+        V = ops.dgemm(PB, P * sv[:, None], tri_a=1, tri_b=1, out_tri=1, C=torch.zeros_like(P))
+        return SGPRPosterior(self, "st", P=P, V=V, u=u, s=s, noise=noise, ell_z=ell_z, alpha=alpha, hyp=hyp, zt=zt,
+                             use_i8=getattr(self, "use_i8", True))
+
+    def neg_objective_and_grad(self, x, y, chunk: int = 32768, n_total: Optional[int] = None, all_reduce=None):
+        """As SGPRGibbsStream.neg_objective_and_grad, for x (n, 3) = (time, lon, lat).
+
+        Numerics: Kzz of the temporal kernel (M inducing times on a smooth 1-D kernel) is nearly singular, and at
+        N ~ 4e6 rows the unwhitened Gram matrix F^T F / noise has norm ~1e12, so `Kzz + F^T F / noise` cannot be
+        factored in fp64.  Rows are therefore whitened chunk by chunk BEFORE they are accumulated, G = F L^-T, exactly
+        as the reference forms its root; then B = I + D G^T G D / noise has eigenvalues >= 1 and the log-determinants of
+        Kzz cancel analytically.  Cost per row: 22 M^2 flop for both passes instead of 12 M^2."""
+        dev = x.device
+        n_loc = x.shape[0]
+        n = n_total if n_total is not None else n_loc
+        M = self.Z.shape[0]
+        M2 = 2 * M
+        ell_z, alpha, hyp, zt, (_, _, Ps), (_, _, Pt), lp = self._z_side()
+        ell_zd, alphad, hypd = ell_z.detach().contiguous(), alpha.detach().contiguous(), hyp.detach().contiguous()
+        Ptd, Psd = Pt.detach(), Ps.detach()
+        zs = self.Z.detach()[:, 1:3].contiguous()
+
+        W, c, yy, Fbuf, Gbuf = self._pass1(x, y, chunk, zs, zt, hypd, ell_zd, alphad, Ptd, Psd, all_reduce)
         W = W.clone().requires_grad_(True)
         c = c.clone().requires_grad_(True)
 
@@ -397,3 +467,124 @@ class SGPRSpatioTemporalStream(torch.nn.Module):
             if need_dz:
                 self.Z.grad[:, 1:3] += dZs
         return loss.detach()
+
+
+class SGPRPosterior:
+    """Snapshot of a streamed SGPR posterior, returned by SGPRGibbsStream.posterior ("diag") and
+    SGPRSpatioTemporalStream.posterior ("st").  It holds copies of everything the predictive needs (Z, the lengthscale
+    field's interpolation weights, u, and P and V -- as digit planes when the feature width is a multiple of 128), so later
+    optimiser steps on the model do not change its predictions."""
+
+    def __init__(self, model, kind, *, P, V, u, s, noise, ell_z, alpha, use_i8, hyp=None, zt=None):
+        self.kind = kind
+        self.M = model.Z.shape[0]
+        self.width = P.shape[0]  # M (diag) or 2M (st): the feature columns of a test row
+        self.Z = model.Z.detach().clone()
+        self.zs = self.Z[:, 1:3].contiguous() if kind == "st" else self.Z
+        self.prior_c, self.prior_os, self.prior_lam = (b.detach().clone() for b in
+                                                       (model.prior_c, model.prior_os, model.prior_lam))
+        self.ell_z, self.alpha, self.u = ell_z.detach().clone(), alpha.detach().clone(), u.detach().contiguous().clone()
+        self.s, self.noise = s.detach().clone(), noise.detach().clone()
+        self.hyp = hyp.detach().clone() if hyp is not None else None
+        self.zt = zt.detach().clone() if zt is not None else None
+        self.digits = bool(use_i8) and self.width % 128 == 0
+        if self.digits:
+            self.planes = []
+            for Mx in (P, V):  # B operands of npgp_o8_trinorm_digits: block_rows 64, per-row exponents
+                d = torch.empty(ops.digits_bytes(self.width, self.width, 64), dtype=torch.uint8, device=P.device)
+                e = torch.empty(self.width, dtype=torch.int32, device=P.device)
+                ops.o8_slice_rows(Mx.contiguous(), 64, d, e)
+                self.planes.append((d, e))
+            self.one = torch.ones((), dtype=torch.float64, device=P.device)  # bound of the unscaled Gibbs entries
+        else:
+            M = self.M
+            self.V = V.detach().clone()
+            self.Pblocks = [P[:M, :M].contiguous(), P[M:, M:].contiguous()] if kind == "st" else [P.detach().clone()]
+
+    @torch.no_grad()
+    def predictive(self, xs, y=None, *, field: bool = False, chunk: int = 65536):
+        """Posterior marginals at the rows xs (n, D), streamed in chunks of `chunk` rows: svgp.Predictive with mean, var
+        (of f), var_y = var + noise, field (field=True): ell(x) (D, n) on the Gibbs columns, and with y: lpd = log N(y |
+        mean, var_y) and sums = [sum (y - mean)^2, sum -lpd, n].  Buffers are allocated once per call, the chunk loop does
+        not synchronise with the host, and every reduction has a fixed order.  Rows may be sharded over ranks with no
+        collective: one all-reduce of the three sums gives the global RMSE and NLPD."""
+        from .svgp import Predictive
+        xs = xs.contiguous()
+        n = xs.shape[0]
+        dev = xs.device
+        f64 = dict(dtype=torch.float64, device=dev)
+        st = self.kind == "st"
+        M, W = self.M, self.width
+        D = 2 if st else self.Z.shape[1]
+        mean, var, var_y = (torch.empty(n, **f64) for _ in range(3))
+        fld = torch.empty(D, n, **f64) if field else None
+        lpd = sums = None
+        if y is not None:
+            y = y.contiguous()
+            lpd, sums = torch.empty(n, **f64), torch.zeros(3, **f64)
+        if n == 0:
+            return Predictive(mean, var, var_y, fld, lpd, sums)
+        rows = min(chunk, n)
+        cdiv = lambda a, b: (a + b - 1) // b  # noqa: E731
+        nb_t = (M // 64 if self.digits else cdiv(M, 64)) if st else 0
+        nbn = W // 64 if self.digits else (2 if st else 1) * cdiv(M, 64)
+        qn = torch.empty(nbn, rows, **f64)
+        qv = torch.empty(cdiv(W, 64), rows, **f64)
+        work = ops.sgpr_predict_workspace(rows, dev) if y is not None else None
+        ell_buf = torch.empty(D * rows, **f64)
+        if st:
+            xt_all, xs_all = xs[:, 0].contiguous(), xs[:, 1:3].contiguous()
+            Fbuf = torch.empty(rows, W, **f64)
+        if self.digits:
+            Ad = torch.empty(ops.digits_bytes(rows, W, 128), dtype=torch.uint8, device=dev)
+            if st:
+                Ae = torch.empty(cdiv(rows, 128) * 128, dtype=torch.int32, device=dev)
+            else:
+                sizes = {rows, n - (n - 1) // chunk * chunk}
+                ku = torch.empty(max(ops.gibbs_digits_splits(r, M) for r in sizes) * rows, **f64)
+            (Pd, Pe), (Vd, Ve) = self.planes
+        else:
+            Gbuf = torch.empty(rows, W, **f64)
+            if not st:
+                Kbuf = torch.empty(rows, M, **f64)
+        for lo in range(0, n, chunk):
+            nc = min(chunk, n - lo)
+            ell = ell_buf[:D * nc].view(D, nc, 1)
+            xc = xs_all[lo:lo + nc] if st else xs[lo:lo + nc]
+            ops.rbf_matvec_fwd(xc, self.zs, self.prior_lam, self.prior_os, self.alpha.unsqueeze(-1), bias=self.prior_c,
+                               apply_exp=True, out=ell)
+            ell_x = ell.view(D, nc)
+            mc = mean[lo:lo + nc]
+            if st:
+                Fc = Fbuf[:nc]
+                ops.rbfper_fwd(xt_all[lo:lo + nc], self.zt, self.hyp, out=Fc[:, :M])
+                ops.gibbs_diag_fwd(xc, ell_x, self.zs, self.ell_z, out=Fc[:, M:])
+                ops.gemv_n(Fc, self.u, out=mc)
+                if self.digits:
+                    ops.o8_slice_rows(Fc, 128, Ad, Ae)
+                    ops.o8_trinorm_digits(nc, W, W, Ad, None, Pd, Pe, qn, Ms=M, a_expo=Ae)
+                    ops.o8_trinorm_digits(nc, W, W, Ad, None, Vd, Ve, qv, a_expo=Ae)
+                else:
+                    Gc = Gbuf[:nc]
+                    for h, Ph in enumerate(self.Pblocks):
+                        cols = slice(h * M, (h + 1) * M)
+                        ops.dgemm(Fc[:, cols], Ph, transB=True, tri_b=2, C=Gc[:, cols])
+                        ops.sgpr_rownorm_parts(Gc[:, cols], qn[h * nb_t:(h + 1) * nb_t])
+                    ops.sgpr_rownorm_parts(ops.dgemm(Fc, self.V, transB=True, tri_b=2, C=Gc), qv)
+            elif self.digits:
+                kup = ku[:ops.gibbs_digits_splits(nc, M) * nc].view(-1, nc)
+                ops.gibbs_diag_fwd_digits(xc, ell_x, self.Z, self.ell_z, self.one, Ad, u=self.u, Ku_part=kup)
+                ops.o8_sum_partials(kup, out=mc)
+                ops.o8_trinorm_digits(nc, M, M, Ad, self.one, Pd, Pe, qn)
+                ops.o8_trinorm_digits(nc, M, M, Ad, self.one, Vd, Ve, qv)
+            else:
+                K = ops.gibbs_diag_fwd(xc, ell_x, self.Z, self.ell_z, out=Kbuf[:nc])
+                ops.gemv_n(K, self.u, out=mc)
+                ops.sgpr_rownorm_parts(ops.dgemm(K, self.Pblocks[0], transB=True, tri_b=2, C=Gbuf[:nc]), qn)
+                ops.sgpr_rownorm_parts(ops.dgemm(K, self.V, transB=True, tri_b=2, C=Gbuf[:nc]), qv)
+            if field:
+                fld[:, lo:lo + nc] = ell_x
+            ops.sgpr_predict_finish(qn, nb_t, qv, self.s, self.noise, var[lo:lo + nc], os_t=self.hyp[3:] if st else None,
+                                    mean=mc, y=y[lo:lo + nc] if y is not None else None, var_y=var_y[lo:lo + nc],
+                                    lpd=lpd[lo:lo + nc] if y is not None else None, sums=sums, work=work)
+        return Predictive(mean, var, var_y, fld, lpd, sums)
