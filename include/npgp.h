@@ -385,6 +385,9 @@ int npgp_svgp_predict(npgp_svgp_plan* plan, long n, const double* xs, const doub
  * fixed plan and prepared factors the draws are bitwise reproducible (the prepares split their M x M products over K with FP64
  * atomics from M = 512 on). */
 long npgp_svgp_sample_workspace_bytes(const npgp_svgp_config* cfg, int S);
+/* E^T of S draws of width W, the one generator of both samplers' row-independent normals: Et (Sp x W, contiguous)
+ * Et[s * W + j] = E[j, s] = normal_from_index(seed, (s << 32) + j) for s < S, 0 for S <= s < Sp.  Sp >= S. */
+int npgp_sample_normals(int W, int S, int Sp, unsigned long long seed, double* Et, npgp_stream_t stream);
 int npgp_svgp_sample_prepare(npgp_svgp_plan* plan, const double* theta, int S, unsigned long long seed, void* work,
                              long work_bytes, npgp_stream_t stream);
 int npgp_svgp_sample(npgp_svgp_plan* plan, long n, const double* xs, long row_offset, const double* theta, int noise,
@@ -412,6 +415,15 @@ int npgp_sgpr_predict_finish(int n, const double* qn, long qn_stride, int nb_t, 
 /* FP64 per-column-block row norms q[cb * q_stride + i] = sum_{j in [64 cb, min(64 cb + 64, W))} G_ij^2 (one warp per row,
  * fixed order): the partials npgp_o8_trinorm_digits gives, for widths the digit path does not take. */
 int npgp_sgpr_rownorm_parts(int n, int W, const double* G, long ldg, double* q, long q_stride, npgp_stream_t stream);
+/* Finishing kernel of the SGPR posterior draws (sgpr.py posterior().sample()) for one chunk of n rows, one launch: with the
+ * residual r_i = [nb_t > 0] max(os_t - q_t, 0) + s max(1 - q_s, 0) of the partials qn (as npgp_sgpr_predict_finish, no V term)
+ *   out[s * ldo + i] = mean[i] + F[i * ldf + s] + sqrt(r_i (+ *noise if add_noise)) xi_s(row0 + i),   s < S, i < n
+ * xi_s(row) = normal_from_index(seed, 2^63 + (s << 48) + row) as in npgp_svgp_sample.  F (n x ldf, ldf >= S) = K V^T E, its
+ * columns s >= S are never read.  Device scalars s, noise (with add_noise), os_t (with nb_t > 0).  S in 1 .. 1024, ldo >= n,
+ * row0 >= 0, row0 + n <= 2^48; anything else (and NULL operands) is NPGP_EINVAL. */
+int npgp_sgpr_sample_finish(int n, int S, const double* mean, const double* qn, long qn_stride, int nb_t, int nb_s,
+                            const double* F, long ldf, const double* s, const double* noise, const double* os_t, int add_noise,
+                            unsigned long long seed, long row0, double* out, long ldo, npgp_stream_t stream);
 
 /* ---- the path's one collective (csrc/comm.cu; SURVEY.md section 8(e)): sum all-reduce of the flat fp64 gradient buffer.
  * NCCL is bound at run time (dlopen), the communicator is an opaque handle.  id128: 128-byte token made on one rank by

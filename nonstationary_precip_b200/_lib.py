@@ -111,10 +111,12 @@ _SIGS = {
     "npgp_svgp_sample_workspace_bytes": ([_p, _i], _l),
     "npgp_svgp_sample_prepare": ([_p, _p, _i, C.c_ulonglong, _p, _l, _p], _i),
     "npgp_svgp_sample": ([_p, _l, _p, _l, _p, _i, _p, _l, _p, _l, _p], _i),
+    "npgp_sample_normals": ([_i, _i, _i, C.c_ulonglong, _p, _p], _i),
     "npgp_svgp_buffer": ([_p, _i], _p),
     "npgp_sgpr_predict_workspace_bytes": ([_i], _l),
     "npgp_sgpr_predict_finish": ([_i, _p, _l, _i, _i, _p, _l, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _l, _p], _i),
     "npgp_sgpr_rownorm_parts": ([_i, _i, _p, _l, _p, _l, _p], _i),
+    "npgp_sgpr_sample_finish": ([_i, _i, _p, _p, _l, _i, _i, _p, _l, _p, _p, _p, _i, C.c_ulonglong, _l, _p, _l, _p], _i),
     "npgp_comm_unique_id": ([_p], _i),
     "npgp_comm_create": ([_p, _p, _i, _i], _i),
     "npgp_comm_destroy": ([_p], _i),

@@ -24,6 +24,7 @@
 
 #include "common.cuh"
 #include "philox.cuh"
+#include "sample.cuh"
 #include "svgp_glue.cuh"
 #include "../../include/npgp.h"
 
@@ -270,18 +271,18 @@ __global__ void __launch_bounds__(256) svgp_predict_sums_kernel(int nblk, int n,
 }
 
 
-// Et (Sp x M) = E^T of the sampler: Et[s][j] = E[j, s] = normal_from_index(seed, (s << 32) + j) for s < S, zero rows s >= S
-__global__ void svgp_sample_normals_kernel(int M, int S, int Sp, unsigned long long seed, double* __restrict__ Et) {
+// Et (Sp x W) = E^T of the samplers: Et[s][j] = E[j, s] = normal_from_index(seed, (s << 32) + j) for s < S, zero rows s >= S
+__global__ void sample_normals_kernel(int W, int S, int Sp, unsigned long long seed, double* __restrict__ Et) {
   const long k = (long)blockIdx.x * 256 + threadIdx.x;
-  if (k >= (long)Sp * M) return;
-  const int s = (int)(k / M), j = (int)(k % M);
+  if (k >= (long)Sp * W) return;
+  const int s = (int)(k / W), j = (int)(k % W);
   Et[k] = s < S ? normal_from_index(seed, ((unsigned long long)s << 32) + (unsigned long long)j) : 0.0;
 }
 
 // Posterior draws of one chunk of n rows (scal = [s, noise, ...]), CTA = 32 rows x 8 thread rows:
 //   out[s ldo + i] = mean_i + (F[i ldf + s] + sqrt(r_i) xi_s(row0 + i)),  r_i = max(s + jitter_xx - q_i, 0) (+ noise)
-// mean_i and q_i are the partials added in index order (mean as in svgp_predict_finish_kernel); F (n x ldf) = K W is read
-// along s and written along i through a shared-memory tile; xi_s(row) = normal_from_index(seed, 2^63 + (s << 48) + row).
+// mean_i and q_i are the partials added in index order (mean as in svgp_predict_finish_kernel); F (n x ldf) = K W is stored
+// by sample_store_rows (sample.cuh).
 __global__ void __launch_bounds__(256) svgp_sample_finish_kernel(int n, int S, const double* __restrict__ mu_part, int nsplit,
                                                                  const double* __restrict__ q_part, int nq,
                                                                  const double* __restrict__ scal, double jitter_xx, int noise,
@@ -289,7 +290,7 @@ __global__ void __launch_bounds__(256) svgp_sample_finish_kernel(int n, int S, c
                                                                  long row0, double* __restrict__ out, long ldo) {
   __shared__ double tile[32][33];
   __shared__ double smean[32], ssd[32];
-  const int tx = threadIdx.x, ty = threadIdx.y, i0 = blockIdx.x * 32, i = i0 + tx;
+  const int tx = threadIdx.x, ty = threadIdx.y, i = blockIdx.x * 32 + tx;
   if (ty == 0) {
     double mu = 0.0, q = 0.0;
     if (i < n) {
@@ -302,21 +303,7 @@ __global__ void __launch_bounds__(256) svgp_sample_finish_kernel(int n, int S, c
     smean[tx] = mu;
     ssd[tx] = sqrt(r);
   }
-  for (int s0 = 0; s0 < S; s0 += 32) {
-    for (int rr = ty; rr < 32; rr += 8) {
-      const int s = s0 + tx;
-      tile[rr][tx] = (i0 + rr < n && s < S) ? F[(long)(i0 + rr) * ldf + s] : 0.0;
-    }
-    __syncthreads();
-    for (int c = ty; c < 32; c += 8) {
-      const int s = s0 + c;
-      if (s < S && i < n) {
-        const double xi = normal_from_index(seed, (1ull << 63) + ((unsigned long long)s << 48) + (unsigned long long)(row0 + i));
-        out[(long)s * ldo + i] = smean[tx] + fma(ssd[tx], xi, tile[tx][c]);
-      }
-    }
-    __syncthreads();
-  }
+  sample_store_rows(n, S, F, ldf, seed, row0, out, ldo, tile, smean, ssd);
 }
 }  // namespace npgp
 
@@ -982,6 +969,16 @@ extern "C" int npgp_svgp_predict(npgp_svgp_plan* p, long n, const double* xs, co
 // Everything beyond the plan lives in the caller's `work`: G = P^T P and its planes, W^T (Sp = 64 ceil(S / 64) rows; E^T and
 // Y = E^T Ls^T on the way) and its planes, and the B_local x Sp chunk of F = K W.
 // ---------------------------------------------------------------------------------------------------------------------
+/* E^T of S draws (Sp x W, zero rows s >= S), the one generator of both samplers' E (the SGPR one calls it from sgpr.py). */
+extern "C" int npgp_sample_normals(int W, int S, int Sp, unsigned long long seed, double* Et, cudaStream_t st) {
+  if (W < 0 || S < 0 || Sp < S) return NPGP_EINVAL;
+  if ((long)Sp * W == 0) return NPGP_OK;
+  if (!Et) return NPGP_EINVAL;
+  sample_normals_kernel<<<(unsigned)ceil_div((long)Sp * W, 256), 256, 0, st>>>(W, S, Sp, seed, Et);
+  NPGP_LAUNCH_CHECK();
+  return NPGP_OK;
+}
+
 struct SampleBufs {
   double *G, *Y, *Wt, *F;
   int8_t *Gd, *Wd;
@@ -1026,8 +1023,7 @@ extern "C" int npgp_svgp_sample_prepare(npgp_svgp_plan* p, const double* theta, 
   NPGP_TRY(npgp_symmetrize(M, b.G, M, 0, st));
   NPGP_TRY(npgp_o8_slice_rows(M, M, b.G, M, 64, b.Gd, b.gexp, st));
   // W^T = E^T Ls^T P: E^T into Wt, Y = E^T Ls^T (Ls_t lower), then Wt = Y P (P lower)
-  svgp_sample_normals_kernel<<<(unsigned)ceil_div((long)Sp * M, 256), 256, 0, st>>>(M, S, Sp, seed, b.Wt);
-  NPGP_LAUNCH_CHECK();
+  NPGP_TRY(npgp_sample_normals(M, S, Sp, seed, b.Wt, st));
   NPGP_TRY(npgp_dgemm(0, 1, Sp, M, M, 1.0, b.Wt, M, p->Ls_t, M, 0.0, b.Y, M, 0, 2, 0, st));
   NPGP_TRY(npgp_dgemm(0, 0, Sp, M, M, 1.0, b.Y, M, p->P, M, 0.0, b.Wt, M, 0, 1, 0, st));
   NPGP_TRY(npgp_o8_slice_rows(Sp, M, b.Wt, M, 64, b.Wd, b.wexp, st));

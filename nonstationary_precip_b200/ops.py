@@ -338,6 +338,32 @@ def o8_trinorm_digits(n, N, Kd, a_digits, a_scale, b_digits, b_expo, q_part, Ms=
     return q_part
 
 
+def o8_gemm_digits(n, N, Kd, a_digits, a_scale, b_digits, b_expo, T, a_expo=None):
+    """T (n x N) = A B^T from planes, stored only: A (n x Kd, block_rows 128), B (N x Kd, block_rows 64, per-row exponents
+    b_expo).  a_scale: device scalar bounding A unless per-row exponents a_expo.  T: row stride even and >= N."""
+    check(lib().npgp_o8_gemm_digits(n, N, Kd, ptr(a_digits), ptr(a_expo), ptr(a_scale), ptr(b_digits), ptr(b_expo), ptr(T),
+                                    T.stride(0), stream()), "npgp_o8_gemm_digits")
+    return T
+
+
+def sample_normals(W, S, seed, Et):
+    """Et (Sp, W) = E^T of S draws: Et[s, j] = normal_from_index(seed, (s << 32) + j) for s < S, zero rows s >= S."""
+    assert Et.shape[1] == W and Et.is_contiguous()
+    check(lib().npgp_sample_normals(W, S, Et.shape[0], int(seed), ptr(Et), stream()), "npgp_sample_normals")
+    return Et
+
+
+def sgpr_sample_finish(mean, qn, nb_t, F, S, s, noise, out, os_t=None, add_noise=False, seed=0, row0=0):
+    """Draws of one chunk: out[s, i] = mean_i + F[i, s] + sqrt(r_i (+ noise)) xi_s(row0 + i) for s < S, with the residual r
+    of the row-norm partials qn (nb_t temporal blocks, then the Gibbs ones); out may be a column view (row stride >= n)."""
+    n = mean.shape[0]
+    assert F.stride(1) == 1 and out.stride(1) == 1
+    check(lib().npgp_sgpr_sample_finish(n, S, ptr(mean), ptr(qn), qn.stride(0), nb_t, qn.shape[0] - nb_t, ptr(F), F.stride(0),
+                                        ptr(s), ptr(noise), ptr(os_t), int(bool(add_noise)), int(seed), int(row0), ptr(out),
+                                        out.stride(0), stream()), "npgp_sgpr_sample_finish")
+    return out
+
+
 def sgpr_rownorm_parts(G, q_part):
     """q_part[cb, i] = sum_{j in [64 cb, 64 cb + 64)} G_ij^2 (FP64; G may be a column view)."""
     n, W = G.shape

@@ -471,9 +471,10 @@ class SGPRSpatioTemporalStream(torch.nn.Module):
 
 class SGPRPosterior:
     """Snapshot of a streamed SGPR posterior, returned by SGPRGibbsStream.posterior ("diag") and
-    SGPRSpatioTemporalStream.posterior ("st").  It holds copies of everything the predictive needs (Z, the lengthscale
-    field's interpolation weights, u, and P and V -- as digit planes when the feature width is a multiple of 128), so later
-    optimiser steps on the model do not change its predictions."""
+    SGPRSpatioTemporalStream.posterior ("st").  It holds copies of everything the predictive and the sampler need (Z, the
+    lengthscale field's interpolation weights, u, P -- as digit planes when the feature width W is a multiple of 128 -- and V
+    in FP64, plus its planes on that path), so later optimiser steps on the model do not change its predictions or draws.
+    V costs 8 W^2 bytes in FP64 (134 MB at W = 4096); sample() needs it to form W^T = E^T V."""
 
     def __init__(self, model, kind, *, P, V, u, s, noise, ell_z, alpha, use_i8, hyp=None, zt=None):
         self.kind = kind
@@ -488,6 +489,7 @@ class SGPRPosterior:
         self.hyp = hyp.detach().clone() if hyp is not None else None
         self.zt = zt.detach().clone() if zt is not None else None
         self.digits = bool(use_i8) and self.width % 128 == 0
+        self.V = V.detach().clone()
         if self.digits:
             self.planes = []
             for Mx in (P, V):  # B operands of npgp_o8_trinorm_digits: block_rows 64, per-row exponents
@@ -498,8 +500,75 @@ class SGPRPosterior:
             self.one = torch.ones((), dtype=torch.float64, device=P.device)  # bound of the unscaled Gibbs entries
         else:
             M = self.M
-            self.V = V.detach().clone()
             self.Pblocks = [P[:M, :M].contiguous(), P[M:, M:].contiguous()] if kind == "st" else [P.detach().clone()]
+
+    def _row_buffers(self, xs, chunk):
+        """Buffers of the row pass (_row_chunk) over xs in chunks of up to `chunk` rows, allocated once per call."""
+        n, dev = xs.shape[0], xs.device
+        f64 = dict(dtype=torch.float64, device=dev)
+        st = self.kind == "st"
+        M, W = self.M, self.width
+        rows = min(chunk, n)
+        cdiv = lambda a, b: (a + b - 1) // b  # noqa: E731
+        b = dict(D=2 if st else self.Z.shape[1], rows=rows)
+        b["nb_t"] = (M // 64 if self.digits else cdiv(M, 64)) if st else 0
+        nbn = W // 64 if self.digits else (2 if st else 1) * cdiv(M, 64)
+        b["qn"] = torch.empty(nbn, rows, **f64)
+        b["ell"] = torch.empty(b["D"] * rows, **f64)
+        if st:
+            b["xt"], b["xs"] = xs[:, 0].contiguous(), xs[:, 1:3].contiguous()
+            b["F"] = torch.empty(rows, W, **f64)
+        else:
+            b["xs"] = xs
+        if self.digits:
+            b["Ad"] = torch.empty(ops.digits_bytes(rows, W, 128), dtype=torch.uint8, device=dev)
+            if st:
+                b["Ae"] = torch.empty(cdiv(rows, 128) * 128, dtype=torch.int32, device=dev)
+            else:
+                sizes = {rows, n - (n - 1) // chunk * chunk}
+                b["ku"] = torch.empty(max(ops.gibbs_digits_splits(r, M) for r in sizes) * rows, **f64)
+        else:
+            b["G"] = torch.empty(rows, W, **f64)
+            if not st:
+                b["K"] = torch.empty(rows, M, **f64)
+        return b
+
+    def _row_chunk(self, b, lo, nc, mean):
+        """The part of a chunk of rows lo .. lo + nc that predictive() and sample() share: the lengthscale field, the feature
+        rows k(x) (FP64 and/or digit planes in b), the mean k^T u into `mean` and the partials of |P k|^2 into b["qn"].
+        Returns (ell(x) (D, nc), the FP64 feature rows (nc, W) or None on the diagonal model's digit path)."""
+        st = self.kind == "st"
+        M, W, D, qn = self.M, self.width, b["D"], b["qn"]
+        ell = b["ell"][:D * nc].view(D, nc, 1)
+        xc = b["xs"][lo:lo + nc]
+        ops.rbf_matvec_fwd(xc, self.zs, self.prior_lam, self.prior_os, self.alpha.unsqueeze(-1), bias=self.prior_c,
+                           apply_exp=True, out=ell)
+        ell_x = ell.view(D, nc)
+        if st:
+            Fc = b["F"][:nc]
+            ops.rbfper_fwd(b["xt"][lo:lo + nc], self.zt, self.hyp, out=Fc[:, :M])
+            ops.gibbs_diag_fwd(xc, ell_x, self.zs, self.ell_z, out=Fc[:, M:])
+            ops.gemv_n(Fc, self.u, out=mean)
+            if self.digits:
+                ops.o8_slice_rows(Fc, 128, b["Ad"], b["Ae"])
+                ops.o8_trinorm_digits(nc, W, W, b["Ad"], None, *self.planes[0], qn, Ms=M, a_expo=b["Ae"])
+            else:
+                Gc, nb_t = b["G"][:nc], b["nb_t"]
+                for h, Ph in enumerate(self.Pblocks):
+                    cols = slice(h * M, (h + 1) * M)
+                    ops.dgemm(Fc[:, cols], Ph, transB=True, tri_b=2, C=Gc[:, cols])
+                    ops.sgpr_rownorm_parts(Gc[:, cols], qn[h * nb_t:(h + 1) * nb_t])
+            return ell_x, Fc
+        if self.digits:
+            kup = b["ku"][:ops.gibbs_digits_splits(nc, M) * nc].view(-1, nc)
+            ops.gibbs_diag_fwd_digits(xc, ell_x, self.Z, self.ell_z, self.one, b["Ad"], u=self.u, Ku_part=kup)
+            ops.o8_sum_partials(kup, out=mean)
+            ops.o8_trinorm_digits(nc, M, M, b["Ad"], self.one, *self.planes[0], qn)
+            return ell_x, None
+        K = ops.gibbs_diag_fwd(xc, ell_x, self.Z, self.ell_z, out=b["K"][:nc])
+        ops.gemv_n(K, self.u, out=mean)
+        ops.sgpr_rownorm_parts(ops.dgemm(K, self.Pblocks[0], transB=True, tri_b=2, C=b["G"][:nc]), qn)
+        return ell_x, K
 
     @torch.no_grad()
     def predictive(self, xs, y=None, *, field: bool = False, chunk: int = 65536):
@@ -514,7 +583,7 @@ class SGPRPosterior:
         dev = xs.device
         f64 = dict(dtype=torch.float64, device=dev)
         st = self.kind == "st"
-        M, W = self.M, self.width
+        W = self.width
         D = 2 if st else self.Z.shape[1]
         mean, var, var_y = (torch.empty(n, **f64) for _ in range(3))
         fld = torch.empty(D, n, **f64) if field else None
@@ -524,67 +593,74 @@ class SGPRPosterior:
             lpd, sums = torch.empty(n, **f64), torch.zeros(3, **f64)
         if n == 0:
             return Predictive(mean, var, var_y, fld, lpd, sums)
-        rows = min(chunk, n)
-        cdiv = lambda a, b: (a + b - 1) // b  # noqa: E731
-        nb_t = (M // 64 if self.digits else cdiv(M, 64)) if st else 0
-        nbn = W // 64 if self.digits else (2 if st else 1) * cdiv(M, 64)
-        qn = torch.empty(nbn, rows, **f64)
-        qv = torch.empty(cdiv(W, 64), rows, **f64)
-        work = ops.sgpr_predict_workspace(rows, dev) if y is not None else None
-        ell_buf = torch.empty(D * rows, **f64)
-        if st:
-            xt_all, xs_all = xs[:, 0].contiguous(), xs[:, 1:3].contiguous()
-            Fbuf = torch.empty(rows, W, **f64)
-        if self.digits:
-            Ad = torch.empty(ops.digits_bytes(rows, W, 128), dtype=torch.uint8, device=dev)
-            if st:
-                Ae = torch.empty(cdiv(rows, 128) * 128, dtype=torch.int32, device=dev)
-            else:
-                sizes = {rows, n - (n - 1) // chunk * chunk}
-                ku = torch.empty(max(ops.gibbs_digits_splits(r, M) for r in sizes) * rows, **f64)
-            (Pd, Pe), (Vd, Ve) = self.planes
-        else:
-            Gbuf = torch.empty(rows, W, **f64)
-            if not st:
-                Kbuf = torch.empty(rows, M, **f64)
+        b = self._row_buffers(xs, chunk)
+        qn, nb_t = b["qn"], b["nb_t"]
+        qv = torch.empty((W + 63) // 64, b["rows"], **f64)
+        work = ops.sgpr_predict_workspace(b["rows"], dev) if y is not None else None
         for lo in range(0, n, chunk):
             nc = min(chunk, n - lo)
-            ell = ell_buf[:D * nc].view(D, nc, 1)
-            xc = xs_all[lo:lo + nc] if st else xs[lo:lo + nc]
-            ops.rbf_matvec_fwd(xc, self.zs, self.prior_lam, self.prior_os, self.alpha.unsqueeze(-1), bias=self.prior_c,
-                               apply_exp=True, out=ell)
-            ell_x = ell.view(D, nc)
             mc = mean[lo:lo + nc]
-            if st:
-                Fc = Fbuf[:nc]
-                ops.rbfper_fwd(xt_all[lo:lo + nc], self.zt, self.hyp, out=Fc[:, :M])
-                ops.gibbs_diag_fwd(xc, ell_x, self.zs, self.ell_z, out=Fc[:, M:])
-                ops.gemv_n(Fc, self.u, out=mc)
-                if self.digits:
-                    ops.o8_slice_rows(Fc, 128, Ad, Ae)
-                    ops.o8_trinorm_digits(nc, W, W, Ad, None, Pd, Pe, qn, Ms=M, a_expo=Ae)
-                    ops.o8_trinorm_digits(nc, W, W, Ad, None, Vd, Ve, qv, a_expo=Ae)
-                else:
-                    Gc = Gbuf[:nc]
-                    for h, Ph in enumerate(self.Pblocks):
-                        cols = slice(h * M, (h + 1) * M)
-                        ops.dgemm(Fc[:, cols], Ph, transB=True, tri_b=2, C=Gc[:, cols])
-                        ops.sgpr_rownorm_parts(Gc[:, cols], qn[h * nb_t:(h + 1) * nb_t])
-                    ops.sgpr_rownorm_parts(ops.dgemm(Fc, self.V, transB=True, tri_b=2, C=Gc), qv)
-            elif self.digits:
-                kup = ku[:ops.gibbs_digits_splits(nc, M) * nc].view(-1, nc)
-                ops.gibbs_diag_fwd_digits(xc, ell_x, self.Z, self.ell_z, self.one, Ad, u=self.u, Ku_part=kup)
-                ops.o8_sum_partials(kup, out=mc)
-                ops.o8_trinorm_digits(nc, M, M, Ad, self.one, Pd, Pe, qn)
-                ops.o8_trinorm_digits(nc, M, M, Ad, self.one, Vd, Ve, qv)
+            ell_x, feats = self._row_chunk(b, lo, nc, mc)
+            if self.digits:
+                ops.o8_trinorm_digits(nc, W, W, b["Ad"], None if st else self.one, *self.planes[1], qv,
+                                      a_expo=b["Ae"] if st else None)
             else:
-                K = ops.gibbs_diag_fwd(xc, ell_x, self.Z, self.ell_z, out=Kbuf[:nc])
-                ops.gemv_n(K, self.u, out=mc)
-                ops.sgpr_rownorm_parts(ops.dgemm(K, self.Pblocks[0], transB=True, tri_b=2, C=Gbuf[:nc]), qn)
-                ops.sgpr_rownorm_parts(ops.dgemm(K, self.V, transB=True, tri_b=2, C=Gbuf[:nc]), qv)
+                ops.sgpr_rownorm_parts(ops.dgemm(feats, self.V, transB=True, tri_b=2, C=b["G"][:nc]), qv)
             if field:
                 fld[:, lo:lo + nc] = ell_x
             ops.sgpr_predict_finish(qn, nb_t, qv, self.s, self.noise, var[lo:lo + nc], os_t=self.hyp[3:] if st else None,
                                     mean=mc, y=y[lo:lo + nc] if y is not None else None, var_y=var_y[lo:lo + nc],
                                     lpd=lpd[lo:lo + nc] if y is not None else None, sums=sums, work=work)
         return Predictive(mean, var, var_y, fld, lpd, sums)
+
+    @torch.no_grad()
+    def sample(self, xs, num_samples: int, *, seed: int = 0, noise: bool = False, row_offset: int = 0,
+               chunk: int = 65536) -> torch.Tensor:
+        """num_samples posterior draws of f (noise=True: of y) at the rows xs (n, D), correlated across rows: (num_samples,
+        n), streamed in chunks of `chunk` rows.  The draws are exact samples of the joint predictive of posterior(), i.e. of
+        the reference's eval-mode predictive with the low-rank root (for the spatio-temporal model its literal=False form,
+        not the default literal=True one, whose dense-row factors give a covariance of another form):
+            f_s(x) = k(x)^T u + (V k(x))^T e_s + sqrt(r(x)) xi_s(x),   e_s ~ N(0, I_W),  xi_s(x) ~ N(0, 1)
+            Cov(f(x), f(x')) = (V k(x))^T (V k(x')) + delta(x, x') r(x),   r(x) = predictive().var - |V k(x)|^2
+        with r(x) = [st] max(os_t - |P_t k_t|^2, 0) + s max(1 - |P_s k_s|^2, 0).  noise=True adds the noise variance to r.
+        The mean term is predictive().mean.  Keys as SVGPGibbs.sample: e_s[j] = normal(seed, (s << 32) + j) and xi_s(row) =
+        normal(seed, 2^63 + (s << 48) + row_offset + i), so draw s does not depend on num_samples and rows sharded over ranks
+        with their global row_offset are parts of one joint draw (up to the rounding of the M x M algebra that posterior()
+        replicates after its all-reduce).  Per call: E^T (64 ceil(S / 64) x W), W^T = E^T V and its digit planes, then per
+        chunk the rows as in predictive() without its V pass, K W^T^T and one finishing kernel; buffers are allocated once
+        per call and the chunk loop does not synchronise with the host.  For the same snapshot, rows, chunking and seed the
+        draws are bitwise reproducible below W = 512; from there on npgp_dgemm may split the product E^T V over its inner
+        dimension with FP64 atomics (small outputs with a long inner dimension), and two calls then agree to rounding."""
+        S = int(num_samples)
+        if not 1 <= S <= 1024:
+            raise ValueError("num_samples must be in 1 .. 1024 (got %d)" % S)
+        xs = xs.contiguous()
+        n = xs.shape[0]
+        if row_offset < 0 or row_offset + n > 1 << 48:
+            raise ValueError("rows row_offset .. row_offset + n must lie in [0, 2^48) (got %d + %d)" % (row_offset, n))
+        dev = xs.device
+        f64 = dict(dtype=torch.float64, device=dev)
+        out = torch.empty(S, n, **f64)
+        if n == 0:
+            return out
+        st = self.kind == "st"
+        W, Sp = self.width, (S + 63) // 64 * 64
+        Wt = ops.dgemm(ops.sample_normals(W, S, seed, torch.empty(Sp, W, **f64)), self.V, tri_b=1)  # W^T = E^T V
+        b = self._row_buffers(xs, chunk)
+        if self.digits:
+            Wd = torch.empty(ops.digits_bytes(Sp, W, 64), dtype=torch.uint8, device=dev)
+            We = torch.empty(Sp, dtype=torch.int32, device=dev)
+            ops.o8_slice_rows(Wt, 64, Wd, We)
+        mean = torch.empty(b["rows"], **f64)
+        Fbuf = torch.empty(b["rows"], Sp, **f64)
+        for lo in range(0, n, chunk):
+            nc = min(chunk, n - lo)
+            mc, Fc = mean[:nc], Fbuf[:nc]
+            _, feats = self._row_chunk(b, lo, nc, mc)
+            if self.digits:
+                ops.o8_gemm_digits(nc, Sp, W, b["Ad"], None if st else self.one, Wd, We, Fc, a_expo=b["Ae"] if st else None)
+            else:
+                ops.dgemm(feats, Wt, transB=True, C=Fc)
+            ops.sgpr_sample_finish(mc, b["qn"], b["nb_t"], Fc, S, self.s, self.noise, out[:, lo:lo + nc],
+                                   os_t=self.hyp[3:] if st else None, add_noise=noise, seed=seed, row0=row_offset + lo)
+        return out
