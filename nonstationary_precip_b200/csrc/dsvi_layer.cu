@@ -19,11 +19,14 @@
 
 namespace npgp {
 
-// var_i = max(os + add_var + q_i, min_var)
+// var_i = max(os + add_var + q_i, min_var), written as a comparison so that a NaN (a row with a missing coordinate) stays NaN
 static __global__ void dsvi_var_kernel(int n, const double* __restrict__ q, const double* __restrict__ os, double add_var,
                                        double min_var, double* __restrict__ var) {
   const int i = blockIdx.x * 256 + threadIdx.x;
-  if (i < n) var[i] = fmax(*os + add_var + q[i], min_var);
+  if (i < n) {
+    const double v = *os + add_var + q[i];
+    var[i] = (v < min_var) ? min_var : v;
+  }
 }
 
 // gv_i = dvar_i where the variance was not clamped, else 0; gv2 = 2 gv; cnt += #(gv_i == gv_0); sum += gv_i

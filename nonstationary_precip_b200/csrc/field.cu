@@ -13,7 +13,18 @@ namespace npgp {
 constexpr int kFT = 128;   // threads per CTA
 constexpr int kFR = 32;    // rows (fwd) / columns (bwd) per CTA = lanes
 constexpr int kFS = 4;     // slices of the reduced axis per CTA = warps
-constexpr int kFChunk = 64;  // reduced-axis points staged per slice per round
+
+// Reduced-axis points staged per slice per round: 64 while the kernel's static shared memory (the staged points, the
+// per-warp accumulators and the exp table) stays within 48 KB, which holds for every configuration up to d = 3; above
+// that the largest multiple of 8 that fits (d = nb = 4: 64 forward, 56 backward; 5: 40 / 32; 6: 24 / 24).
+template <int d, int NB, int NV, bool BWD>
+constexpr int field_chunk() {
+  constexpr long kLimit = 48 * 1024;
+  constexpr long fixed = 8L * kFS * kFR * (NB * NV + (BWD ? d : 0)) + 8L * 256;
+  constexpr long per_point = 8L * kFS * NB * (d + NV);
+  constexpr long fit = (kLimit - fixed) / per_point / 8 * 8;
+  return fit > 64 ? 64 : (int)fit;
+}
 
 // forward: lanes own rows, warps own column slices
 template <int d, int NB, int NV>
@@ -24,10 +35,13 @@ __global__ void __launch_bounds__(kFT) rbf_matvec_fwd_kernel(int n, int m, const
                                                              const double* __restrict__ V,
                                                              const double* __restrict__ bias, int apply_exp,
                                                              double* __restrict__ out) {
-  __shared__ double sz[kFS][kFChunk][NB][d];   // pre-scaled column coordinates z/lam_b
-  __shared__ double sv[kFS][kFChunk][NB][NV];  // os_b * V
+  constexpr int kChunk = field_chunk<d, NB, NV, false>();
+  static_assert(kChunk >= 8, "field_chunk: configuration too large for static shared memory");
+  __shared__ double sz[kFS][kChunk][NB][d];   // pre-scaled column coordinates z/lam_b
+  __shared__ double sv[kFS][kChunk][NB][NV];  // os_b * V
   __shared__ double sacc[kFS][kFR][NB * NV];
   __shared__ double sexp[256];
+  static_assert(sizeof(sz) + sizeof(sv) + sizeof(sacc) + sizeof(sexp) <= 48 * 1024, "static shared memory over 48 KB");
   load_exp_table(sexp);
   __syncthreads();
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -46,8 +60,8 @@ __global__ void __launch_bounds__(kFT) rbf_matvec_fwd_kernel(int n, int m, const
   // warp w handles columns [w*per, (w+1)*per)
   const int per = (m + kFS - 1) / kFS;
   const int jlo = warp * per, jhi = min(m, jlo + per);
-  for (int j0 = jlo; j0 < jhi; j0 += kFChunk) {
-    const int nc = min(kFChunk, jhi - j0);
+  for (int j0 = jlo; j0 < jhi; j0 += kChunk) {
+    const int nc = min(kChunk, jhi - j0);
     __syncwarp();
     for (int t = lane; t < nc; t += 32) {
       const int j = j0 + t;
@@ -102,10 +116,13 @@ __global__ void __launch_bounds__(kFT) rbf_matvec_bwd_kernel(int n, int m, const
                                                              const double* __restrict__ V,
                                                              const double* __restrict__ dOut, int rows_per_cta,
                                                              double* __restrict__ dV, double* __restrict__ dz) {
-  __shared__ double sxr[kFS][kFChunk][NB][d];   // pre-scaled row coordinates x/lam_b
-  __shared__ double sg[kFS][kFChunk][NB][NV];   // os_b * dOut
+  constexpr int kChunk = field_chunk<d, NB, NV, true>();
+  static_assert(kChunk >= 8, "field_chunk: configuration too large for static shared memory");
+  __shared__ double sxr[kFS][kChunk][NB][d];   // pre-scaled row coordinates x/lam_b
+  __shared__ double sg[kFS][kChunk][NB][NV];   // os_b * dOut
   __shared__ double sacc[kFS][kFR][NB * NV + d];
   __shared__ double sexp[256];
+  static_assert(sizeof(sxr) + sizeof(sg) + sizeof(sacc) + sizeof(sexp) <= 48 * 1024, "static shared memory over 48 KB");
   load_exp_table(sexp);
   __syncthreads();
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -129,8 +146,8 @@ __global__ void __launch_bounds__(kFT) rbf_matvec_bwd_kernel(int n, int m, const
   const int rb = blockIdx.y * rows_per_cta, re = min(n, rb + rows_per_cta);
   const int per = (re - rb + kFS - 1) / kFS;
   const int ilo = rb + warp * per, ihi = min(re, ilo + per);
-  for (int i0 = ilo; i0 < ihi; i0 += kFChunk) {
-    const int nc = min(kFChunk, ihi - i0);
+  for (int i0 = ilo; i0 < ihi; i0 += kChunk) {
+    const int nc = min(kChunk, ihi - i0);
     __syncwarp();
     for (int t = lane; t < nc; t += 32) {
       const int i = i0 + t;
@@ -207,7 +224,8 @@ static int launch_rbf_bwd(int n, int m, const double* x, const double* z, const 
   long want = (long)kNumSMs * 8;
   long row_ctas = (want + col_blocks - 1) / col_blocks;
   long rpc = (n + row_ctas - 1) / row_ctas;
-  if (rpc < 4 * kFChunk) rpc = 4 * kFChunk;
+  constexpr int kChunk = field_chunk<d, NB, NV, true>();
+  if (rpc < 4 * kChunk) rpc = 4 * kChunk;
   dim3 grid(col_blocks, ceil_div(n, rpc));
   rbf_matvec_bwd_kernel<d, NB, NV><<<grid, kFT, 0, st>>>(n, m, x, z, lam, os, V, dOut, (int)rpc, dV, dz);
   NPGP_LAUNCH_CHECK();
@@ -227,6 +245,9 @@ using namespace npgp;
   if (d == 3 && nb == 1 && nv == 3) return FN<3, 1, 3>(__VA_ARGS__);      \
   if (d == 3 && nb == 1 && nv == 1) return FN<3, 1, 1>(__VA_ARGS__);      \
   if (d == 3 && nb == 2 && nv == 1) return FN<3, 2, 1>(__VA_ARGS__);      \
+  if (d == 4 && nb == 4 && nv == 1) return FN<4, 4, 1>(__VA_ARGS__);      \
+  if (d == 5 && nb == 5 && nv == 1) return FN<5, 5, 1>(__VA_ARGS__);      \
+  if (d == 6 && nb == 6 && nv == 1) return FN<6, 6, 1>(__VA_ARGS__);      \
   return NPGP_EUNSUPPORTED;
 
 extern "C" int npgp_rbf_matvec_fwd(int d, int nb, int nv, int n, int m, const double* x, const double* z,

@@ -1,5 +1,5 @@
-// Per-pair arithmetic of the Gibbs kernels, shared by every tile kernel.  __host__ __device__ so that the formulas can
-// also be checked on a CPU (tests/hostcheck) -- the product only ever calls them from CUDA kernels.
+// Per-pair arithmetic of the Gibbs kernels, shared by every tile kernel (the host branches only keep the header compilable
+// by a host compiler; the product calls these from CUDA kernels, and tests/test_pairmath_range_gpu.py checks them there).
 //
 // Diagonal kernel  (reference: models/gibbs_kernels.py:154-162):
 //     K_ij = prod_d sqrt(2 l_id l_jd / s_d) * exp(-sum_d delta_d^2 / s_d),  s_d = l_id^2 + l_jd^2
@@ -25,7 +25,9 @@ namespace npgp {
 // 1/sqrt(x) and 1/x for the tile kernels: hardware seed (MUFU.RSQ64H / MUFU.RCP64H, ~20 bits) + two Newton steps, branch
 // free.  The library versions carry special-case paths (BSSY/CALL around every use) that cost ~30 % of the tile kernels'
 // issue slots; the arguments here (products of squared lengthscales, determinants of positive definite 2x2 / 3x3
-// matrices) are positive normal numbers, anything else ends in NaN/inf exactly as a failed factorisation would.
+// matrices) are positive normal numbers.  A NaN argument returns NaN (the seed instructions and FMAs propagate it); so do
+// 0 and +inf (the Newton step forms 0 * inf) and, for fast_rsqrt, negative numbers.  A singular or indefinite Sigma thus
+// shows up as NaN in K, as a failed factorisation would.
 NPGP_HD double fast_rsqrt(double x) {
 #if defined(__CUDA_ARCH__)
   double y;
@@ -51,7 +53,10 @@ __host__ __device__
 // exp per pair.  `tab` is the 256-entry table of 2^(j/256) (in shared memory on the device).
 NPGP_HD double exp_neg(double x, const double* tab) {
 #if defined(__CUDA_ARCH__)
-  x = fmax(x, -708.0);  // branch free: exp(-708) = 3e-308 stands in for the underflowed tail
+  // Branch free.  exp(-708) = 3e-308 stands in for the underflowed tail; the clamp is a compare-and-select rather than fmax
+  // so that a NaN argument (a missing coordinate) passes through to t, whose high word is >= 0x7ff00000 exactly when x is
+  // NaN (or +inf).  The last line returns t then: the exponent-field add would turn a NaN v into a finite number.
+  x = (x < -708.0) ? -708.0 : x;
   const double t = fma(x, kInvLn2x256, 6755399441055744.0);  // 2^52 + 2^51: the integer lands in the low mantissa bits
   const int n = __double2loint(t);
   const double nd = t - 6755399441055744.0;
@@ -62,7 +67,8 @@ NPGP_HD double exp_neg(double x, const double* tab) {
   p = fma(p, r, 1.0);
   p = fma(p, r, 1.0);
   const double v = tab[n & 255] * p;  // in [1, 2) up to rounding
-  return __hiloint2double(__double2hiint(v) + ((n >> 8) << 20), __double2loint(v));  // * 2^k through the exponent field
+  const double e = __hiloint2double(__double2hiint(v) + ((n >> 8) << 20), __double2loint(v));  // * 2^k via the exponent
+  return (static_cast<unsigned>(__double2hiint(t)) >= 0x7ff00000u) ? t : e;
 #else
   (void)tab;
   return exp(x);

@@ -34,8 +34,13 @@ __device__ __forceinline__ double sgpr_row_var(int i, const double* __restrict__
   for (int c = 0; c < nb_t; ++c) qt += qn[(long)c * qn_stride + i];
   for (int c = nb_t; c < nb_t + nb_s; ++c) qs += qn[(long)c * qn_stride + i];
   for (int c = 0; c < nb_v; ++c) q2 += qv[(long)c * qv_stride + i];
-  double v = s[0] * fmax(1.0 - qs, 0.0) + q2;
-  if (nb_t > 0) v += fmax(os_t[0] - qt, 0.0);
+  // max(., 0) as comparisons: a NaN row norm (a row with a missing coordinate) stays NaN
+  const double rs = 1.0 - qs;
+  double v = s[0] * (rs < 0.0 ? 0.0 : rs) + q2;
+  if (nb_t > 0) {
+    const double rt = os_t[0] - qt;
+    v += (rt < 0.0 ? 0.0 : rt);
+  }
   return v;
 }
 
