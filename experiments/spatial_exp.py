@@ -10,6 +10,10 @@ plotting tail (cartopy, a results CSV that is not in the repository) is dropped,
 variant come from `utils.dataprep.kmeans_inducing_points` instead of pymc3.
 
     python experiments/spatial_exp.py --n_iter 5000 --splits 10 [--inference sparse --M 250] [--data path/to.csv]
+        [--map_grid 1000 --map_samples 16 --map_out map.npz]
+
+With --map_grid G the model of the last split also predicts over a G x G grid of the data's bounding box through its
+posterior() snapshot (write_map), at any G the device memory allows.
 
 Without --data the table is read from tests/golden/uib_spatial_dataprep.npz (the reference's data fixture, exported by
 tests/golden/make_golden.py).  Needs a GPU: the models run on the npgp CUDA kernels only."""
@@ -62,6 +66,10 @@ def parse_args(argv=None):
     p.add_argument("--scale", type=float, default=0.644, help="0: learn the outputscale, else fixed")
     p.add_argument("--log_every", type=int, default=400)
     p.add_argument("--json", default=None, help="write the per-split metrics here")
+    p.add_argument("--map_grid", type=int, default=0,
+                   help="G > 0: after the last split, predict over a G x G grid spanning the data's bounding box")
+    p.add_argument("--map_samples", type=int, default=0, help="posterior sample fields drawn over the map grid")
+    p.add_argument("--map_out", default="spatial_map.npz", help="where the map arrays are written (.npz)")
     return p.parse_args(argv)
 
 
@@ -128,8 +136,33 @@ def run_split(i, x, y, args, device, log=print):
         pred_y_test = likelihood(model.predict(x_test))
     rmse_test = float(rmse(pred_y_test.loc.detach(), y_test, stdy))
     nlpd_test = float(nlpd(pred_y_test, y_test, stdy.to(device)))
+    if args.map_grid > 0 and i == args.splits - 1:
+        write_map(model, x_norm, meanx, stdx, meany, stdy, args)
     return dict(split=i, rmse=rmse_test, nlpd=nlpd_test, first_loss=losses[0], last_loss=losses[-1],
                 train_s=train_s, steps_per_s=args.n_iter / train_s, trainable=get_trainable_param_names(model))
+
+
+def write_map(model, x_norm, meanx, stdx, meany, stdy, args):
+    """Posterior over a G x G grid spanning the bounding box of the normalised inputs, streamed through the model's
+    posterior() snapshot: mean and var_y in the original units of the target, the lengthscale field (D, G, G) in normalised
+    input units and `map_samples` correlated draws of f in the target's units.  Row i of a (G, G) map is latitude i, column
+    j longitude j; lon / lat (G,) are the grid axes in the original units."""
+    G = args.map_grid
+    lo, hi = x_norm.min(0).values, x_norm.max(0).values
+    axes = [torch.linspace(float(lo[d]), float(hi[d]), G, dtype=torch.float64) for d in range(2)]
+    lat, lon = torch.meshgrid(axes[1], axes[0], indexing="ij")
+    xs = torch.stack([lon.reshape(-1), lat.reshape(-1)], 1).to(model.train_inputs[0].device)
+    post = model.posterior()
+    pred = post.predictive(xs, field=True)
+    out = dict(lon=(axes[0] * stdx[0] + meanx[0]).numpy(), lat=(axes[1] * stdx[1] + meanx[1]).numpy(),
+               mean=(pred.mean * stdy + meany).reshape(G, G).cpu().numpy(),
+               var_y=(pred.var_y * stdy ** 2).reshape(G, G).cpu().numpy(),
+               ell=pred.field.reshape(-1, G, G).cpu().numpy())
+    if args.map_samples > 0:
+        draws = post.sample(xs, args.map_samples, seed=BASE_SEED)
+        out["samples"] = (draws * stdy + meany).reshape(-1, G, G).cpu().numpy()
+    np.savez(args.map_out, **out)
+    print("Map %d x %d (%d draws) written to %s" % (G, G, args.map_samples, args.map_out))
 
 
 def main(argv=None):

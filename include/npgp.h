@@ -412,6 +412,16 @@ int npgp_sgpr_predict_finish(int n, const double* qn, long qn_stride, int nb_t, 
                              int nb_v, const double* mean, const double* y, const double* s, const double* noise,
                              const double* os_t, double* var_f, double* var_y, double* lpd, double* sums, void* work,
                              long work_bytes, npgp_stream_t stream);
+/* Finishing kernel of the exact Gibbs GP's predictive (models/nonstationary_models.py DiagonalExactGP.posterior()) for one
+ * chunk of n rows, one launch.  qn: the nb per-column-block partials of |P_y k(x)|^2 (row c * qn_stride + i), added in index
+ * order; P_y = chol(K + tau I)^-1 of the unscaled training kernel.  Device scalars s, noise; host scalar add_var:
+ *   var_f (n) = s max(1 - q, 0) + add_var                                     required
+ *   var_y, lpd, sums                                                          as npgp_sgpr_predict_finish
+ * work: npgp_sgpr_predict_workspace_bytes(n) bytes, zeroed before its first use (the kernel leaves it so); needed with sums.
+ * n, nb >= 0; anything else (and NULL required operands) is NPGP_EINVAL. */
+int npgp_exact_predict_finish(int n, const double* qn, long qn_stride, int nb, const double* mean, const double* y,
+                              const double* s, const double* noise, double add_var, double* var_f, double* var_y, double* lpd,
+                              double* sums, void* work, long work_bytes, npgp_stream_t stream);
 /* FP64 per-column-block row norms q[cb * q_stride + i] = sum_{j in [64 cb, min(64 cb + 64, W))} G_ij^2 (one warp per row,
  * fixed order): the partials npgp_o8_trinorm_digits gives, for widths the digit path does not take. */
 int npgp_sgpr_rownorm_parts(int n, int W, const double* G, long ldg, double* q, long q_stride, npgp_stream_t stream);

@@ -116,6 +116,7 @@ _SIGS = {
     "npgp_sgpr_predict_workspace_bytes": ([_i], _l),
     "npgp_sgpr_predict_finish": ([_i, _p, _l, _i, _i, _p, _l, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _l, _p], _i),
     "npgp_sgpr_rownorm_parts": ([_i, _i, _p, _l, _p, _l, _p], _i),
+    "npgp_exact_predict_finish": ([_i, _p, _l, _i, _p, _p, _p, _p, _d, _p, _p, _p, _p, _p, _l, _p], _i),
     "npgp_sgpr_sample_finish": ([_i, _i, _p, _p, _l, _i, _i, _p, _l, _p, _p, _p, _i, C.c_ulonglong, _l, _p, _l, _p], _i),
     "npgp_comm_unique_id": ([_p], _i),
     "npgp_comm_create": ([_p, _p, _i, _i], _i),

@@ -1,7 +1,8 @@
 // Row-side kernels of the streamed SGPR posterior (sgpr.py, posterior().predictive() and .sample()): the finishing kernel that
 // turns the per-column-block row norms of P k(x) and V k(x) into the predictive variances and test log-densities, the FP64
 // per-column-block row norms that stand in for npgp_o8_trinorm_digits when the feature width is not a multiple of 128, and
-// the finishing kernel of the posterior draws.
+// the finishing kernel of the posterior draws.  The exact Gibbs GP's snapshot (models/nonstationary_models.py) runs the same
+// row pass and has a finishing kernel of its own for its predictive variances.
 #include "common.cuh"
 #include "sample.cuh"
 
@@ -44,22 +45,21 @@ __device__ __forceinline__ double sgpr_row_var(int i, const double* __restrict__
   return v;
 }
 
-// Per row i of a chunk (scalars s, noise, os_t read from device memory):
-//   q1_t = sum_{c < nb_t} qn[c, i],  q1_s = sum_{nb_t <= c < nb_t + nb_s} qn[c, i],  q2 = sum_{c < nb_v} qv[c, i]  (index order)
-//   var_f = [nb_t > 0] max(os_t - q1_t, 0) + s max(1 - q1_s, 0) + q2,   var_y = var_f + noise
-//   y: lpd = log N(y | mean, var_y);  sums += [sum (y - mean)^2, sum -lpd, n]: block partials in blk, added in index order by the
-//   last block to finish (ticket), which leaves the ticket at 0 again.
-__global__ void __launch_bounds__(256) sgpr_predict_finish_kernel(
-    int n, const double* __restrict__ qn, long qn_stride, int nb_t, int nb_s, const double* __restrict__ qv, long qv_stride,
-    int nb_v, const double* __restrict__ mean, const double* __restrict__ y, const double* __restrict__ s,
-    const double* __restrict__ noise, const double* __restrict__ os_t, double* __restrict__ var_f, double* __restrict__ var_y,
-    double* __restrict__ lpd, double* __restrict__ sums, double* __restrict__ blk, unsigned int* __restrict__ ticket) {
+// The body of the predictive finishers, per row i of a chunk (noise read from device memory), with var_f = row_var(i):
+//   var_y = var_f + noise;  y: lpd = log N(y | mean, var_y);  sums += [sum (y - mean)^2, sum -lpd, n]: block partials in blk,
+//   added in index order by the last block to finish (ticket), which leaves the ticket at 0 again.
+template <class RowVar>
+__device__ __forceinline__ void sgpr_finish_rows(int n, RowVar row_var, const double* __restrict__ mean,
+                                                 const double* __restrict__ y, const double* __restrict__ noise,
+                                                 double* __restrict__ var_f, double* __restrict__ var_y,
+                                                 double* __restrict__ lpd, double* __restrict__ sums,
+                                                 double* __restrict__ blk, unsigned int* __restrict__ ticket) {
   __shared__ double red[32];
   __shared__ bool last;
   const int i = blockIdx.x * 256 + threadIdx.x;
   double r2 = 0.0, nl = 0.0;
   if (i < n) {
-    const double v = sgpr_row_var(i, qn, qn_stride, nb_t, nb_s, qv, qv_stride, nb_v, s, os_t);
+    const double v = row_var(i);
     const double vy = v + noise[0];
     var_f[i] = v;
     if (var_y) var_y[i] = vy;
@@ -93,6 +93,32 @@ __global__ void __launch_bounds__(256) sgpr_predict_finish_kernel(
     sums[2] += (double)n;
     *ticket = 0u;
   }
+}
+
+// Per row i of a chunk (scalars s, noise, os_t read from device memory):
+//   q1_t = sum_{c < nb_t} qn[c, i],  q1_s = sum_{nb_t <= c < nb_t + nb_s} qn[c, i],  q2 = sum_{c < nb_v} qv[c, i]  (index order)
+//   var_f = [nb_t > 0] max(os_t - q1_t, 0) + s max(1 - q1_s, 0) + q2,   then var_y, lpd and sums as sgpr_finish_rows.
+__global__ void __launch_bounds__(256) sgpr_predict_finish_kernel(
+    int n, const double* __restrict__ qn, long qn_stride, int nb_t, int nb_s, const double* __restrict__ qv, long qv_stride,
+    int nb_v, const double* __restrict__ mean, const double* __restrict__ y, const double* __restrict__ s,
+    const double* __restrict__ noise, const double* __restrict__ os_t, double* __restrict__ var_f, double* __restrict__ var_y,
+    double* __restrict__ lpd, double* __restrict__ sums, double* __restrict__ blk, unsigned int* __restrict__ ticket) {
+  sgpr_finish_rows(
+      n, [&](int i) { return sgpr_row_var(i, qn, qn_stride, nb_t, nb_s, qv, qv_stride, nb_v, s, os_t); }, mean, y, noise,
+      var_f, var_y, lpd, sums, blk, ticket);
+}
+
+// The exact GP's finisher (models/nonstationary_models.py DiagonalExactGP.posterior().predictive()), per row i of a chunk:
+//   q = sum_{c < nb} qn[c, i] (index order),  var_f = s max(1 - q, 0) + add_var,   then var_y, lpd and sums as sgpr_finish_rows.
+// q = |P_y k(x)|^2 = k^T (K + tau I)^-1 k < 1 for the unscaled Gibbs kernel, so the clamp changes nothing beyond rounding.
+__global__ void __launch_bounds__(256) exact_predict_finish_kernel(
+    int n, const double* __restrict__ qn, long qn_stride, int nb, const double* __restrict__ mean, const double* __restrict__ y,
+    const double* __restrict__ s, const double* __restrict__ noise, double add_var, double* __restrict__ var_f,
+    double* __restrict__ var_y, double* __restrict__ lpd, double* __restrict__ sums, double* __restrict__ blk,
+    unsigned int* __restrict__ ticket) {
+  sgpr_finish_rows(
+      n, [&](int i) { return sgpr_row_var(i, qn, qn_stride, 0, nb, nullptr, 0, 0, s, nullptr) + add_var; }, mean, y, noise,
+      var_f, var_y, lpd, sums, blk, ticket);
 }
 
 // Posterior draws of one chunk of n rows, CTA = 32 rows x 8 thread rows (scalars s, noise, os_t read from device memory):
@@ -152,6 +178,22 @@ extern "C" int npgp_sgpr_predict_finish(int n, const double* qn, long qn_stride,
   double* blk = sums ? reinterpret_cast<double*>(static_cast<char*>(work) + 256) : nullptr;
   sgpr_predict_finish_kernel<<<ceil_div(n, 256), 256, 0, stream>>>(n, qn, qn_stride, nb_t, nb_s, qv, qv_stride, nb_v, mean, y,
                                                                   s, noise, os_t, var_f, var_y, lpd, sums, blk, ticket);
+  NPGP_LAUNCH_CHECK();
+  return NPGP_OK;
+}
+
+extern "C" int npgp_exact_predict_finish(int n, const double* qn, long qn_stride, int nb, const double* mean, const double* y,
+                                         const double* s, const double* noise, double add_var, double* var_f, double* var_y,
+                                         double* lpd, double* sums, void* work, long work_bytes, cudaStream_t stream) {
+  if (n < 0 || nb < 0) return NPGP_EINVAL;
+  if (n == 0) return NPGP_OK;
+  if (!s || !noise || !var_f || ((lpd || sums) && (!y || !mean))) return NPGP_EINVAL;
+  if (nb > 0 && (!qn || qn_stride < n)) return NPGP_EINVAL;
+  if (sums && (!work || work_bytes < npgp_sgpr_predict_workspace_bytes(n))) return NPGP_EINVAL;
+  unsigned int* ticket = static_cast<unsigned int*>(work);
+  double* blk = sums ? reinterpret_cast<double*>(static_cast<char*>(work) + 256) : nullptr;
+  exact_predict_finish_kernel<<<ceil_div(n, 256), 256, 0, stream>>>(n, qn, qn_stride, nb, mean, y, s, noise, add_var, var_f,
+                                                                   var_y, lpd, sums, blk, ticket);
   NPGP_LAUNCH_CHECK();
   return NPGP_OK;
 }

@@ -72,19 +72,25 @@ class LogNormalPriorProcess(PositivePriorProcess):
     def sample(self, x, **kwargs):
         return torch.exp(self.forward(x).rsample(**kwargs))
 
-    def conditional_sample(self, x, given: Tuple[torch.Tensor, torch.Tensor], **kwargs):
-        """exp(c + K(x, Xg) (K(Xg,Xg) + 1e-4 I)^-1 (log ell_g - c))  (reference :80-100) -> (D, n)."""
-        xg, ell_g = given
-        x, xg = self._active(x), self._active(xg)
+    def conditional_weights(self, xg, ell_g):
+        """alpha (D, m) = (K(Xg,Xg) + 1e-4 I)^-1 (log ell_g - c), per dimension: the weights of the conditional mean given
+        the lengthscales ell_g (D, m) at the (active columns of the) points xg."""
+        xg = self._active(xg)
         c, os, lam = self._hypers()
-        D, m = self.input_dim, xg.shape[0]
-        eye = torch.eye(m, dtype=x.dtype, device=x.device)
+        eye = torch.eye(xg.shape[0], dtype=xg.dtype, device=xg.device)
         alphas = []
-        for b in range(D):
+        for b in range(self.input_dim):
             Kgg = F.rbf_ard(xg, xg, lam[b], os[b]) + 1e-4 * eye
             _, P = F.psd_safe_chol_inv(Kgg)
             alphas.append(F.spd_solve(P, torch.log(ell_g[b]) - c[b]))
-        alpha = torch.stack(alphas).unsqueeze(-1)  # (D, m, 1)
+        return torch.stack(alphas)
+
+    def conditional_sample(self, x, given: Tuple[torch.Tensor, torch.Tensor], **kwargs):
+        """exp(c + K(x, Xg) (K(Xg,Xg) + 1e-4 I)^-1 (log ell_g - c))  (reference :80-100) -> (D, n)."""
+        xg, ell_g = given
+        alpha = self.conditional_weights(xg, ell_g).unsqueeze(-1)  # (D, m, 1)
+        x, xg = self._active(x), self._active(xg)
+        c, os, lam = self._hypers()
         out = F.rbf_matvec(x.contiguous(), xg.contiguous(), lam, os, alpha, c, True)
         return out.squeeze(-1)
 

@@ -4,13 +4,18 @@
   DiagonalSparseGP(train_x, train_y, likelihood, prior, z, num_dim=1)  reference models/nonstationary_models.py:64-153
 
 `forward(x)` returns the prior MultivariateNormal at the training inputs (to be scored by ExactMarginalLogLikelihood),
-`predict(x_new)` the predictive distribution, exactly as in the reference."""
+`predict(x_new)` the predictive distribution, exactly as in the reference, and `posterior()` a snapshot that predicts and
+draws correlated sample fields at any number of rows (sgpr.SGPRPosterior)."""
 from __future__ import annotations
+
+from types import SimpleNamespace
 
 import torch
 
 from .. import functional as F
+from .. import ops
 from ..gp_base import ExactGP, LowRankRootCovar, MultivariateNormal, ZeroMean
+from ..sgpr import SGPRGibbsStream, SGPRPosterior
 from .gibbs_kernels import GibbsKernel, GibbsSafeScaleKernel, InducingGibbsKernel
 
 
@@ -48,6 +53,75 @@ class DiagonalExactGP(ExactGP):
         sigma = K_ss - F.matmul(A, A.T)
         ns = K_ss.shape[-1]
         return MultivariateNormal(mu, sigma + 1e-4 * torch.eye(ns, dtype=x.dtype, device=x.device))
+
+    @torch.no_grad()
+    def posterior(self, *, knots=None) -> SGPRPosterior:
+        """Snapshot of the posterior at the current parameters for prediction and sample fields at any number of rows
+        (sgpr.SGPRPosterior: .predictive(xs, y=None, *, field, chunk), .sample(xs, num_samples, *, seed, noise, row_offset,
+        chunk)); predict() builds n* x n* matrices.  With the unscaled kernel k, outputscale s, noise sigma^2,
+        tau = sigma^2 / s and P_y = chol(K_XX + tau I)^-1 the marginals are those of predict():
+            mean = k^T u,  u = P_y^T P_y y,    var_f = s max(1 - |P_y k|^2, 0) + 1e-4,    var_y = var_f + sigma^2,
+        where k^T (K + tau I)^-1 k < 1, so the clamp changes nothing beyond rounding; the field at new rows is the prior's
+        conditional mean given the training lengthscales, as in predict().
+        The draws are a predictive process on the knots U = [X; knots] (knots (m, D), optional; their lengthscales come from
+        the same field): the collapsed SGPR posterior with inducing set U, which contains the training rows.  With
+        P_U = chol(K_UU + j I)^-1 (j the first of 0, 1e-8, 1e-7, 1e-6 that factors), W = P_U K_UX K_XU P_U^T,
+        B = I + (s / sigma^2) W and V = sqrt(s) chol(B)^-1 P_U,
+            f_s(x) = mean(x) + (V k_U(x))^T e_s + sqrt(s max(1 - |P_U k_U(x)|^2, 0) + 1e-4 [+ sigma^2 if noise]) xi_s(x).
+        With j = 0 each marginal equals var_f; the covariance departs from predict()'s only by the off-diagonal Nystrom
+        residual s (k(x, x') - k_U(x)^T K_UU^-1 k_U(x')), set to zero, which knots make smaller.  The columns are padded to
+        a multiple of 128 (copies of a training row, zero rows and columns in P_y, P_U, V and zeros in u) so that any n takes
+        the int8 digit path (use_i8 = False: the FP64 path); the results do not depend on the padding beyond rounding."""
+        x = self.train_inputs[0]
+        n, D = x.shape
+        prior = self.covar_module.base_kernel.lengthscale_prior
+        if knots is not None and (knots.dim() != 2 or knots.shape[1] != D):
+            raise ValueError("knots must have shape (m, %d) (got %s)" % (D, tuple(knots.shape)))
+        m = 0 if knots is None else knots.shape[0]
+        Wp = -(-(n + m) // 128) * 128
+        if Wp > 16384:
+            raise ValueError("n + m = %d padded to %d exceeds the digit engine's 16384 columns" % (n + m, Wp))
+        f64 = dict(dtype=torch.float64, device=x.device)
+        ell = torch.exp(self.log_ell_train_x)
+        s = self.covar_module.outputscale.reshape(()).clone()
+        noise = self.likelihood.noise.reshape(()).clone()
+        tau = noise / s
+        U, ell_u = x, ell
+        if m:
+            knots = knots.to(**f64).contiguous()
+            U = torch.cat([x, knots])
+            ell_u = torch.cat([ell, prior.conditional_sample(knots, given=(x, ell))], 1)
+        K = F.gibbs_diag(U, ell_u, U, ell_u)
+        eye = torch.eye(n + m, **f64)
+        _, Py = F.psd_safe_chol_inv(K[:n, :n] + tau * eye[:n, :n])
+        u = F.spd_solve(Py, self.train_targets)
+        tau_h = float(tau)
+        for jit in (0.0, 1e-8, 1e-7, 1e-6):  # psd_safe_cholesky ladder, as SGPRGibbsStream._z_side
+            if jit >= tau_h:
+                raise ValueError("K_UU needs jitter %g, not below tau = noise / outputscale = %g" % (jit, tau_h))
+            _, PU, info = F.chol_inv(K + jit * eye if jit else K)
+            if int(info) == 0:
+                break
+        else:
+            raise ValueError("K_UU not positive definite after adding jitter up to 1e-6")
+        G = F.matmul(K[:n], PU.T)  # K_XU P_U^T
+        Bm = eye + (s / noise) * F.matmul(G.T, G)
+        _, PB = F.psd_safe_chol_inv(0.5 * (Bm + Bm.T))
+        V = ops.dgemm(F._aligned(PB), F._aligned(PU), tri_a=1, tri_b=1, out_tri=1, C=torch.zeros_like(PU))
+        V *= torch.sqrt(s)
+
+        def pad(A, rows, cols):
+            out = torch.zeros(rows, cols, **f64)
+            out[:A.shape[0], :A.shape[1]] = A
+            return out
+        up = torch.zeros(Wp, **f64)
+        up[:n] = u
+        c, os_, lam = prior._hypers()
+        cols = SimpleNamespace(Z=torch.cat([U, x[:1].expand(Wp - n - m, D)]), prior_c=c, prior_os=os_, prior_lam=lam)
+        return SGPRPosterior(cols, "exact", P=pad(Py, Wp, Wp), V=pad(V, Wp, Wp), u=up, s=s, noise=noise,
+                             ell_z=torch.cat([ell_u, ell[:, :1].expand(D, Wp - n - m)], 1).contiguous(),
+                             alpha=prior.conditional_weights(x, ell), use_i8=getattr(self, "use_i8", True), field_x=x,
+                             P_draws=pad(PU, Wp, Wp), add_var=1e-4)
 
 
 class DiagonalSparseGP(ExactGP):
@@ -96,3 +170,19 @@ class DiagonalSparseGP(ExactGP):
             test_test = test_test + torch.diag(full_covar.added_diag[n:])
         covar = test_test - F.matmul(L, F.matmul(eye - Binv, L.T))
         return MultivariateNormal(mean, covar)
+
+    @torch.no_grad()
+    def posterior(self) -> SGPRPosterior:
+        """Snapshot of the posterior at the current parameters for prediction and sample fields at any number of rows: the
+        one SGPRGibbsStream.posterior returns for this model's inducing points, lengthscales, outputscale, noise, prior and
+        training data.  Its marginals are those of predict() and its draws are exact samples of predict()'s joint
+        Lr B^-1 Lr^T + diag(clamp(s - |Lr|^2, 0)).  Inducing sets whose size is not a multiple of 128 take the FP64 path."""
+        x, y = self.train_inputs[0], self.train_targets
+        ind = self.covar_module.base_kernel
+        prior = ind.base_kernel.lengthscale_prior
+        c, os_, lam = prior._hypers()
+        stream = SGPRGibbsStream(ind.inducing_points.detach(), self.log_ell_z.detach(), c, os_, lam,
+                                 outputscale=float(self.covar_module.outputscale), noise=float(self.likelihood.noise),
+                                 learn_inducing_locations=False, include_prior=False)
+        stream.use_i8 = getattr(self, "use_i8", True)
+        return stream.posterior(x.contiguous(), y.contiguous())

@@ -391,6 +391,17 @@ def sgpr_predict_finish(qn, nb_t, qv, s, noise, var_f, os_t=None, mean=None, y=N
     return var_f
 
 
+def exact_predict_finish(qn, s, noise, add_var, var_f, mean=None, y=None, var_y=None, lpd=None, sums=None, work=None):
+    """The exact GP's predictive variances (and with y: lpd, accumulated sums) of one chunk from the partials qn of
+    |P_y k|^2: var_f = s max(1 - q, 0) + add_var; see npgp_exact_predict_finish."""
+    n = var_f.shape[0]
+    nbytes = work.numel() if work is not None else 0
+    check(lib().npgp_exact_predict_finish(n, ptr(qn), qn.stride(0), qn.shape[0], ptr(mean), ptr(y), ptr(s), ptr(noise),
+                                          float(add_var), ptr(var_f), ptr(var_y), ptr(lpd), ptr(sums), ptr(work), nbytes,
+                                          stream()), "npgp_exact_predict_finish")
+    return var_f
+
+
 def o8_syrk_part_bytes(n, M):
     return lib().npgp_o8_syrk_part_bytes(n, M)
 

@@ -471,17 +471,26 @@ class SGPRSpatioTemporalStream(torch.nn.Module):
 
 class SGPRPosterior:
     """Snapshot of a streamed SGPR posterior, returned by SGPRGibbsStream.posterior ("diag") and
-    SGPRSpatioTemporalStream.posterior ("st").  It holds copies of everything the predictive and the sampler need (Z, the
-    lengthscale field's interpolation weights, u, P -- as digit planes when the feature width W is a multiple of 128 -- and V
-    in FP64, plus its planes on that path), so later optimiser steps on the model do not change its predictions or draws.
-    V costs 8 W^2 bytes in FP64 (134 MB at W = 4096); sample() needs it to form W^T = E^T V."""
+    SGPRSpatioTemporalStream.posterior ("st"), and of the exact Gibbs GP's posterior, returned by DiagonalExactGP.posterior
+    ("exact").  It holds copies of everything the predictive and the sampler need (Z, the lengthscale field's interpolation
+    weights, u, P -- as digit planes when the feature width W is a multiple of 128 -- and V in FP64, plus its planes on that
+    path), so later optimiser steps on the model do not change its predictions or draws.  V costs 8 W^2 bytes in FP64 (134 MB
+    at W = 4096); sample() needs it to form W^T = E^T V.
 
-    def __init__(self, model, kind, *, P, V, u, s, noise, ell_z, alpha, use_i8, hyp=None, zt=None):
+    The exact kind has the Gibbs columns Z = U (the knots, padded) and in addition: the points field_x the lengthscale field
+    is conditioned on (the training rows; otherwise the field is conditioned on the columns), the factor P_draws whose
+    |P_draws k|^2 gives the residual of the draws (otherwise P), and the variance add_var that its predictive adds to var_f
+    and its draws to the residual.  `model` supplies Z and the prior's hyperparameters prior_c, prior_os, prior_lam."""
+
+    def __init__(self, model, kind, *, P, V, u, s, noise, ell_z, alpha, use_i8, hyp=None, zt=None, field_x=None,
+                 P_draws=None, add_var=0.0):
         self.kind = kind
         self.M = model.Z.shape[0]
-        self.width = P.shape[0]  # M (diag) or 2M (st): the feature columns of a test row
+        self.width = P.shape[0]  # M (diag, exact) or 2M (st): the feature columns of a test row
         self.Z = model.Z.detach().clone()
         self.zs = self.Z[:, 1:3].contiguous() if kind == "st" else self.Z
+        self.field_x = self.zs if field_x is None else field_x.detach().contiguous().clone()
+        self.add_var = float(add_var)
         self.prior_c, self.prior_os, self.prior_lam = (b.detach().clone() for b in
                                                        (model.prior_c, model.prior_os, model.prior_lam))
         self.ell_z, self.alpha, self.u = ell_z.detach().clone(), alpha.detach().clone(), u.detach().contiguous().clone()
@@ -498,9 +507,18 @@ class SGPRPosterior:
                 ops.o8_slice_rows(Mx.contiguous(), 64, d, e)
                 self.planes.append((d, e))
             self.one = torch.ones((), dtype=torch.float64, device=P.device)  # bound of the unscaled Gibbs entries
+            self.draw_planes = self.planes[0]
+            if P_draws is not None:
+                d = torch.empty(ops.digits_bytes(self.width, self.width, 64), dtype=torch.uint8, device=P.device)
+                e = torch.empty(self.width, dtype=torch.int32, device=P.device)
+                ops.o8_slice_rows(P_draws.contiguous(), 64, d, e)
+                self.draw_planes = (d, e)
         else:
             M = self.M
             self.Pblocks = [P[:M, :M].contiguous(), P[M:, M:].contiguous()] if kind == "st" else [P.detach().clone()]
+            self.draw_Pblocks = self.Pblocks if P_draws is None else [P_draws.detach().clone()]
+        if kind == "exact":  # the residual variance the draws add: add_var, and with noise=True the noise as well
+            self.draw_var = [self.noise.new_tensor(self.add_var), self.noise + self.add_var]
 
     def _row_buffers(self, xs, chunk):
         """Buffers of the row pass (_row_chunk) over xs in chunks of up to `chunk` rows, allocated once per call."""
@@ -533,15 +551,16 @@ class SGPRPosterior:
                 b["K"] = torch.empty(rows, M, **f64)
         return b
 
-    def _row_chunk(self, b, lo, nc, mean):
+    def _row_chunk(self, b, lo, nc, mean, draws=False):
         """The part of a chunk of rows lo .. lo + nc that predictive() and sample() share: the lengthscale field, the feature
-        rows k(x) (FP64 and/or digit planes in b), the mean k^T u into `mean` and the partials of |P k|^2 into b["qn"].
-        Returns (ell(x) (D, nc), the FP64 feature rows (nc, W) or None on the diagonal model's digit path)."""
+        rows k(x) (FP64 and/or digit planes in b), the mean k^T u into `mean` and the partials of |P k|^2 into b["qn"] (of
+        |P_draws k|^2 with draws=True).  Returns (ell(x) (D, nc), the FP64 feature rows (nc, W) or None on the Gibbs-only
+        digit path)."""
         st = self.kind == "st"
         M, W, D, qn = self.M, self.width, b["D"], b["qn"]
         ell = b["ell"][:D * nc].view(D, nc, 1)
         xc = b["xs"][lo:lo + nc]
-        ops.rbf_matvec_fwd(xc, self.zs, self.prior_lam, self.prior_os, self.alpha.unsqueeze(-1), bias=self.prior_c,
+        ops.rbf_matvec_fwd(xc, self.field_x, self.prior_lam, self.prior_os, self.alpha.unsqueeze(-1), bias=self.prior_c,
                            apply_exp=True, out=ell)
         ell_x = ell.view(D, nc)
         if st:
@@ -563,11 +582,12 @@ class SGPRPosterior:
             kup = b["ku"][:ops.gibbs_digits_splits(nc, M) * nc].view(-1, nc)
             ops.gibbs_diag_fwd_digits(xc, ell_x, self.Z, self.ell_z, self.one, b["Ad"], u=self.u, Ku_part=kup)
             ops.o8_sum_partials(kup, out=mean)
-            ops.o8_trinorm_digits(nc, M, M, b["Ad"], self.one, *self.planes[0], qn)
+            ops.o8_trinorm_digits(nc, M, M, b["Ad"], self.one, *(self.draw_planes if draws else self.planes[0]), qn)
             return ell_x, None
         K = ops.gibbs_diag_fwd(xc, ell_x, self.Z, self.ell_z, out=b["K"][:nc])
         ops.gemv_n(K, self.u, out=mean)
-        ops.sgpr_rownorm_parts(ops.dgemm(K, self.Pblocks[0], transB=True, tri_b=2, C=b["G"][:nc]), qn)
+        Pk = (self.draw_Pblocks if draws else self.Pblocks)[0]
+        ops.sgpr_rownorm_parts(ops.dgemm(K, Pk, transB=True, tri_b=2, C=b["G"][:nc]), qn)
         return ell_x, K
 
     @torch.no_grad()
@@ -595,22 +615,31 @@ class SGPRPosterior:
             return Predictive(mean, var, var_y, fld, lpd, sums)
         b = self._row_buffers(xs, chunk)
         qn, nb_t = b["qn"], b["nb_t"]
-        qv = torch.empty((W + 63) // 64, b["rows"], **f64)
+        exact = self.kind == "exact"
+        qv = None if exact else torch.empty((W + 63) // 64, b["rows"], **f64)
         work = ops.sgpr_predict_workspace(b["rows"], dev) if y is not None else None
         for lo in range(0, n, chunk):
             nc = min(chunk, n - lo)
             mc = mean[lo:lo + nc]
             ell_x, feats = self._row_chunk(b, lo, nc, mc)
-            if self.digits:
+            if exact:
+                pass  # var_f = s max(1 - |P_y k|^2, 0) + add_var has no V term
+            elif self.digits:
                 ops.o8_trinorm_digits(nc, W, W, b["Ad"], None if st else self.one, *self.planes[1], qv,
                                       a_expo=b["Ae"] if st else None)
             else:
                 ops.sgpr_rownorm_parts(ops.dgemm(feats, self.V, transB=True, tri_b=2, C=b["G"][:nc]), qv)
             if field:
                 fld[:, lo:lo + nc] = ell_x
-            ops.sgpr_predict_finish(qn, nb_t, qv, self.s, self.noise, var[lo:lo + nc], os_t=self.hyp[3:] if st else None,
-                                    mean=mc, y=y[lo:lo + nc] if y is not None else None, var_y=var_y[lo:lo + nc],
-                                    lpd=lpd[lo:lo + nc] if y is not None else None, sums=sums, work=work)
+            yc = y[lo:lo + nc] if y is not None else None
+            lc = lpd[lo:lo + nc] if y is not None else None
+            if exact:
+                ops.exact_predict_finish(qn, self.s, self.noise, self.add_var, var[lo:lo + nc], mean=mc, y=yc,
+                                         var_y=var_y[lo:lo + nc], lpd=lc, sums=sums, work=work)
+            else:
+                ops.sgpr_predict_finish(qn, nb_t, qv, self.s, self.noise, var[lo:lo + nc],
+                                        os_t=self.hyp[3:] if st else None, mean=mc, y=yc, var_y=var_y[lo:lo + nc], lpd=lc,
+                                        sums=sums, work=work)
         return Predictive(mean, var, var_y, fld, lpd, sums)
 
     @torch.no_grad()
@@ -623,6 +652,8 @@ class SGPRPosterior:
             f_s(x) = k(x)^T u + (V k(x))^T e_s + sqrt(r(x)) xi_s(x),   e_s ~ N(0, I_W),  xi_s(x) ~ N(0, 1)
             Cov(f(x), f(x')) = (V k(x))^T (V k(x')) + delta(x, x') r(x),   r(x) = predictive().var - |V k(x)|^2
         with r(x) = [st] max(os_t - |P_t k_t|^2, 0) + s max(1 - |P_s k_s|^2, 0).  noise=True adds the noise variance to r.
+        For the exact kind r(x) = s max(1 - |P_draws k|^2, 0) + add_var and the mean term is the exact GP's mean; see
+        DiagonalExactGP.posterior for the covariance of its draws.
         The mean term is predictive().mean.  Keys as SVGPGibbs.sample: e_s[j] = normal(seed, (s << 32) + j) and xi_s(row) =
         normal(seed, 2^63 + (s << 48) + row_offset + i), so draw s does not depend on num_samples and rows sharded over ranks
         with their global row_offset are parts of one joint draw (up to the rounding of the M x M algebra that posterior()
@@ -653,14 +684,17 @@ class SGPRPosterior:
             ops.o8_slice_rows(Wt, 64, Wd, We)
         mean = torch.empty(b["rows"], **f64)
         Fbuf = torch.empty(b["rows"], Sp, **f64)
+        add_noise, r_add = noise, self.noise
+        if self.kind == "exact":
+            add_noise, r_add = True, self.draw_var[int(bool(noise))]
         for lo in range(0, n, chunk):
             nc = min(chunk, n - lo)
             mc, Fc = mean[:nc], Fbuf[:nc]
-            _, feats = self._row_chunk(b, lo, nc, mc)
+            _, feats = self._row_chunk(b, lo, nc, mc, draws=True)
             if self.digits:
                 ops.o8_gemm_digits(nc, Sp, W, b["Ad"], None if st else self.one, Wd, We, Fc, a_expo=b["Ae"] if st else None)
             else:
                 ops.dgemm(feats, Wt, transB=True, C=Fc)
-            ops.sgpr_sample_finish(mc, b["qn"], b["nb_t"], Fc, S, self.s, self.noise, out[:, lo:lo + nc],
-                                   os_t=self.hyp[3:] if st else None, add_noise=noise, seed=seed, row0=row_offset + lo)
+            ops.sgpr_sample_finish(mc, b["qn"], b["nb_t"], Fc, S, self.s, r_add, out[:, lo:lo + nc],
+                                   os_t=self.hyp[3:] if st else None, add_noise=add_noise, seed=seed, row0=row_offset + lo)
         return out
