@@ -8,6 +8,8 @@ small row of a gradient) is checked at its own scale.  For K the bound is |K - K
 the exponent argument and c = C_PAIR(D) = 8 (D + 2); a gradient entry is bounded by c eps times the sum over the reduced
 axis of |G_ij| |dK_ij/dtheta| (1 + Q_ij), |dK/dtheta| taken term by term, plus the rounding of that sum."""
 import math
+import os
+import re
 
 import mpmath
 import numpy as np
@@ -132,8 +134,34 @@ def check_reduced(got, ref, scale, D, n_red, what, floor=0.0):
     full (their K is exp(-708) times the prefactor instead of ~0), with the same weights as in scale."""
     got = np.asarray(got.detach().cpu().numpy(), dtype=LD)
     tol = (C_PAIR(D) * EPS + sum_slack(n_red)) * scale + floor + SUBNORMAL_SLACK
-    bad = np.abs(got - ref) > tol
+    bad = ~(np.abs(got - ref) <= tol)  # a NaN in got or in the reference fails too
     assert not bad.any(), (what, int(bad.sum()), float((np.abs(got - ref) / np.maximum(tol, 1e-300)).max()))
+
+
+# Forms of the upstream gradient G_ij = rowscale_i T_ij + rowvec_i colvec_j that the backward kernels take: formed in memory,
+# composed inside the kernel (the C step's data term), rowscale only, and the rank-one part alone with G = None (the C
+# step's -beta alpha^T through the lengthscale field's covariance when the prior term is off).  Values: the keyword
+# arguments each form passes.
+G_FORMS = dict(formed=("G",), composed=("T", "rowscale", "rowvec", "colvec"), rowscale=("T", "rowscale"),
+               rankone=("rowvec", "colvec"))
+
+
+def g_form_args(how, G, T, rs, rv, cv):
+    """Keyword arguments of ops().gibbs_*_bwd for one form of G (CUDA tensors; T goes in the G slot)."""
+    t = dict(G=G, T=T, rowscale=rs, rowvec=rv, colvec=cv)
+    return {("G" if k == "T" else k): t[k].cuda() for k in G_FORMS[how]}
+
+
+def g_form_ref(how, T, rs, rv, cv):
+    """(G, |G| term by term) in long double for one form.  The formed G is the FP64 rounding of the composed one: the
+    C_PAIR eps of the bound covers the difference."""
+    T, rs, rv, cv = ld(T), ld(rs), ld(rv), ld(cv)
+    if how == "rankone":
+        T = 0 * T
+    if how == "rowscale":
+        rv = 0 * rv
+    return (rs[:, None] * T + rv[:, None] * cv[None, :],
+            np.abs(rs)[:, None] * np.abs(T) + np.abs(rv)[:, None] * np.abs(cv)[None, :])
 
 
 DIAG_SHAPES = [(1, 1), (33, 257), (300, 1023), (1, 257)]
@@ -158,17 +186,28 @@ def test_gibbs_diag_entrywise_every_dimension(D, n1, n2):
     Kf = np.where(r["Q"] > 700, LD(SCALE) * r["pref"] * LD(EXP_FLOOR), 0)  # pairs past the clamp, in full
     check_reduced(Ku, r["K"] @ ld(u), Kw @ np.abs(ld(u)), D, n2, "K u", floor=Kf @ np.abs(ld(u)))
 
-    # backward: G_ij = rowscale_i T_ij + rowvec_i colvec_j, given formed (G) and composed inside the kernel
+    # backward: G_ij = rowscale_i T_ij + rowvec_i colvec_j, in each of the forms of G_FORMS
     T, rs, rv, cv = torch.randn(n1, n2, generator=g), torch.randn(n1, generator=g), torch.randn(n1, generator=g), torch.randn(n2, generator=g)
     G = rs[:, None] * T + rv[:, None] * cv[None, :]
-    Gl = ld(rs)[:, None] * ld(T) + ld(rv)[:, None] * ld(cv)[None, :]
-    Ga = np.abs(ld(rs))[:, None] * np.abs(ld(T)) + np.abs(ld(rv))[:, None] * np.abs(ld(cv))[None, :]
+    args = (x1.cuda(), e1.cuda(), x2.cuda(), e2.cuda(), s)
+    for how in G_FORMS:
+        res = ops().gibbs_diag_bwd(*args, **g_form_args(how, G, T, rs, rv, cv), need_dx1=True, need_dx2=True, need_dscale=True)
+        want, scale, floor, red = diag_bwd_reference(r, *g_form_ref(how, T, rs, rv, cv))
+        for k in want:
+            check_reduced(res[k], want[k], scale[k], D, red[k], (how, k), floor=floor[k])
+
+
+def diag_bwd_reference(r, Gl, Ga):
+    """Gradients of sum_ij G_ij K_ij for the pieces r of diag_reference and G = Gl, with check_reduced's rounding scale and
+    clamp floor for |G| <= Ga term by term, and the length of each reduction."""
     a, b, S, dl, Kr = r["a"], r["b"], r["S"], r["dl"], r["K"][..., None]
+    n1, n2 = r["K"].shape
     # d log K / d l1 = 1/(2 a) - a/S + 2 a dl^2/S^2 (SURVEY Appendix A.4), same for l2 with b; d log K / d x1 = -2 dl / S
     t_a = [1 / (2 * a) + 0 * b, -a / S, 2 * a * dl * dl / (S * S)]
     t_b = [1 / (2 * b) + 0 * a, -b / S, 2 * b * dl * dl / (S * S)]
     dx = -2 * dl / S
-    Kw, Kf = Kw[..., None], Kf[..., None]
+    Kw = ((1 + r["Q"]) * np.abs(r["K"]))[..., None]                              # weight of the rounding of each pair
+    Kf = np.where(r["Q"] > 700, LD(SCALE) * r["pref"] * LD(EXP_FLOOR), 0)[..., None]  # pairs past the clamp, in full
     want = dict(d_ell1=np.einsum("ij,ijd->di", Gl, Kr * sum(t_a)), d_ell2=np.einsum("ij,ijd->dj", Gl, Kr * sum(t_b)),
                 d_x1=np.einsum("ij,ijd->id", Gl, Kr * dx), d_x2=np.einsum("ij,ijd->jd", Gl, -Kr * dx),
                 d_scale=np.sum(Gl * r["K"]) / LD(SCALE))
@@ -177,13 +216,7 @@ def test_gibbs_diag_entrywise_every_dimension(D, n1, n2):
     scale = {k: np.einsum(e, Ga, Kw * t) for k, (e, t) in absd.items()}
     floor = {k: np.einsum(e, Ga, Kf * t) for k, (e, t) in absd.items()}
     red = dict(d_ell1=n2, d_x1=n2, d_ell2=n1, d_x2=n1, d_scale=n1 * n2)
-    args = (x1.cuda(), e1.cuda(), x2.cuda(), e2.cuda(), s)
-    formed = ops().gibbs_diag_bwd(*args, G=G.cuda(), need_dx1=True, need_dx2=True, need_dscale=True)
-    composed = ops().gibbs_diag_bwd(*args, G=T.cuda(), rowscale=rs.cuda(), rowvec=rv.cuda(), colvec=cv.cuda(), need_dx1=True,
-                                    need_dx2=True, need_dscale=True)
-    for res, how in ((formed, "G"), (composed, "rowscale/rowvec/colvec")):
-        for k in want:
-            check_reduced(res[k], want[k], scale[k], D, red[k], (how, k), floor=floor[k])
+    return want, scale, floor, red
 
 
 # -------------------------------------------------------------------------------------------- 3. full-matrix Gibbs
@@ -211,6 +244,9 @@ def full_inputs(n1, n2, d, seed, near_singular):
         Dm = 0.5 * (Dm + Dm.T)  # D o D must be symmetric
         S1 = o.sigma_from_H(torch.randn(n1, d, generator=g), Dm)
         S2 = o.sigma_from_H(torch.randn(n2, d, generator=g), Dm)
+        for S in (S1, S2):  # with a non-diagonal D a few draws of h (about 1 in 10^4) give an indefinite Sigma: use others
+            pd = torch.linalg.eigvalsh(S)[:, 0] > 0
+            S[~pd] = S[pd][:int((~pd).sum())]
     return x1, S1, x2, S2
 
 
@@ -230,23 +266,78 @@ def _det_inv_ld(A):
 
 
 def full_reference(x1, S1, x2, S2, jitter):
-    """oracle.gibbs_full_K's formulas in long double: prefactor det(S_i)^1/4 det(S_j)^1/4 det(A)^-1/2, Q = dl^T (A + jit I)^-1 dl."""
+    """oracle.gibbs_full_K's formulas in long double: prefactor det(S_i)^1/4 det(S_j)^1/4 det(A)^-1/2, Q = dl^T w with
+    w = (A + jit I)^-1 dl, A = (S_i + S_j)/2; also A^-1 (no jitter), S_i^-1 and S_j^-1 for the backward."""
     d = x1.shape[1]
     S1l, S2l = ld(S1), ld(S2)
     A = LD(0.5) * (S1l[:, None] + S2l[None, :])
-    detA, _ = _det_inv_ld(A)
+    detA, Ainv = _det_inv_ld(A)
     _, inv = _det_inv_ld(A + LD(jitter) * np.eye(d, dtype=LD))
-    det1, _ = _det_inv_ld(S1l)
-    det2, _ = _det_inv_ld(S2l)
+    det1, S1inv = _det_inv_ld(S1l)
+    det2, S2inv = _det_inv_ld(S2l)
     dl = ld(x1)[:, None, :] - ld(x2)[None, :, :]
-    Q = np.einsum("ija,ijab,ijb->ij", dl, inv, dl)
+    w = np.einsum("ijab,ijb->ija", inv, dl)
+    Q = np.einsum("ija,ija->ij", dl, w)
     pref = (det1 ** LD(0.25))[:, None] * (det2 ** LD(0.25))[None, :] / np.sqrt(detA)
     At = (S1[:, None] + S2[None, :]).numpy()
     ev = np.linalg.eigvalsh(At)
     cond = ev[..., -1] / ev[..., 0]
     ev1, ev2 = np.linalg.eigvalsh(S1.numpy()), np.linalg.eigvalsh(S2.numpy())
     cond_s = np.maximum((ev1[:, -1] / ev1[:, 0])[:, None], (ev2[:, -1] / ev2[:, 0])[None, :])
-    return dict(K=LD(SCALE) * pref * np.exp(-Q), Q=Q, pref=pref, cond=np.maximum(cond, cond_s))
+    return dict(K=LD(SCALE) * pref * np.exp(-Q), Q=Q, pref=pref, cond=np.maximum(cond, cond_s), w=w, Ainv=Ainv,
+                S1inv=S1inv, S2inv=S2inv)
+
+
+def check_full_K(K, r, d):
+    """Closed-form determinant and adjugate: relative error <= c eps cond(At); Q inherits it times (1 + Q)."""
+    got = K.cpu().numpy().astype(LD)
+    tol = C_PAIR(d) * EPS * r["cond"] * (1 + r["Q"]) * np.abs(r["K"]) + SUBNORMAL_SLACK
+    tail = r["Q"] > 707.0
+    ok = (np.abs(got - r["K"]) <= tol) | (tail & (got >= 0) & (got <= LD(SCALE) * r["pref"] * LD(EXP_FLOOR) * 1.0001))
+    assert ok.all(), (int((~ok).sum()), float((np.abs(got - r["K"]) / tol).max()))
+
+
+def full_bwd_reference(r, Gl, Ga):
+    """Gradients of sum_ij G_ij K_ij for the pieces r of full_reference and G = Gl, as the kernel returns them (entries of
+    the symmetric matrix dL/dSigma, packed upper), with g_ij = G_ij K_ij:
+        dL/dS_i = sum_j g_ij (1/4 S_i^-1 - 1/4 A_ij^-1 + 1/2 w_ij w_ij^T),  dL/dS_j likewise with S_j^-1,
+        dL/dx_i = -2 sum_j g_ij w_ij,  dL/dx_j = 2 sum_i g_ij w_ij,  dL/ds = sum_ij g_ij / s;
+    and check_reduced's rounding scale (the same sums of absolute terms with |G| <= Ga and the forward's weight
+    cond (1 + Q) |K|) and clamp floor, and the length of each reduction."""
+    d = r["w"].shape[-1]
+    n1, n2 = r["K"].shape
+    iu = np.triu_indices(d)
+    pk = lambda M: M[..., iu[0], iu[1]]
+    w = r["w"]
+    ww, Ai = pk(w[..., :, None] * w[..., None, :]), pk(r["Ainv"])
+    s1, s2 = LD(0.25) * pk(r["S1inv"]), LD(0.25) * pk(r["S2inv"])
+
+    def sums(g, pair, s1, s2, w):
+        return dict(d_S1=np.einsum("ij,ijp->ip", g, pair) + s1 * g.sum(1)[:, None],
+                    d_S2=np.einsum("ij,ijp->jp", g, pair) + s2 * g.sum(0)[:, None],
+                    d_x1=-2 * np.einsum("ij,ija->ia", g, w), d_x2=2 * np.einsum("ij,ija->ja", g, w), d_scale=g.sum() / LD(SCALE))
+
+    want = sums(Gl * r["K"], LD(0.5) * ww - LD(0.25) * Ai, s1, s2, w)
+    pair_abs = LD(0.5) * np.abs(ww) + LD(0.25) * np.abs(Ai)
+    weight = r["cond"] * (1 + r["Q"]) * np.abs(r["K"])
+    clamp = np.where(r["Q"] > 700, LD(SCALE) * r["pref"] * LD(EXP_FLOOR), 0)
+    scale = {k: np.abs(v) for k, v in sums(Ga * weight, pair_abs, np.abs(s1), np.abs(s2), np.abs(w)).items()}
+    floor = {k: np.abs(v) for k, v in sums(Ga * clamp, pair_abs, np.abs(s1), np.abs(s2), np.abs(w)).items()}
+    red = dict(d_S1=n2, d_x1=n2, d_S2=n1, d_x2=n1, d_scale=n1 * n2)
+    return want, scale, floor, red
+
+
+def full_case(n1, n2, d, near_singular, seed):
+    x1, S1, x2, S2 = full_inputs(n1, n2, d, seed=seed, near_singular=near_singular)
+    if near_singular:
+        x1 = x1 * 2e-3  # keep Q moderate along the nearly flat direction
+        x2 = x2 * 2e-3
+    return x1, S1, x2, S2
+
+
+def full_args(x1, S1, x2, S2, jitter):
+    return (x1.cuda(), ops().sym_pack(S1.cuda()), x2.cuda(), ops().sym_pack(S2.cuda()), jitter,
+            torch.tensor(SCALE).cuda())
 
 
 @pytest.mark.parametrize("d", [2, 3])
@@ -254,21 +345,223 @@ def full_reference(x1, S1, x2, S2, jitter):
 @pytest.mark.parametrize("jitter", [1e-5, 1e-3, 0.0])
 def test_gibbs_full_entrywise_conditioning(d, near_singular, jitter):
     n1, n2 = 65, 300
-    x1, S1, x2, S2 = full_inputs(n1, n2, d, seed=10 * d + int(near_singular), near_singular=near_singular)
-    if near_singular:
-        x1 = x1 * 2e-3  # keep Q moderate along the nearly flat direction
-        x2 = x2 * 2e-3
+    x1, S1, x2, S2 = full_case(n1, n2, d, near_singular, seed=10 * d + int(near_singular))
     r = full_reference(x1, S1, x2, S2, jitter)
     if near_singular:
         assert r["cond"].max() > 1e7
+    check_full_K(ops().gibbs_full_fwd(*full_args(x1, S1, x2, S2, jitter)), r, d)
+
+
+def full_bwd_problem(n1, n2, d, near_singular, jitter, seed):
+    """full_case with its reference and an upstream gradient (T, rowscale, rowvec, colvec) and its formed G."""
+    x1, S1, x2, S2 = full_case(n1, n2, d, near_singular, seed)
+    r = full_reference(x1, S1, x2, S2, jitter)
+    g = torch.Generator().manual_seed(seed + 1000)
+    T, rs, rv, cv = torch.randn(n1, n2, generator=g), torch.randn(n1, generator=g), torch.randn(n1, generator=g), torch.randn(n2, generator=g)
+    return (x1, S1, x2, S2), r, (rs[:, None] * T + rv[:, None] * cv[None, :], T, rs, rv, cv)
+
+
+def check_full_bwd(res, r, how, T, rs, rv, cv, d):
+    want, scale, floor, red = full_bwd_reference(r, *g_form_ref(how, T, rs, rv, cv))
+    for k in want:
+        if res[k] is not None:
+            check_reduced(res[k], want[k], scale[k], d, red[k], (how, k), floor=floor[k])
+
+
+@pytest.mark.parametrize("d", [2, 3])
+@pytest.mark.parametrize("near_singular", [False, True])
+@pytest.mark.parametrize("jitter,n1,n2", [(1e-5, 65, 300), (1e-3, 65, 300), (0.0, 65, 300), (1e-5, 1, 1), (1e-5, 33, 257)])
+def test_gibbs_full_bwd_entrywise(d, near_singular, jitter, n1, n2):
+    """All five outputs of the full-matrix backward, every entry at its own scale, for each form of G; the same inputs as
+    the forward test above (near-singular Sigmas: cond(At) up to ~1e8)."""
+    xs, r, (G, T, rs, rv, cv) = full_bwd_problem(n1, n2, d, near_singular, jitter, seed=10 * d + int(near_singular))
+    args = full_args(*xs, jitter)
+    for how in G_FORMS:
+        res = ops().gibbs_full_bwd(*args, **g_form_args(how, G, T, rs, rv, cv), need_dx1=True, need_dx2=True, need_dscale=True)
+        assert all(res[k] is not None for k in ("d_x1", "d_x2", "d_scale"))
+        check_full_bwd(res, r, how, T, rs, rv, cv, d)
+
+
+@pytest.mark.parametrize("d", [2, 3])
+def test_gibbs_full_bwd_every_instantiation_and_unaligned_G(d):
+    """The four (d_x1, d_x2) instantiations of the kernel, each with and without d_scale (the C step's data term requests
+    d_x2 only, and nothing but d_S when the inducing points are frozen); then a formed G that starts 8 bytes past a 16-byte
+    boundary, with an odd row length: the launcher has to pick the scalar G loads by itself."""
+    n1, n2 = 33, 257
+    xs, r, (G, T, rs, rv, cv) = full_bwd_problem(n1, n2, d, False, 1e-5, seed=50 + d)
+    args = full_args(*xs, 1e-5)
+    for dx1 in (False, True):
+        for dx2 in (False, True):
+            for dscale in (False, True):
+                res = ops().gibbs_full_bwd(*args, **g_form_args("composed", G, T, rs, rv, cv), need_dx1=dx1, need_dx2=dx2,
+                                           need_dscale=dscale)
+                assert [res[k] is not None for k in ("d_x1", "d_x2", "d_scale")] == [dx1, dx2, dscale]
+                check_full_bwd(res, r, "composed", T, rs, rv, cv, d)
+    buf = torch.empty(n1 * n2 + 1).cuda()
+    Gu = buf[1:].view(n1, n2)
+    Gu.copy_(G.cuda())
+    assert Gu.data_ptr() % 16 == 8 and Gu.is_contiguous()
+    res = ops().gibbs_full_bwd(*args, G=Gu, need_dx1=True, need_dx2=True, need_dscale=True)
+    check_full_bwd(res, r, "formed", T, rs, rv, cv, d)
+
+
+@pytest.mark.parametrize("kind", ["full", "diag"])
+def test_gibbs_bwd_aliased_self_pair(kind):
+    """The Kzz backward of the C step and of the DSVI layer: K(Z, Z) with one x and one Sigma / lengthscale buffer on both
+    sides and one d_Sigma / d_ell and one d_x buffer in both output slots, so that every entry gathers its row and its
+    column sums.  M = 1024: the step's 4 column tiles.  The reference is the sum of the two slots' reference gradients."""
+    from nonstationary_precip_b200._lib import check, lib, ptr, stream
+    M, d, jitter = 1024, 3, 1e-5
+    g = torch.Generator().manual_seed(61)
+    R = torch.randn(M, M, generator=g)
+    G = 0.5 * (R + R.T)
+    Gl, Gc = ld(G), G.cuda()
     s = torch.tensor(SCALE, device="cuda")
-    K = ops().gibbs_full_fwd(x1.cuda(), ops().sym_pack(S1.cuda()), x2.cuda(), ops().sym_pack(S2.cuda()), jitter, s)
-    # closed-form determinant and adjugate: relative error <= c eps cond(At); Q inherits it times (1 + Q)
-    got = K.cpu().numpy().astype(LD)
-    tol = C_PAIR(d) * EPS * r["cond"] * (1 + r["Q"]) * np.abs(r["K"]) + SUBNORMAL_SLACK
-    tail = r["Q"] > 707.0
-    ok = (np.abs(got - r["K"]) <= tol) | (tail & (got >= 0) & (got <= LD(SCALE) * r["pref"] * LD(EXP_FLOOR) * 1.0001))
-    assert ok.all(), (int((~ok).sum()), float((np.abs(got - r["K"]) / tol).max()))
+    ds = torch.zeros((), device="cuda")
+    if kind == "full":
+        x, S, _, _ = full_inputs(M, 1, d, seed=62, near_singular=False)
+        Sp = ops().sym_pack(S.cuda())
+        dS, dx = torch.zeros(M, d * (d + 1) // 2, device="cuda"), torch.zeros(M, d, device="cuda")
+        xc = x.cuda()
+        check(lib().npgp_gibbs_full_bwd(d, M, M, ptr(xc), ptr(Sp), ptr(xc), ptr(Sp), jitter, ptr(s), ptr(Gc), M, None,
+                                        None, None, ptr(dS), ptr(dx), ptr(dS), ptr(dx), ptr(ds), stream()), "npgp_gibbs_full_bwd")
+        want, scale, floor, _ = full_bwd_reference(full_reference(x, S, x, S, jitter), Gl, np.abs(Gl))
+        pairs = dict(d_S=(dS, "d_S1", "d_S2"), d_x=(dx, "d_x1", "d_x2"))
+    else:
+        x, e, _, _ = diag_inputs(M, 1, d, seed=63)
+        xc, ec = x.cuda(), e.cuda()
+        de, dx = torch.zeros(d, M, device="cuda"), torch.zeros(M, d, device="cuda")
+        check(lib().npgp_gibbs_diag_bwd(d, M, M, ptr(xc), ptr(ec), ptr(xc), ptr(ec), ptr(s), ptr(Gc), M, None, None,
+                                        None, ptr(de), ptr(dx), ptr(de), ptr(dx), ptr(ds), stream()), "npgp_gibbs_diag_bwd")
+        want, scale, floor, _ = diag_bwd_reference(diag_reference(x, e, x, e), Gl, np.abs(Gl))
+        pairs = dict(d_ell=(de, "d_ell1", "d_ell2"), d_x=(dx, "d_x1", "d_x2"))
+    for name, (got, a, b) in pairs.items():
+        check_reduced(got, want[a] + want[b], scale[a] + scale[b], d, 2 * M, name, floor=floor[a] + floor[b])
+    check_reduced(ds, want["d_scale"], scale["d_scale"], d, M * M, "d_scale", floor=floor["d_scale"])
+
+
+# ---- both Gibbs kernels at the benchmark's shape: several staged chunks of kTI rows per CTA
+BENCH_N1, BENCH_N2 = 65536, 1024  # B and M of the 1-GPU benchmark (BASELINE config 2)
+
+
+def _csrc(name):
+    with open(os.path.join(os.path.dirname(__file__), "..", "nonstationary_precip_b200", "csrc", name)) as f:
+        return f.read()
+
+
+def rows_per_cta(n1, col_tiles, waves_target):
+    """pick_rows_per_cta of csrc/common.cuh, with its constants read from the source."""
+    common = _csrc("common.cuh")
+    sms = int(re.search(r"kNumSMs\s*=\s*(\d+)", common).group(1))
+    kti = int(re.search(r"kTI\s*=\s*(\d+)", common).group(1))
+    row_ctas = -(-sms * waves_target // col_tiles)
+    rpc = -(-n1 // row_ctas)
+    return max(kti, -(-rpc // kti) * kti), kti
+
+
+def launch_waves(src):
+    """Wave targets (forward, backward) that gibbs_{full,diag}.cu pass to pick_rows_per_cta."""
+    waves = [int(w) for w in re.findall(r"pick_rows_per_cta\(n1, col_tiles, (\d+)\)", _csrc(src))]
+    assert len(waves) == 2, "expected one forward and one backward launcher"
+    return waves
+
+
+def bench_split(kind, n1, n2):
+    """((forward rows per CTA, kTI), (backward rows per CTA, kTI)) of gibbs_{kind}.cu at n1 x n2: both launchers tile the
+    columns 256 at a time (128 threads x 2 columns)."""
+    return [rows_per_cta(n1, -(-n2 // 256), w) for w in launch_waves("gibbs_%s.cu" % kind)]
+
+
+def bench_rows(n1, fwd_rpc, bwd_rpc, kti, seed):
+    """First and last row of every CTA under both splits, both sides of every chunk boundary inside three CTAs of each
+    split (first, middle, last full one), the whole ragged last CTA, and random rows."""
+    rows = set()
+    for rpc in (fwd_rpc, bwd_rpc):
+        starts = list(range(0, n1, rpc))
+        for r0 in starts:
+            rows |= {r0, min(r0 + rpc, n1) - 1}
+        full = [r0 for r0 in starts if r0 + rpc <= n1]
+        for r0 in (full[0], full[len(full) // 2], full[-1]):
+            for c in range(kti, rpc, kti):
+                rows |= {r0 + c - 1, r0 + c}
+        rows |= set(range(starts[-1], n1))
+    rows |= set(np.random.default_rng(seed).choice(n1, 64, replace=False).tolist())
+    return torch.tensor(sorted(rows))
+
+
+def bench_cols(n2, seed):
+    fixed = [0, 1, 254, 255, 256, 257, 511, 512, n2 - 2, n2 - 1]
+    rest = np.setdiff1d(np.arange(n2), fixed)
+    return torch.tensor(sorted(fixed + np.random.default_rng(seed).choice(rest, 6, replace=False).tolist()))
+
+
+def check_bench_shape(kind, n1, n2):
+    """Forward (K entry by entry on the sampled rows, all columns, and K u) and the backward as the C step calls it
+    (composed G, d_x2 and d_scale, no d_x1; then once more with d_x1): row outputs on the sampled rows, whose reference runs
+    over the whole row, column outputs on the sampled columns, whose reference runs over all n1 rows, and d_scale against
+    an FP64 sum of G o K with the kernel's own K (pinned entry by entry on the sampled rows)."""
+    D, jitter = 3, 1e-5
+    full = kind == "full"
+    g = torch.Generator().manual_seed(7)
+    if full:
+        x1, S1, x2, S2 = full_inputs(n1, n2, D, seed=81, near_singular=False)
+        args = full_args(x1, S1, x2, S2, jitter)
+        fwd, bwd = ops().gibbs_full_fwd, ops().gibbs_full_bwd
+        ref = lambda rows, cols: full_reference(x1[rows], S1[rows], x2[cols], S2[cols], jitter)
+        bwd_ref, check_k = full_bwd_reference, lambda K, r: check_full_K(K, r, D)
+        row_keys, col_keys = ("d_S1", "d_x1"), ("d_S2", "d_x2")
+        pick = dict(d_S1=lambda t, i: t[i], d_x1=lambda t, i: t[i], d_S2=lambda t, j: t[j], d_x2=lambda t, j: t[j])
+    else:
+        x1, e1, x2, e2 = diag_inputs(n1, n2, D, seed=82)
+        args = (x1.cuda(), e1.cuda(), x2.cuda(), e2.cuda(), torch.tensor(SCALE).cuda())
+        fwd, bwd = ops().gibbs_diag_fwd, ops().gibbs_diag_bwd
+        ref = lambda rows, cols: diag_reference(x1[rows], e1[:, rows], x2[cols], e2[:, cols])
+        bwd_ref, check_k = diag_bwd_reference, lambda K, r: check_K(K, r, D)
+        row_keys, col_keys = ("d_ell1", "d_x1"), ("d_ell2", "d_x2")
+        pick = dict(d_ell1=lambda t, i: t[:, i], d_x1=lambda t, i: t[i], d_ell2=lambda t, j: t[:, j], d_x2=lambda t, j: t[j])
+    (fwd_rpc, kti), (bwd_rpc, _) = bench_split(kind, n1, n2)
+    rows, cols = bench_rows(n1, fwd_rpc, bwd_rpc, kti, seed=5), bench_cols(n2, seed=6)
+    u = torch.randn(n2, generator=g)
+    T, rs, rv, cv = torch.randn(n1, n2, generator=g), torch.randn(n1, generator=g), torch.randn(n1, generator=g), torch.randn(n2, generator=g)
+
+    # forward
+    K, Ku = fwd(*args, u=u.cuda())
+    rr = ref(rows, torch.arange(n2))
+    check_k(K[rows.cuda()], rr)
+    weight = (rr["cond"] if full else 1) * (1 + rr["Q"]) * np.abs(rr["K"])
+    clamp = np.where(rr["Q"] > 700, LD(SCALE) * rr["pref"] * LD(EXP_FLOOR), 0)
+    check_reduced(Ku[rows.cuda()], rr["K"] @ ld(u), weight @ np.abs(ld(u)), D, n2, "K u", floor=clamp @ np.abs(ld(u)))
+
+    # backward, C-step form
+    Tc, rsc, rvc, cvc = T.cuda(), rs.cuda(), rv.cuda(), cv.cuda()
+    gabs = (rsc.abs()[:, None] * Tc.abs() + rvc.abs()[:, None] * cvc.abs()[None, :]) * K.abs()
+    want_ds = ((rsc[:, None] * Tc + rvc[:, None] * cvc[None, :]) * K).sum() / SCALE
+    scale_ds = gabs.sum().item() / SCALE
+    del gabs
+    rc = ref(torch.arange(n1), cols)
+    want_r, scale_r, floor_r, red_r = bwd_ref(rr, *g_form_ref("composed", T[rows], rs[rows], rv[rows], cv))
+    want_c, scale_c, floor_c, red_c = bwd_ref(rc, *g_form_ref("composed", T[:, cols], rs, rv, cv[cols]))
+    for dx1 in (False, True):
+        res = bwd(*args, G=Tc, rowscale=rsc, rowvec=rvc, colvec=cvc, need_dx1=dx1, need_dx2=True, need_dscale=True)
+        assert (res["d_x1"] is not None) == dx1
+        for k in row_keys:
+            if res[k] is not None:
+                check_reduced(pick[k](res[k], rows.cuda()), want_r[k], scale_r[k], D, red_r[k], ("rows", dx1, k), floor=floor_r[k])
+        for k in col_keys:
+            check_reduced(pick[k](res[k], cols.cuda()), want_c[k], scale_c[k], D, red_c[k], ("cols", dx1, k), floor=floor_c[k])
+        tol = (C_PAIR(D) * EPS + sum_slack(n1 * n2)) * scale_ds
+        assert abs(res["d_scale"].item() - want_ds.item()) <= tol, ("d_scale", dx1)
+
+
+@pytest.mark.parametrize("kind", ["full", "diag"])
+def test_gibbs_bench_shape_every_cta_and_chunk(kind):
+    """n1 = 65536 rows against n2 = 1024 columns, the shape of the benchmark's step: pick_rows_per_cta gives each CTA 128
+    rows in the forward and 224 in the backward, so the chunk loop, the G prefetch queue across chunk boundaries and the
+    row reducer's flushes of later chunks all run, and the last backward CTA is ragged.  No smaller test reaches past the
+    first chunk."""
+    (fwd_rpc, kti), (bwd_rpc, _) = bench_split(kind, BENCH_N1, BENCH_N2)
+    assert fwd_rpc > kti and bwd_rpc > kti, "the benchmark's shape no longer runs several chunks per CTA"
+    check_bench_shape(kind, BENCH_N1, BENCH_N2)
 
 
 @pytest.mark.parametrize("d", [2, 3])

@@ -52,10 +52,19 @@ def test_c_step_options(variant, opts):
     mc, x, y, Z, p, N = build(variant, "c", B=400, M=128, d=3, seed=2, **opts)
     mp, *_ = build(variant, "python", B=400, M=128, d=3, seed=2, **opts)
     lc, lp = mc.loss_and_grad(x, y, world_size=2), mp.loss_and_grad(x, y, world_size=2)
+    frozen_z = opts.get("learn_inducing_locations") is False
+    # this rank's share with B_global = 2 B and the replicated terms weighted 1/2 is half the one-rank -ELBO of (x, y)
+    want_loss, want = oracle_loss_and_grads(variant, x, y, Z, p, N, include_prior=opts.get("include_prior", True),
+                                            learn_z=not frozen_z)
+    assert abs(2 * lc.item() - want_loss.item()) < 1e-9 * abs(want_loss.item())
+    for name, gw in want.items():
+        if name == "Z" and frozen_z:
+            continue  # frozen by the Adam mask; the engines need not agree on the unused slot
+        assert rel(2 * mc.g[name], gw) < 1e-6, name  # the north-star bound of the test above
     assert abs(lc.item() - lp.item()) < 1e-8 * abs(lp.item())
     for name in mp.g:
-        if name == "Z" and opts.get("learn_inducing_locations") is False:
-            continue  # frozen by the Adam mask; the engines need not agree on the unused slot
+        if name == "Z" and frozen_z:
+            continue
         assert rel(mc.g[name], mp.g[name]) < 1e-7, name  # FP64 atomics in both engines; the oracle bound above is the parity claim
 
 
