@@ -1,9 +1,9 @@
 /* npgp -- C ABI of the B200-native non-stationary (Gibbs) GP hot path.
  *
  * Every entry point takes raw DEVICE pointers (fp64, row-major), explicit sizes / leading dimensions and the CUDA
- * stream to run on; nothing allocates device memory, nothing synchronises.  The only process-global state are three
- * measurement / debugging switches (npgp_set_gemm_config, npgp_o8_set_collector, npgp_rowquad_i8_debug), the diagnostic launch
- * counter and the lazily resolved driver / NCCL entry points; none of them affects results.  Return value:
+ * stream to run on; nothing allocates device memory, nothing synchronises.  The only process-global state are the debugging
+ * switch npgp_rowquad_i8_debug, the diagnostic launch counter and the lazily resolved driver / NCCL entry points; none of
+ * them affects results.  Return value:
  * 0 = ok, < 0 = argument error (NPGP_E*), > 0 = a cudaError_t from the launch.  All calls are asynchronous.
  * Outputs documented as "accumulated" are added to with atomics and must be zeroed by the caller.
  *
@@ -104,9 +104,6 @@ int npgp_symmetrize(int M, double* C, long ldc, int from_upper, npgp_stream_t st
  * (models/gibbs_kernels.py:205-208,222-225).  B, X (M,k). */
 int npgp_trsm(int trans, int M, int k, const double* P, long ldp, const double* B, long ldb, double* X, long ldx,
               npgp_stream_t stream);
-/* measurement switch for the GEMM family: 0 = 128x128 tiles (1 CTA/SM), 1/2 = 128x64 (2 CTAs/SM), 3/4 = 64x64 tiles with
- * 4-warp CTAs (3/4 CTAs/SM), 5 = auto (default) */
-int npgp_set_gemm_config(int cfg);
 
 /* ---- (c) blocked Cholesky + inverse factor --------------------------------------------------------------------------
  * A = L L^T in place (upper zeroed), P = L^-1; *info = 0 or 1-based index of the first non-positive pivot.
@@ -212,10 +209,6 @@ int npgp_rbfper_bwd(int n1, int n2, const double* t1, const double* t2, const do
  * T 16-byte aligned with even ldt.  work: the *_workspace_bytes(n, M) bytes of device memory (digit planes, exponents,
  * SYRK chunk partials).  The SYRK adds its row chunks in a fixed order: bitwise reproducible. */
 long npgp_rowquad_i8_workspace_bytes(int n, int M);
-int npgp_rowquad_i8_gemm_only(int n, int M, const double* K, long ldk, double* T, long ldt, double* q, void* work,
-                              long work_bytes, npgp_stream_t stream); /* measurement helper: GEMM on the planes left in work */
-int npgp_rowquad_i8_slice_only(int n, int M, const double* K, long ldk, const double* C, long ldc, void* work,
-                               long work_bytes, npgp_stream_t stream); /* slicing passes only; then ..._gemm_only */
 void npgp_rowquad_i8_debug(long long* dev_counters); /* debugging aid: 8 cycle counters written by CTA 0 (NULL = off) */
 int npgp_rowquad_i8(int n, int M, const double* K, long ldk, const double* C, long ldc, double* T, long ldt, double* q,
                     void* work, long work_bytes, npgp_stream_t stream);
@@ -225,10 +218,8 @@ int npgp_rowquad_i8(int n, int M, const double* K, long ldk, const double* C, lo
  * when the weights are NOT all equal, else untouched. */
 long npgp_syrk_i8_workspace_bytes(int n, int M);
 int npgp_syrk_i8(int n, int M, double alpha, const double* K, long ldk, const double* w0_dev, const double* uniform_count,
-                 double uniform_target, int accumulate, int phase, double* Out, long ldo, void* work, long work_bytes,
-                 npgp_stream_t stream); /* phase: 0 slice + run, 1 slicing passes only, 2 run on the planes left in work */
-int npgp_syrk_i8_prepare(int n, int M, const double* K, long ldk, const double* w, double* wsum, void* work,
-                         long work_bytes, npgp_stream_t stream); /* phase 1 + fused wsum[j] = sum_i w_i K_ij (w, wsum may be NULL) */
+                 double uniform_target, int accumulate, double* Out, long ldo, void* work, long work_bytes,
+                 npgp_stream_t stream);
 int npgp_wsyrk_weighted_only(int n, int M, double alpha, const double* K, long ldk, const double* w,
                              const double* uniform_count, double uniform_target, double* Out, long ldo,
                              npgp_stream_t stream);
@@ -281,8 +272,6 @@ long npgp_o8_syrk_part_bytes(int n, int M);
 int npgp_o8_syrk_digits(int n, int M, const void* x_digits, const double* x_scale, double alpha, const double* w0_dev,
                         const int* skip_count, const int* skip_rows, int accumulate, double* Out, long ldo, void* part,
                         long part_bytes, npgp_stream_t stream);
-int npgp_o8_set_collector(int on); /* measurement switch: A-operand collector reuse hints (default 1) */
-int npgp_o8_set_syrk_split(int on); /* measurement switch: split the SYRK's last partial wave evenly over the CTAs (default 1) */
 
 /* Deterministic (two-stage, fixed order) variants of the ELBO reductions used with the digit-plane path. */
 int npgp_mu_gmu_parts(int n, const double* y, const double* mu_part, int nparts, long stride, const double* noise,

@@ -44,15 +44,10 @@ _SIGS = {
     "npgp_rowquad": ([_i, _i, _p, _l, _p, _l, _p, _l, _p, _p], _i),
     "npgp_rowquad_i8_workspace_bytes": ([_i, _i], _l),
     "npgp_rowquad_i8_debug": ([_p], None),
-    "npgp_rowquad_i8_slice_only": ([_i, _i, _p, _l, _p, _l, _p, _l, _p], _i),
-    "npgp_rowquad_i8_gemm_only": ([_i, _i, _p, _l, _p, _l, _p, _p, _l, _p], _i),
     "npgp_syrk_i8_workspace_bytes": ([_i, _i], _l),
-    "npgp_syrk_i8": ([_i, _i, _d, _p, _l, _p, _p, _d, _i, _i, _p, _l, _p, _l, _p], _i),
-    "npgp_syrk_i8_prepare": ([_i, _i, _p, _l, _p, _p, _p, _l, _p], _i),
+    "npgp_syrk_i8": ([_i, _i, _d, _p, _l, _p, _p, _d, _i, _p, _l, _p, _l, _p], _i),
     "npgp_wsyrk_weighted_only": ([_i, _i, _d, _p, _l, _p, _p, _d, _p, _l, _p], _i),
     "npgp_rowquad_i8": ([_i, _i, _p, _l, _p, _l, _p, _l, _p, _p, _l, _p], _i),
-    "npgp_o8_set_collector": ([_i], _i),
-    "npgp_o8_set_syrk_split": ([_i], _i),
     "npgp_o8_digits_bytes": ([_i, _i, _i], _l),
     "npgp_o8_slice_rows": ([_i, _i, _p, _l, _i, _p, _p, _p], _i),
     "npgp_o8_rowquad_digits": ([_i, _i, _p, _p, _p, _p, _p, _p, _l, _p, _l, _p, _l, _p, _p, _p], _i),
@@ -79,7 +74,6 @@ _SIGS = {
     "npgp_fp64_peak_probe": ([_i, _i, _i, _p, _p], _i),
     "npgp_i8_peak_probe": ([_i, _i, _i, _i, _p], _i),
     "npgp_i8_peak_probe_pair": ([_i, _i, _i, _i, _p], _i),
-    "npgp_set_gemm_config": ([_i], _i),
     "npgp_colwsum": ([_i, _i, _p, _l, _p, _p, _p], _i),
     "npgp_gemv_n": ([_i, _i, _p, _l, _p, _p, _p], _i),
     "npgp_gauss_ell": ([_i, _p, _p, _p, _p, _d, _d, _p, _d, _p, _p, _p, _p, _p], _i),
@@ -149,8 +143,6 @@ def lib():
             fn = getattr(handle, name)
             fn.argtypes = argtypes
             fn.restype = restype
-        if os.environ.get("NPGP_O8_COLLECTOR") == "0":  # measurement / debugging switch (see npgp_o8_set_collector)
-            handle.npgp_o8_set_collector(0)
         _lib = handle
     return _lib
 

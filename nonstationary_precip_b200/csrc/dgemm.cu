@@ -278,10 +278,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, MINB) dgemm_kernel(GemmParams p)
   }
 }
 
-// tile configurations (switchable at run time for A/B measurements, see npgp_set_gemm_config)
-struct Cfg0 { static constexpr int BM = 128, BN = 128, WM = 64, WN = 32, BK = 16, ST = 3, MINB = 1, NT = 256; };  // 1 CTA/SM
-struct Cfg1 { static constexpr int BM = 128, BN = 64, WM = 32, WN = 32, BK = 16, ST = 3, MINB = 2, NT = 256; };   // 2 CTAs/SM
-struct Cfg2 { static constexpr int BM = 128, BN = 64, WM = 32, WN = 32, BK = 32, ST = 2, MINB = 2, NT = 256; };
+// tile configurations: 64x64 tiles of 4 warps; Cfg4 for tall problems (M N > 4096^2 or K > 8192), Cfg3 for the others
 struct Cfg3 { static constexpr int BM = 64, BN = 64, WM = 32, WN = 32, BK = 16, ST = 3, MINB = 3, NT = 128; };     // 3 CTAs/SM
 struct Cfg4 { static constexpr int BM = 64, BN = 64, WM = 32, WN = 32, BK = 16, ST = 3, MINB = 4, NT = 128; };     // 4 CTAs/SM
 
@@ -334,8 +331,6 @@ static int launch_cfg(const GemmParams& p, cudaStream_t st) {
   return NPGP_OK;
 }
 
-static int g_gemm_cfg = 5;  // 5 = auto: 64x64 tiles, 4 CTAs/SM for tall problems, 3 CTAs/SM for M x M ones
-
 template <class Cfg>
 static int launch_layout(bool a_kc, bool b_kc, const GemmParams& p, cudaStream_t st) {
   if (a_kc && b_kc) return launch_cfg<Cfg, true, true>(p, st);
@@ -345,23 +340,14 @@ static int launch_layout(bool a_kc, bool b_kc, const GemmParams& p, cudaStream_t
 }
 
 static int launch_gemm(bool a_kc, bool b_kc, const GemmParams& p, cudaStream_t st) {
-  switch (g_gemm_cfg) {
-    case 5:
-      if ((long)p.M * p.N > (4096L * 4096L) || p.K > 8192) return launch_layout<Cfg4>(a_kc, b_kc, p, st);
-      return launch_layout<Cfg3>(a_kc, b_kc, p, st);
-    case 0: return launch_layout<Cfg0>(a_kc, b_kc, p, st);
-    case 2: return launch_layout<Cfg2>(a_kc, b_kc, p, st);
-    case 3: return launch_layout<Cfg3>(a_kc, b_kc, p, st);
-    case 4: return launch_layout<Cfg4>(a_kc, b_kc, p, st);
-    case 1: return launch_layout<Cfg1>(a_kc, b_kc, p, st);
-    default: return launch_layout<Cfg4>(a_kc, b_kc, p, st);
-  }
+  if ((long)p.M * p.N > (4096L * 4096L) || p.K > 8192) return launch_layout<Cfg4>(a_kc, b_kc, p, st);
+  return launch_layout<Cfg3>(a_kc, b_kc, p, st);
 }
 
-static int tile_bm() { return (g_gemm_cfg >= 3) ? 64 : 128; }
-static int tile_bn() { return (g_gemm_cfg == 0) ? 128 : 64; }
-static int ctas_per_sm() { return g_gemm_cfg == 0 ? 1 : (g_gemm_cfg >= 4 ? 4 : (g_gemm_cfg == 3 ? 3 : 2)); }
-constexpr int kMaxBK = 32;
+// Split-K sizing: tile shape, resident CTAs per SM and the least k (rows of the SYRK) per split.  kCtasPerSm is 4 although
+// Cfg3 keeps 3 CTAs resident: the split count follows from it, and the split count decides which products accumulate with
+// atomics, so another value would change results, not just speed.
+constexpr int kTileBM = 64, kTileBN = 64, kCtasPerSm = 4, kMinSplitK = 256;
 
 static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
@@ -378,10 +364,10 @@ int dgemm_impl(int transA, int transB, int M, int N, int K, double alpha, const 
   // fill the resident-CTA slots: measured on the nine M = 1024 GEMMs of the SVGP O(M^3) chain (tools/bench_tri_gemm.py),
   // 2 splits (512 CTAs on 444 slots: 1.15 waves) cost 0.100 ms for the dense product against 0.075 ms with 4, and the
   // triangular ones gain 5-20 % because the k-range of each tile is split, which evens out their unequal lengths.
-  const long tiles = (long)ceil_div(M, tile_bm()) * ceil_div(N, tile_bn());
-  if (tiles * 2 <= kNumSMs * ctas_per_sm() && K >= 8 * kMaxBK * 2) {
-    int s = (int)max(4L, kNumSMs * ctas_per_sm() / tiles);
-    s = min(s, K / (8 * kMaxBK));
+  const long tiles = (long)ceil_div(M, kTileBM) * ceil_div(N, kTileBN);
+  if (tiles * 2 <= kNumSMs * kCtasPerSm && K >= 2 * kMinSplitK) {
+    int s = (int)max(4L, kNumSMs * kCtasPerSm / tiles);
+    s = min(s, K / kMinSplitK);
     s = min(s, 16);
     if (s > 1) p.splits = s;
   }
@@ -448,11 +434,11 @@ static int wsyrk_impl(int n, int M, double alpha, const double* K, long ldk, con
   p.alpha = alpha; p.beta = 0.0; p.out_tri = 2; p.w = w;
   p.w_uniform_count = w ? w_uniform_count : nullptr; p.w_uniform_target = w_uniform_target;
   p.weighted_only = weighted_only;
-  const long tiles = ((long)ceil_div(M, tile_bm()) * ceil_div(M, tile_bn()) + ceil_div(M, tile_bm())) / 2;
+  const long tiles = ((long)ceil_div(M, kTileBM) * ceil_div(M, kTileBN) + ceil_div(M, kTileBM)) / 2;
   // split the row range so that tiles x splits fills whole waves of resident CTAs: the cost of a choice is
   // (number of waves) / splits; take the cheapest among 1..32 splits of at least 512 rows each
-  const long slots = (long)kNumSMs * ctas_per_sm();
-  const int smax = (int)max(1L, min(32L, (long)n / (16 * kMaxBK)));
+  const long slots = (long)kNumSMs * kCtasPerSm;
+  const int smax = (int)max(1L, min(32L, (long)n / (2 * kMinSplitK)));
   int best_s = 1;
   double best_cost = 1e300;
   for (int sp = 1; sp <= smax; ++sp) {
@@ -491,13 +477,6 @@ extern "C" int npgp_symmetrize(int M, double* C, long ldc, int from_upper, cudaS
   dim3 blk(32, 8), grd(ceil_div(M, 32), ceil_div(M, 8));
   symmetrize_kernel<<<grd, blk, 0, stream>>>(M, C, ldc, from_upper);
   NPGP_LAUNCH_CHECK();
-  return NPGP_OK;
-}
-
-// measurement switch: 0 = 128x128 tiles (1 CTA/SM), 1 = 128x64 tiles (2 CTAs/SM, default)
-extern "C" int npgp_set_gemm_config(int cfg) {
-  if (cfg < 0 || cfg > 5) return NPGP_EINVAL;
-  npgp::g_gemm_cfg = cfg;
   return NPGP_OK;
 }
 

@@ -216,7 +216,7 @@ extern "C" int npgp_dsvi_layer_bwd(int n, int M, int d, const double* X, const d
   NPGP_TRY(npgp_colwsum(n, M, w.K, M, dmean, w.du, st));
   if (M % 128 == 0 && n >= kI8MinRows) {
     NPGP_TRY(npgp_wsyrk_weighted_only(n, M, 1.0, w.K, M, w.gv, w.cnt_sum, (double)n, w.dC, M, st));  // unequal weights (else 0)
-    NPGP_TRY(npgp_syrk_i8(n, M, 1.0, w.K, M, w.gv, w.cnt_sum, (double)n, 1, 0, w.dC, M, w.i8, w.i8_bytes, st));  // equal: + w0 K^T K
+    NPGP_TRY(npgp_syrk_i8(n, M, 1.0, w.K, M, w.gv, w.cnt_sum, (double)n, 1, w.dC, M, w.i8, w.i8_bytes, st));  // equal: + w0 K^T K
   } else {
     NPGP_TRY(npgp_wsyrk(n, M, 1.0, w.K, M, w.gv, w.dC, M, st));
   }

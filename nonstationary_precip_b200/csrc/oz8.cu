@@ -112,21 +112,14 @@ __global__ void __launch_bounds__(512, 2) o8_slice_rows_kernel(int R, int Rpad, 
 }
 
 // Column maxima of |X| (R x Kd) as bit patterns (non-negative doubles order like integers; inf / nan sort last); cmax zeroed
-// by the caller.  Optionally the same pass accumulates the weighted column sums wsum[j] += sum_i w_i X_ij.
+// by the caller.
 __global__ void __launch_bounds__(256) o8_colmax_kernel(int R, int Kd, const double* __restrict__ X, long ldx, int rows_per_cta,
-                                                        unsigned long long* __restrict__ cmax, const double* __restrict__ w,
-                                                        double* __restrict__ wsum) {
+                                                        unsigned long long* __restrict__ cmax) {
   const int j = blockIdx.x * 256 + threadIdx.x;
   if (j >= Kd) return;
   const int i0 = blockIdx.y * rows_per_cta, i1 = min(R, i0 + rows_per_cta);
   unsigned long long m = 0;
-  double acc = 0.0;
-  for (int i = i0; i < i1; ++i) {
-    const double v = X[(long)i * ldx + j];
-    m = max(m, (unsigned long long)__double_as_longlong(fabs(v)));
-    if (w) acc = fma(w[i], v, acc);
-  }
-  if (w) atomicAdd(&wsum[j], acc);
+  for (int i = i0; i < i1; ++i) m = max(m, (unsigned long long)__double_as_longlong(fabs(X[(long)i * ldx + j])));
   atomicMax(&cmax[j], m);
 }
 
@@ -229,7 +222,6 @@ O8_DEFINE_MMA(o8_mma_last, ".collector::a::lastuse")
 
 // The 28 digit products of one k-step: A digit p (descriptor a_lo + p * a_plane16) against B digits q = 0 .. 6 - p, into
 // accumulator p + q.  The A operand of a fixed p is reused across its B digits (collector hints).
-template <bool COLL>
 __device__ __forceinline__ void o8_issue_kstep(uint32_t tmem, uint32_t a_lo, uint32_t a_hi, uint32_t a_plane16, uint32_t b_lo,
                                                uint32_t b_hi, uint32_t b_plane16, uint32_t idesc_base, uint32_t first) {
 #pragma unroll
@@ -241,7 +233,7 @@ __device__ __forceinline__ void o8_issue_kstep(uint32_t tmem, uint32_t a_lo, uin
       const uint32_t idesc = idesc_base;  // every digit is signed: S8 x S8
       const uint32_t d = tmem + (uint32_t)((p + qq) * O8_BN);
       const uint32_t acc = p > 0 ? 1u : first;
-      if (!COLL || p == O8_NS - 1) o8_mma_plain(d, da, db, idesc, acc);
+      if (p == O8_NS - 1) o8_mma_plain(d, da, db, idesc, acc);
       else if (qq == 0) o8_mma_fill(d, da, db, idesc, acc);
       else if (qq == O8_NS - 1 - p) o8_mma_last(d, da, db, idesc, acc);
       else o8_mma_use(d, da, db, idesc, acc);
@@ -288,7 +280,7 @@ __device__ __forceinline__ int o8_rq_cb(int tile, int rb, int n_cb) {
 //            the split column (ms_ks k-steps; 0: no split), else 0.  The tiles of a row block run in snake order (cb
 //            descending on odd row blocks) so that the persistent CTAs, which take every gridDim.x-th tile, get even work.
 // ---------------------------------------------------------------------------------------------------------------------
-template <bool COLL, bool WT, bool TRI = false>
+template <bool WT, bool TRI = false>
 __global__ void __launch_bounds__(O8_RQ_THREADS, 1)
 o8_rowquad_kernel(int n, int N, int Kd, const int8_t* __restrict__ As, const int* __restrict__ ea,
                   const double* __restrict__ a_scale, const int8_t* __restrict__ Bs, const int* __restrict__ eb,
@@ -373,7 +365,7 @@ o8_rowquad_kernel(int n, int N, int Kd, const int8_t* __restrict__ As, const int
           // leading byte offset = distance of the two 16-byte halves of the k-step (BR * 16)
           const uint32_t a_lo = ((o8_smem(sA + stage * O8_A_STAGE) >> 4) & 0x3FFFu) | ((uint32_t)(O8_BM * 16 >> 4) << 16);
           const uint32_t b_lo = ((o8_smem(sB + stage * O8_B_STAGE) >> 4) & 0x3FFFu) | ((uint32_t)(O8_BN * 16 >> 4) << 16);
-          o8_issue_kstep<COLL>(tmem, a_lo, kHi, 2 * O8_BM * 16 >> 4, b_lo, kHi, 2 * O8_BN * 16 >> 4, idesc, ks > k_lo ? 1u : 0u);
+          o8_issue_kstep(tmem, a_lo, kHi, 2 * O8_BM * 16 >> 4, b_lo, kHi, 2 * O8_BN * 16 >> 4, idesc, ks > k_lo ? 1u : 0u);
           o8_commit(&empty[stage]);  // frees the stage when these MMAs have read it
         }
         __syncwarp();
@@ -517,27 +509,23 @@ struct O8SegIter {
   int n_items, full;     // items, full waves
   int wave;              // phase A cursor
   long posB, endB;       // phase B: range of this CTA in the remainder's (item, stage) space, stride spc per item
-  // spc_ < 0: measurement switch, whole items only (the last wave stays partial, as before the remainder split)
   __host__ __device__ O8SegIter(int n_tiles_, int nks_, int spc_, int cta_, int n_cta_, bool remainder_only = false)
-      : n_tiles(n_tiles_), nks(nks_), spc(spc_ < 0 ? -spc_ : spc_), n_cta(n_cta_), cta(cta_) {
+      : n_tiles(n_tiles_), nks(nks_), spc(spc_), n_cta(n_cta_), cta(cta_) {
     const int n_chunks = (nks + spc - 1) / spc;
     n_items = n_tiles * n_chunks;
-    full = spc_ < 0 ? (n_items + n_cta - 1) / n_cta : n_items / n_cta;
+    full = n_items / n_cta;
     wave = remainder_only ? full : 0;
-    long totalB = (long)(n_items - full * n_cta) * spc;
-    if (totalB < 0) totalB = 0;
+    const long totalB = (long)(n_items - full * n_cta) * spc;
     const long LB = (totalB + n_cta - 1) / n_cta;
     posB = (long)cta * LB;
     endB = posB + LB < totalB ? posB + LB : totalB;
   }
   __host__ __device__ long remainder_share() const {
-    long totalB = (long)(n_items - full * n_cta) * spc;
-    if (totalB < 0) totalB = 0;
+    const long totalB = (long)(n_items - full * n_cta) * spc;
     const long lb = (totalB + n_cta - 1) / n_cta;
     return lb > 0 ? lb : 1;
   }
   __host__ __device__ bool next(int& tile, int& k0, int& k1) {
-    while (wave < full && wave * n_cta + cta >= n_items) ++wave;  // (only with the measurement switch)
     if (wave < full) {
       const int item = wave * n_cta + cta;
       ++wave;
@@ -574,7 +562,7 @@ struct O8SegIter {
 //   MN = false: Xs = transposed planes (operand rows = columns of X, o8_slice_t_kernel), per-column exponents ex; K-major.
 // Work item = (chunk, tile), chunk-major so that the CTAs running together read the same rows (L2 reuse).
 // ---------------------------------------------------------------------------------------------------------------------
-template <bool MN, bool COLL>
+template <bool MN>
 __global__ void __launch_bounds__(O8_THREADS, 1)
 o8_syrk_kernel(int M, int nks_total, int spc, int slots_per_cta, const int8_t* __restrict__ Xs, const int* __restrict__ ex,
                const double* __restrict__ x_scale, const double* __restrict__ uniform_count, double uniform_target,
@@ -673,7 +661,7 @@ o8_syrk_kernel(int M, int nks_total, int spc, int slots_per_cta, const int8_t* _
         if (leader) {
           const uint32_t a_lo = ((o8_smem(sA + stage * O8_A_STAGE) >> 4) & 0x3FFFu) | ((lboA >> 4) << 16);
           const uint32_t b_lo = ((o8_smem(sB + stage * O8_B_STAGE) >> 4) & 0x3FFFu) | ((lboB >> 4) << 16);
-          o8_issue_kstep<COLL>(tmem, a_lo, kHi, 4096 >> 4, b_lo, kHi, 2048 >> 4, idesc, ks > k0 ? 1u : 0u);
+          o8_issue_kstep(tmem, a_lo, kHi, 4096 >> 4, b_lo, kHi, 2048 >> 4, idesc, ks > k0 ? 1u : 0u);
           o8_commit(&empty[stage]);
         }
         __syncwarp();
@@ -761,8 +749,7 @@ __global__ void __launch_bounds__(256) o8_syrk_finish_kernel(int M, int nks_tota
   for (int i = 0; i < EPT; ++i) acc[i] = 0.0;
   {
     const O8SegIter probe(n_tiles, nks_total, spc, 0, n_cta);
-    const int aspc = probe.spc;  // (spc < 0 carries the measurement switch)
-    const int n_chunks = (nks_total + aspc - 1) / aspc;
+    const int n_chunks = (nks_total + spc - 1) / spc;
     const long LB = probe.remainder_share();
     for (int chunk = 0; chunk < n_chunks; ++chunk) {
       const int item = chunk * n_tiles + tile;
@@ -774,12 +761,12 @@ __global__ void __launch_bounds__(256) o8_syrk_finish_kernel(int M, int nks_tota
       }
       // an item of the remainder: its stages are spread over the CTAs c_first .. c_last
       const int j = item - probe.full * n_cta;
-      const int c_first = (int)(((long)j * aspc) / LB), c_last = (int)((((long)j + 1) * aspc - 1) / LB);
+      const int c_first = (int)(((long)j * spc) / LB), c_last = (int)((((long)j + 1) * spc - 1) / LB);
       for (int c = c_first; c <= c_last && c < n_cta; ++c) {
         O8SegIter it(n_tiles, nks_total, spc, c, n_cta, true);
         int t2, k0, k1, idx = probe.full;
         while (it.next(t2, k0, k1)) {
-          if (t2 == tile && k0 / aspc == chunk) {
+          if (t2 == tile && k0 / spc == chunk) {
             const double* src = part + ((long)c * slots_per_cta + idx) * (O8_BM * O8_BN) + e0 + threadIdx.x;
 #pragma unroll
             for (int i = 0; i < EPT; ++i) acc[i] += src[256 * i];
@@ -847,8 +834,6 @@ __global__ void __launch_bounds__(256) o8_sum_partials_kernel(int nb, int N, con
   }
 }
 
-static int g_o8_syrk_whole_items = 0;  // measurement switch (npgp_o8_set_syrk_split(0)): no split of the last partial wave
-
 // Launch shape of the SYRK: CTAs, stages per row chunk and the largest number of segments any CTA produces (host run of the
 // device iterator).  The chunk length is the largest that (i) keeps int32 exact (O8_MAX_SEG) and (ii) lets the rows a wave
 // of CTAs works on (kNumSMs / n_tiles chunks) stay resident in L2 (~110 MB of the 126 MB): every extra chunk costs one
@@ -864,13 +849,13 @@ static int o8_syrk_shape(int nks, int n_tiles, int M, int* n_cta_out, int* spc_o
   const int n_cta = (int)(items < kNumSMs ? items : kNumSMs);
   int worst = 1;
   for (int c = 0; c < n_cta; ++c) {
-    O8SegIter it(n_tiles, nks, g_o8_syrk_whole_items ? -spc : spc, c, n_cta);
+    O8SegIter it(n_tiles, nks, spc, c, n_cta);
     int t, k0, k1, cnt = 0;
     while (it.next(t, k0, k1)) ++cnt;
     if (cnt > worst) worst = cnt;
   }
   *n_cta_out = n_cta;
-  *spc_out = g_o8_syrk_whole_items ? -spc : spc;
+  *spc_out = spc;
   return worst;
 }
 
@@ -884,22 +869,9 @@ static inline int o8_syrk_tiles(int M) {
 using namespace npgp;
 
 static long long* g_o8_dbg = nullptr;  // debugging aid only (npgp_rowquad_i8_debug); NULL in production
-static int g_o8_collector = 1;         // measurement switch (npgp_o8_set_collector)
 
 // debugging aid: device buffer of 8 counters filled by CTA 0 (cycles the producer / MMA issuer / epilogue spend waiting)
 extern "C" void npgp_rowquad_i8_debug(long long* dev_counters) { g_o8_dbg = dev_counters; }
-// measurement switch: 1 (default) = A-operand collector reuse hints on the digit products, 0 = plain MMAs
-extern "C" int npgp_o8_set_collector(int on) {
-  g_o8_collector = on ? 1 : 0;
-  return NPGP_OK;
-}
-
-// measurement switch: 1 (default) = the items of the last partial wave of the SYRK are split evenly over the CTAs, 0 = whole items
-extern "C" int npgp_o8_set_syrk_split(int on) {
-  g_o8_syrk_whole_items = on ? 0 : 1;
-  return NPGP_OK;
-}
-
 extern "C" long npgp_o8_digits_bytes(int rows, int Kd, int block_rows) {
   if (rows < 0 || Kd < 0 || (block_rows != O8_BM && block_rows != O8_BN)) return -1;
   return o8_digits_bytes(rows, Kd, block_rows);
@@ -930,7 +902,7 @@ extern "C" int npgp_o8_slice_rows(int R, int Kd, const double* X, long ldx, int 
 //   q (optional): q_stride == 0 -> q[i] += (atomics; zeroed by the caller); q_stride >= n -> q[cb * q_stride + i] = partial of
 //                 column block cb (M / 64 blocks, plain stores: deterministic)
 //   gvec / du_part (optional, both or none): du_part[rb * M + j] = sum over the rows of row block rb of gvec_i K_ij
-template <bool COLL, bool WT, bool TRI = false>
+template <bool WT, bool TRI = false>
 static int o8_rowquad_launch(int n, int N, int Kd, const void* a_digits, const int* a_expo, const double* a_scale,
                              const void* c_digits, const int* c_expo, const double* Kmat, long ldk, double* T, long ldt,
                              double* q, long q_stride, const double* gvec, double* du_part, cudaStream_t stream,
@@ -938,8 +910,8 @@ static int o8_rowquad_launch(int n, int N, int Kd, const void* a_digits, const i
   const long npad = ((long)n + O8_BM - 1) / O8_BM * O8_BM;
   const long tiles = npad / O8_BM * (N / O8_BN);
   const int grid = (int)(tiles < kNumSMs ? tiles : kNumSMs);
-  NPGP_CUDA(cudaFuncSetAttribute(o8_rowquad_kernel<COLL, WT, TRI>, cudaFuncAttributeMaxDynamicSharedMemorySize, O8_RQ_SMEM));
-  o8_rowquad_kernel<COLL, WT, TRI><<<grid, O8_RQ_THREADS, O8_RQ_SMEM, stream>>>(
+  NPGP_CUDA(cudaFuncSetAttribute(o8_rowquad_kernel<WT, TRI>, cudaFuncAttributeMaxDynamicSharedMemorySize, O8_RQ_SMEM));
+  o8_rowquad_kernel<WT, TRI><<<grid, O8_RQ_THREADS, O8_RQ_SMEM, stream>>>(
       n, N, Kd, (const int8_t*)a_digits, a_expo, a_scale, (const int8_t*)c_digits, c_expo, Kmat, ldk, T, ldt, q, q_stride, gvec,
       du_part, g_o8_dbg, ms_ks);
   NPGP_LAUNCH_CHECK();
@@ -957,14 +929,11 @@ extern "C" int npgp_o8_rowquad_digits(int n, int M, const void* a_digits, const 
   if (M % O8_BN || M > O8_MAX_KD || (T && ((ldt & 1) || (reinterpret_cast<uintptr_t>(T) & 15))) ||
       (Kmat && ((ldk & 1) || (reinterpret_cast<uintptr_t>(Kmat) & 15))) || (q_stride != 0 && q_stride < n))
     return NPGP_EUNSUPPORTED;
-#define NPGP_RQ(COLL, WT) \
-  o8_rowquad_launch<COLL, WT>(n, M, M, a_digits, a_expo, a_scale, c_digits, c_expo, Kmat, ldk, T, ldt, q, q_stride, gvec, \
-                              du_part, stream)
-  int rc;
-  if (T) rc = g_o8_collector ? NPGP_RQ(true, true) : NPGP_RQ(false, true);
-  else rc = g_o8_collector ? NPGP_RQ(true, false) : NPGP_RQ(false, false);
-#undef NPGP_RQ
-  return rc;
+  if (T)
+    return o8_rowquad_launch<true>(n, M, M, a_digits, a_expo, a_scale, c_digits, c_expo, Kmat, ldk, T, ldt, q, q_stride, gvec,
+                                   du_part, stream);
+  return o8_rowquad_launch<false>(n, M, M, a_digits, a_expo, a_scale, c_digits, c_expo, Kmat, ldk, T, ldt, q, q_stride, gvec,
+                                  du_part, stream);
 }
 
 // T (n x N) = A B^T from planes: A (n x Kd, block_rows 128; a_expo NULL -> matrix-wide exponent from *a_scale), B (N x Kd,
@@ -977,11 +946,8 @@ extern "C" int npgp_o8_gemm_digits(int n, int N, int Kd, const void* a_digits, c
   if (!a_digits || (!a_expo && !a_scale) || !b_digits || !b_expo || !T) return NPGP_EINVAL;
   if (N % O8_BN || Kd == 0 || Kd % O8_KS || Kd > O8_MAX_KD || ldt < N || (ldt & 1) || (reinterpret_cast<uintptr_t>(T) & 15))
     return NPGP_EUNSUPPORTED;
-  if (g_o8_collector)
-    return o8_rowquad_launch<true, true>(n, N, Kd, a_digits, a_expo, a_scale, b_digits, b_expo, nullptr, 0, T, ldt, nullptr,
-                                         0, nullptr, nullptr, stream);
-  return o8_rowquad_launch<false, true>(n, N, Kd, a_digits, a_expo, a_scale, b_digits, b_expo, nullptr, 0, T, ldt, nullptr, 0,
-                                        nullptr, nullptr, stream);
+  return o8_rowquad_launch<true>(n, N, Kd, a_digits, a_expo, a_scale, b_digits, b_expo, nullptr, 0, T, ldt, nullptr, 0, nullptr,
+                                 nullptr, stream);
 }
 
 // q[cb * q_stride + i] = sum_{j in column block cb} (A B^T)_ij^2 from planes, B (N x Kd, block_rows 64, per-row exponents)
@@ -994,11 +960,8 @@ extern "C" int npgp_o8_trinorm_digits(int n, int N, int Kd, int Ms, const void* 
   if (N % O8_BN || Kd % O8_KS || Kd > O8_MAX_KD || Ms < 0 || Ms % O8_BN || (Ms > 0 && Ms >= Kd) || q_stride < n)
     return NPGP_EINVAL;
   if (n == 0 || N == 0) return NPGP_OK;
-  if (g_o8_collector)
-    return o8_rowquad_launch<true, false, true>(n, N, Kd, a_digits, a_expo, a_scale, b_digits, b_expo, nullptr, 0, nullptr,
-                                                0, q, q_stride, nullptr, nullptr, stream, Ms / O8_KS);
-  return o8_rowquad_launch<false, false, true>(n, N, Kd, a_digits, a_expo, a_scale, b_digits, b_expo, nullptr, 0, nullptr, 0,
-                                               q, q_stride, nullptr, nullptr, stream, Ms / O8_KS);
+  return o8_rowquad_launch<false, true>(n, N, Kd, a_digits, a_expo, a_scale, b_digits, b_expo, nullptr, 0, nullptr, 0, q,
+                                        q_stride, nullptr, nullptr, stream, Ms / O8_KS);
 }
 
 // out[j] = sum_b part[b * N + j], b in index order (e.g. du from the du_part of npgp_o8_rowquad_digits, nb = ceil(n / 128))
@@ -1018,11 +981,13 @@ extern "C" long npgp_rowquad_i8_workspace_bytes(int n, int M) {
   return npad * M * O8_NS + (long)M * M * O8_NS + (npad + M) * (long)sizeof(int) + 1024;
 }
 
-static int rowquad_i8_impl(int n, int M, const double* K, long ldk, const double* C, long ldc, double* T, long ldt, double* q,
-                           void* work, long work_bytes, cudaStream_t stream, bool slice, bool gemm) {
+// T (n x M) = K (n x M) @ C (M x M, symmetric);  q[i] += sum_j T_ij K_ij (q zeroed by the caller; NULL to skip).
+// M must be a multiple of 64 (and <= 16384).  Replaces npgp_rowquad on the integer tensor-core path.
+extern "C" int npgp_rowquad_i8(int n, int M, const double* K, long ldk, const double* C, long ldc, double* T, long ldt,
+                               double* q, void* work, long work_bytes, cudaStream_t stream) {
   if (n < 0 || M < 0) return NPGP_EINVAL;
   if (n == 0 || M == 0) return NPGP_OK;
-  if (!K || !work || (slice && !C) || (gemm && !T)) return NPGP_EINVAL;
+  if (!K || !work || !C || !T) return NPGP_EINVAL;
   if (M % O8_BN || M > O8_MAX_KD) return NPGP_EUNSUPPORTED;
   if (work_bytes < npgp_rowquad_i8_workspace_bytes(n, M)) return NPGP_EWORKSPACE;
   const long npad = ((long)n + O8_BM - 1) / O8_BM * O8_BM;
@@ -1030,31 +995,11 @@ static int rowquad_i8_impl(int n, int M, const double* K, long ldk, const double
   int8_t* Bs = As + npad * M * O8_NS;
   int* ea = reinterpret_cast<int*>(Bs + (long)M * M * O8_NS);
   int* eb = ea + npad;
-  if (slice) {
-    int rc = npgp_o8_slice_rows(n, M, K, ldk, O8_BM, As, ea, stream);
-    if (rc) return rc;
-    rc = npgp_o8_slice_rows(M, M, C, ldc, O8_BN, Bs, eb, stream);
-    if (rc) return rc;
-  }
-  if (!gemm) return NPGP_OK;
+  int rc = npgp_o8_slice_rows(n, M, K, ldk, O8_BM, As, ea, stream);
+  if (rc) return rc;
+  rc = npgp_o8_slice_rows(M, M, C, ldc, O8_BN, Bs, eb, stream);
+  if (rc) return rc;
   return npgp_o8_rowquad_digits(n, M, As, ea, nullptr, Bs, eb, K, ldk, T, ldt, q, 0, nullptr, nullptr, stream);
-}
-
-// T (n x M) = K (n x M) @ C (M x M, symmetric);  q[i] += sum_j T_ij K_ij (q zeroed by the caller; NULL to skip).
-// M must be a multiple of 64 (and <= 16384).  Replaces npgp_rowquad on the integer tensor-core path.
-extern "C" int npgp_rowquad_i8(int n, int M, const double* K, long ldk, const double* C, long ldc, double* T, long ldt,
-                               double* q, void* work, long work_bytes, cudaStream_t stream) {
-  return rowquad_i8_impl(n, M, K, ldk, C, ldc, T, ldt, q, work, work_bytes, stream, true, true);
-}
-// The slicing passes alone (K and C into `work`); follow with npgp_rowquad_i8_gemm_only.
-extern "C" int npgp_rowquad_i8_slice_only(int n, int M, const double* K, long ldk, const double* C, long ldc, void* work,
-                                          long work_bytes, cudaStream_t stream) {
-  return rowquad_i8_impl(n, M, K, ldk, C, ldc, nullptr, 0, nullptr, work, work_bytes, stream, true, false);
-}
-// The tensor-core kernel alone, on the digit planes a previous call with the same shapes left in `work`.
-extern "C" int npgp_rowquad_i8_gemm_only(int n, int M, const double* K, long ldk, double* T, long ldt, double* q, void* work,
-                                         long work_bytes, cudaStream_t stream) {
-  return rowquad_i8_impl(n, M, K, ldk, nullptr, 0, T, ldt, q, work, work_bytes, stream, false, true);
 }
 
 // ---- SYRK ------------------------------------------------------------------------------------------------------------
@@ -1098,8 +1043,7 @@ static int o8_syrk_launch(int M, int nks, const int8_t* Xs, const int* ex, const
                           const double* w0_dev, const double* uniform_count, double uniform_target, int accumulate,
                           double* Out, long ldo, double* part, const int* skip_count, const int* skip_rows,
                           cudaStream_t stream) {
-  NPGP_CUDA(cudaFuncSetAttribute(o8_syrk_kernel<MN, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, O8_SY_SMEM));
-  NPGP_CUDA(cudaFuncSetAttribute(o8_syrk_kernel<MN, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, O8_SY_SMEM));
+  NPGP_CUDA(cudaFuncSetAttribute(o8_syrk_kernel<MN>, cudaFuncAttributeMaxDynamicSharedMemorySize, O8_SY_SMEM));
   CUtensorMap tmA, tmB;
   memset(&tmA, 0, sizeof(tmA));
   memset(&tmB, 0, sizeof(tmB));
@@ -1112,12 +1056,8 @@ static int o8_syrk_launch(int M, int nks, const int8_t* Xs, const int* ex, const
   const int n_tiles = o8_syrk_tiles(M);
   int grid, spc;
   const int slots = o8_syrk_shape(nks, n_tiles, M, &grid, &spc);
-  if (g_o8_collector)
-    o8_syrk_kernel<MN, true><<<grid, O8_THREADS, O8_SY_SMEM, stream>>>(M, nks, spc, slots, Xs, ex, x_scale, uniform_count,
-                                                                      uniform_target, part, tmA, tmB);
-  else
-    o8_syrk_kernel<MN, false><<<grid, O8_THREADS, O8_SY_SMEM, stream>>>(M, nks, spc, slots, Xs, ex, x_scale, uniform_count,
-                                                                       uniform_target, part, tmA, tmB);
+  o8_syrk_kernel<MN><<<grid, O8_THREADS, O8_SY_SMEM, stream>>>(M, nks, spc, slots, Xs, ex, x_scale, uniform_count, uniform_target,
+                                                               part, tmA, tmB);
   NPGP_LAUNCH_CHECK();
   o8_syrk_finish_kernel<<<dim3(n_tiles, 4), 256, 0, stream>>>(M, nks, spc, grid, slots, part, alpha, w0_dev, uniform_count, uniform_target,
                                                      accumulate, Out, ldo, skip_count, skip_rows, MN ? Xs : nullptr, x_scale);
@@ -1152,12 +1092,14 @@ extern "C" long npgp_syrk_i8_workspace_bytes(int n, int M) {
   return npad * M * O8_NS + (long)M * (sizeof(unsigned long long) + sizeof(int)) + 1024 + npgp_o8_syrk_part_bytes(n, M);
 }
 
-static int syrk_i8_impl(int n, int M, double alpha, const double* K, long ldk, const double* w0_dev,
-                        const double* uniform_count, double uniform_target, int accumulate, int phase, double* Out, long ldo,
-                        void* work, long work_bytes, const double* colw, double* colwsum, cudaStream_t stream) {
+// Out (M x M, symmetric) = alpha * w0 * K^T K with w0 = *w0_dev (NULL: 1), K (n x M) arbitrary FP64; M % 128 == 0.
+// uniform_count / uniform_target (optional): device-side gate (see npgp_wsyrk_hint); accumulate != 0: add to Out.
+extern "C" int npgp_syrk_i8(int n, int M, double alpha, const double* K, long ldk, const double* w0_dev,
+                            const double* uniform_count, double uniform_target, int accumulate, double* Out, long ldo,
+                            void* work, long work_bytes, cudaStream_t stream) {
   if (n < 0 || M < 0) return NPGP_EINVAL;
   if (M == 0) return NPGP_OK;
-  if ((phase != 1 && !Out) || (n > 0 && !K) || !work || phase < 0 || phase > 2) return NPGP_EINVAL;
+  if (!Out || (n > 0 && !K) || !work) return NPGP_EINVAL;
   if (M % O8_BM) return NPGP_EUNSUPPORTED;
   if (work_bytes < npgp_syrk_i8_workspace_bytes(n, M)) return NPGP_EWORKSPACE;
   const long npad = ((long)n + O8_BM - 1) / O8_BM * O8_BM;
@@ -1166,42 +1108,20 @@ static int syrk_i8_impl(int n, int M, double alpha, const double* K, long ldk, c
   unsigned long long* cmax = reinterpret_cast<unsigned long long*>(Xs + npad * M * O8_NS);
   int* ex = reinterpret_cast<int*>(cmax + M);
   double* part = reinterpret_cast<double*>((reinterpret_cast<uintptr_t>(ex + M) + 1023) & ~(uintptr_t)1023);
-  if (colwsum) NPGP_CUDA(cudaMemsetAsync(colwsum, 0, sizeof(double) * M, stream));
   if (n == 0) {
-    if (phase != 1 && !accumulate) NPGP_CUDA(cudaMemset2DAsync(Out, sizeof(double) * ldo, 0, sizeof(double) * M, M, stream));
+    if (!accumulate) NPGP_CUDA(cudaMemset2DAsync(Out, sizeof(double) * ldo, 0, sizeof(double) * M, M, stream));
     return NPGP_OK;
   }
-  if (phase != 2) {
-    NPGP_CUDA(cudaMemsetAsync(cmax, 0, sizeof(unsigned long long) * M, stream));
-    const int rows_per_cta = 256;
-    dim3 grid(ceil_div(M, 256), ceil_div(n, rows_per_cta));
-    o8_colmax_kernel<<<grid, 256, 0, stream>>>(n, M, K, ldk, rows_per_cta, cmax, colw, colwsum);
-    NPGP_LAUNCH_CHECK();
-    o8_exp_from_max_kernel<<<ceil_div(M, 256), 256, 0, stream>>>(M, cmax, ex);
-    NPGP_LAUNCH_CHECK();
-    dim3 gs(nks, M / O8_BM);
-    o8_slice_t_kernel<<<gs, 256, 0, stream>>>(n, M, K, ldk, ex, Xs);
-    NPGP_LAUNCH_CHECK();
-  }
-  if (phase == 1) return NPGP_OK;
+  NPGP_CUDA(cudaMemsetAsync(cmax, 0, sizeof(unsigned long long) * M, stream));
+  const int rows_per_cta = 256;
+  dim3 grid(ceil_div(M, 256), ceil_div(n, rows_per_cta));
+  o8_colmax_kernel<<<grid, 256, 0, stream>>>(n, M, K, ldk, rows_per_cta, cmax);
+  NPGP_LAUNCH_CHECK();
+  o8_exp_from_max_kernel<<<ceil_div(M, 256), 256, 0, stream>>>(M, cmax, ex);
+  NPGP_LAUNCH_CHECK();
+  dim3 gs(nks, M / O8_BM);
+  o8_slice_t_kernel<<<gs, 256, 0, stream>>>(n, M, K, ldk, ex, Xs);
+  NPGP_LAUNCH_CHECK();
   return o8_syrk_launch<false>(M, nks, Xs, ex, nullptr, alpha, w0_dev, uniform_count, uniform_target, accumulate, Out, ldo,
                                part, nullptr, nullptr, stream);
-}
-
-// Out (M x M, symmetric) = alpha * w0 * K^T K with w0 = *w0_dev (NULL: 1), K (n x M) arbitrary FP64; M % 128 == 0.
-// uniform_count / uniform_target (optional): device-side gate (see npgp_wsyrk_hint); accumulate != 0: add to Out.
-// phase: 0 = slice K and run; 1 = slicing passes only; 2 = tensor-core kernel only, on the planes a phase-1 call left in work.
-extern "C" int npgp_syrk_i8(int n, int M, double alpha, const double* K, long ldk, const double* w0_dev,
-                            const double* uniform_count, double uniform_target, int accumulate, int phase, double* Out,
-                            long ldo, void* work, long work_bytes, cudaStream_t stream) {
-  return syrk_i8_impl(n, M, alpha, K, ldk, w0_dev, uniform_count, uniform_target, accumulate, phase, Out, ldo, work,
-                      work_bytes, nullptr, nullptr, stream);
-}
-
-// The slicing passes of npgp_syrk_i8 (phase 1) with the weighted column sums wsum[j] = sum_i w_i K_ij (overwritten) fused
-// into the column-maximum pass.
-extern "C" int npgp_syrk_i8_prepare(int n, int M, const double* K, long ldk, const double* w, double* wsum, void* work,
-                                    long work_bytes, cudaStream_t stream) {
-  if ((w == nullptr) != (wsum == nullptr)) return NPGP_EINVAL;
-  return syrk_i8_impl(n, M, 1.0, K, ldk, nullptr, nullptr, 0.0, 0, 1, nullptr, 0, work, work_bytes, w, wsum, stream);
 }

@@ -198,30 +198,17 @@ def _ws(workspace, device):
     return _DEFAULT_I8_WS[key]
 
 
-def set_i8_collector(on: bool):
-    """Measurement switch: A-operand collector-reuse hints of the digit products (default on)."""
-    check(lib().npgp_o8_set_collector(int(bool(on))), "npgp_o8_set_collector")
-
-
-def rowquad_i8(K, Cm, need_q=True, T=None, between=None, workspace=None):
+def rowquad_i8(K, Cm, need_q=True, T=None, workspace=None):
     """rowquad on the integer tensor cores (tcgen05 kind::i8, exact byte-digit split, see csrc/oz8.cu).  Cm must be
-    symmetric and M a multiple of 64.  `between`: callable run after the slicing passes have been enqueued and before the
-    tensor-core kernel."""
+    symmetric and M a multiple of 64."""
     n, M = K.shape
     if T is None:
         T = torch.empty(n, M, dtype=torch.float64, device=K.device)
     q = torch.zeros(n, dtype=torch.float64, device=K.device) if need_q else None
     nbytes = lib().npgp_rowquad_i8_workspace_bytes(n, M)
     work = _ws(workspace, K.device).get(("rowquad", n, M), nbytes, K.device)
-    if between is None:
-        check(lib().npgp_rowquad_i8(n, M, ptr(K), K.stride(0), ptr(Cm), Cm.stride(0), ptr(T), T.stride(0), ptr(q),
-                                    ptr(work), nbytes, stream()), "npgp_rowquad_i8")
-    else:  # slicing passes, then `between()` (e.g. fork other HBM-bound work to a side stream), then the tensor-core kernel
-        check(lib().npgp_rowquad_i8_slice_only(n, M, ptr(K), K.stride(0), ptr(Cm), Cm.stride(0), ptr(work), nbytes,
-                                               stream()), "npgp_rowquad_i8_slice_only")
-        between()
-        check(lib().npgp_rowquad_i8_gemm_only(n, M, ptr(K), K.stride(0), ptr(T), T.stride(0), ptr(q), ptr(work), nbytes,
-                                              stream()), "npgp_rowquad_i8_gemm_only")
+    check(lib().npgp_rowquad_i8(n, M, ptr(K), K.stride(0), ptr(Cm), Cm.stride(0), ptr(T), T.stride(0), ptr(q), ptr(work),
+                                nbytes, stream()), "npgp_rowquad_i8")
     return T, q
 
 
@@ -238,23 +225,12 @@ def syrk_i8(K, w0=None, alpha=1.0, out=None, workspace=None):
     if out is None:
         out = torch.empty(M, M, dtype=torch.float64, device=K.device)
     work, nbytes = _syrk_i8_work(K, workspace)
-    check(lib().npgp_syrk_i8(n, M, float(alpha), ptr(K), K.stride(0), ptr(w0), None, 0.0, 0, 0, ptr(out), out.stride(0),
+    check(lib().npgp_syrk_i8(n, M, float(alpha), ptr(K), K.stride(0), ptr(w0), None, 0.0, 0, ptr(out), out.stride(0),
                              ptr(work), nbytes, stream()), "npgp_syrk_i8")
     return out
 
 
-def syrk_i8_prepare(K, w=None, workspace=None):
-    """Slicing passes of the int8 SYRK only (column maxima, exponents, transposed digit planes into the workspace).  Follow
-    with wsyrk_i8(..., prepared=True) on the same workspace.  With `w` (n,) the column-maximum pass also returns K^T w."""
-    n, M = K.shape
-    work, nbytes = _syrk_i8_work(K, workspace)
-    wsum = torch.empty(M, dtype=torch.float64, device=K.device) if w is not None else None
-    check(lib().npgp_syrk_i8_prepare(n, M, ptr(K), K.stride(0), ptr(_c(w)), ptr(wsum), ptr(work), nbytes, stream()),
-          "npgp_syrk_i8_prepare")
-    return wsum
-
-
-def wsyrk_i8(K, w, uniform_count, uniform_target, alpha=1.0, out=None, prepared=False, workspace=None):
+def wsyrk_i8(K, w, uniform_count, uniform_target, alpha=1.0, out=None, workspace=None):
     """alpha * K^T diag(w) K with the device-side equal-weights gate of `wsyrk`: equal weights run on the integer tensor
     cores, unequal ones on the FP64 weighted kernel; both are enqueued and the one the flag does not select exits at once."""
     n, M = K.shape
@@ -266,7 +242,7 @@ def wsyrk_i8(K, w, uniform_count, uniform_target, alpha=1.0, out=None, prepared=
           "npgp_wsyrk_weighted_only")
     work, nbytes = _syrk_i8_work(K, workspace)
     check(lib().npgp_syrk_i8(n, M, float(alpha), ptr(K), K.stride(0), ptr(w), ptr(uniform_count), float(uniform_target), 1,
-                             2 if prepared else 0, ptr(out), out.stride(0), ptr(work), nbytes, stream()), "npgp_syrk_i8")
+                             ptr(out), out.stride(0), ptr(work), nbytes, stream()), "npgp_syrk_i8")
     return out
 
 

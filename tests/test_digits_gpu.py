@@ -124,24 +124,6 @@ def test_rowquad_and_syrk_from_digits(variant, n, M):
     assert ((got2 - want2).abs() <= syrk_bound).all()
 
 
-def test_collector_switch_gives_identical_results():
-    from nonstationary_precip_b200 import ops
-    g = torch.Generator().manual_seed(1)
-    K = torch.rand(2000, 256, generator=g).cuda()
-    C = torch.randn(256, 256, generator=g).cuda()
-    C = C + C.T
-    try:
-        ops.set_i8_collector(True)
-        T1, q1 = ops.rowquad_i8(K, C)
-        S1 = ops.syrk_i8(K)
-        ops.set_i8_collector(False)
-        T0, q0 = ops.rowquad_i8(K, C)
-        S0 = ops.syrk_i8(K)
-    finally:
-        ops.set_i8_collector(True)
-    assert torch.equal(T0, T1) and torch.equal(S0, S1)
-
-
 def test_non_finite_input_poisons_the_row_not_the_digits():
     """ADVICE r1: the slicer turned NaN / Inf into finite digits.  Now the row's exponent is marked and the result is NaN."""
     from nonstationary_precip_b200 import ops

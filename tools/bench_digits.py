@@ -1,6 +1,6 @@
 #!/usr/bin/env python3
 """Timings of the digit-plane path at the C2 shapes (B=65536, M=1024, d=3): Gibbs kernels emitting digits, the int8
-row-quadratic kernel and the MN-major SYRK with / without A-operand collector reuse, the int8 peak probes.
+row-quadratic kernel and the MN-major SYRK, the int8 peak probes.
 Run on the GPU box:  python tools/bench_digits.py > gpurun_out/bench_digits.jsonl"""
 import json
 import os
@@ -70,21 +70,14 @@ def main():
     gvec = torch.randn(B, **f64)
     part = torch.empty(max(1, ops.o8_syrk_part_bytes(B, M) // 8), **f64)
     Out = torch.empty(M, M, **f64)
-    for coll in (1, 0):
-        ops.set_i8_collector(bool(coll))
-        ms, best = timeit(lambda: ops.o8_rowquad_digits(B, M, digits, s, Cd, cexp, T, q_part=q_part, gvec=gvec, du_part=du_part))
-        report("o8_rowquad_digits[collector=%d] (T, q, K^T g)" % coll, ms, best, int8_tops=round(28 * 2 * B * M * M / best / 1e9, 1),
-               fp64_equiv_tflops=round(2 * B * M * M / best / 1e9, 2))
-        ms, best = timeit(lambda: ops.o8_rowquad_digits(B, M, digits, s, Cd, cexp, T))
-        report("o8_rowquad_digits[collector=%d] (T only)" % coll, ms, best, int8_tops=round(28 * 2 * B * M * M / best / 1e9, 1))
-        ms, best = timeit(lambda: ops.o8_syrk_digits(B, M, digits, s, part, out=Out))
-        report("o8_syrk_digits[collector=%d] (MN-major planes, finish included)" % coll, ms, best,
-               int8_tops_useful=round(28 * B * M * (M + 64) / best / 1e9, 1))
-    ops.set_i8_collector(True)
-    for split in (0, 1, 0, 1):
-        check(lib().npgp_o8_set_syrk_split(split), "split")
-        ms, best = timeit(lambda: ops.o8_syrk_digits(B, M, digits, s, part, out=Out))
-        report("o8_syrk_digits[remainder split=%d]" % split, ms, best, int8_tops_useful=round(28 * B * M * (M + 64) / best / 1e9, 1))
+    ms, best = timeit(lambda: ops.o8_rowquad_digits(B, M, digits, s, Cd, cexp, T, q_part=q_part, gvec=gvec, du_part=du_part))
+    report("o8_rowquad_digits (T, q, K^T g)", ms, best, int8_tops=round(28 * 2 * B * M * M / best / 1e9, 1),
+           fp64_equiv_tflops=round(2 * B * M * M / best / 1e9, 2))
+    ms, best = timeit(lambda: ops.o8_rowquad_digits(B, M, digits, s, Cd, cexp, T))
+    report("o8_rowquad_digits (T only)", ms, best, int8_tops=round(28 * 2 * B * M * M / best / 1e9, 1))
+    ms, best = timeit(lambda: ops.o8_syrk_digits(B, M, digits, s, part, out=Out))
+    report("o8_syrk_digits (MN-major planes, finish included)", ms, best,
+           int8_tops_useful=round(28 * B * M * (M + 64) / best / 1e9, 1))
     Kf = ops.gibbs_full_fwd(x, Sx, z, Sz, 1e-5, s)
     ms, best = timeit(lambda: ops.rowquad_i8(Kf, C, T=T))
     report("rowquad_i8 (general operands: slicing passes included)", ms, best)

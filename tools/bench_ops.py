@@ -94,16 +94,12 @@ def main():
     T = torch.empty(B, M, **f64)
     Out = torch.empty(M, M, **f64)
     A1, A2 = torch.randn(M, M, **f64), torch.randn(M, M, **f64)
-    for cfg, nm in ((0, "128x128,bk16,s3"), (1, "128x64,bk16,s3"), (2, "128x64,bk32,s2"), (3, "64x64,128thr,3cta"), (4, "64x64,128thr,4cta")):
-        check(lib().npgp_set_gemm_config(cfg), "cfg")
-        ms, best = timeit(lambda: ops.rowquad(K, Cm, T=T))
-        report("rowquad[%s]" % nm, ms, best, tflops=round(2 * B * M * M / best / 1e9, 2))
-        ms, best = timeit(lambda: ops.wsyrk(K, None, out=Out))
-        report("wsyrk[%s]" % nm, ms, best, tflops_full=round(2 * B * M * M / best / 1e9, 2),
-               tflops_useful=round(B * M * (M + 128) / best / 1e9, 2))
-        ms, best = timeit(lambda: ops.dgemm(A1, A2, C=Out))
-        report("dgemm_MMM[%s]" % nm, ms, best, tflops=round(2 * M ** 3 / best / 1e9, 2))
-    check(lib().npgp_set_gemm_config(5), "cfg")
+    ms, best = timeit(lambda: ops.rowquad(K, Cm, T=T))
+    report("rowquad", ms, best, tflops=round(2 * B * M * M / best / 1e9, 2))
+    ms, best = timeit(lambda: ops.wsyrk(K, None, out=Out))
+    report("wsyrk", ms, best, tflops_full=round(2 * B * M * M / best / 1e9, 2), tflops_useful=round(B * M * (M + 128) / best / 1e9, 2))
+    ms, best = timeit(lambda: ops.dgemm(A1, A2, C=Out))
+    report("dgemm_MMM", ms, best, tflops=round(2 * M ** 3 / best / 1e9, 2))
     # the same two contractions on the int8 tensor cores (exact Ozaki split, csrc/ozaki.cu), slicing passes included
     Cs = 0.5 * (Cm + Cm.T)
     ms, best = timeit(lambda: ops.rowquad_i8(K, Cs, T=T))

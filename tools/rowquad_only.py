@@ -3,8 +3,6 @@
 import os, sys, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from nonstationary_precip_b200 import ops
-from nonstationary_precip_b200._lib import lib
-lib().npgp_set_gemm_config(int(os.environ.get("GEMM_CFG", 5)))
 B, M = int(os.environ.get("B", 65536)), 1024
 K = torch.randn(B, M, dtype=torch.float64, device="cuda")
 C = torch.randn(M, M, dtype=torch.float64, device="cuda")
