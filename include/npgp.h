@@ -381,6 +381,62 @@ int npgp_svgp_sample_prepare(npgp_svgp_plan* plan, const double* theta, int S, u
                              long work_bytes, npgp_stream_t stream);
 int npgp_svgp_sample(npgp_svgp_plan* plan, long n, const double* xs, long row_offset, const double* theta, int noise,
                      double* out, long ldo, void* work, long work_bytes, npgp_stream_t stream);
+/* Posterior of weighted regional sums t_r = sum_{i in r} w_i f_i (basin totals, area means, block averages), exact under q(u),
+ * with the factors of the last predict_prepare.  With k_i = K(x_i, Z) (scaled by s as the plan scales it), kappa the unscaled
+ * Gibbs kernel (kappa(x, x) = 1) and C = P^T (Ls Ls^T - I) P:
+ *   Cov(f_i, f_j) = s kappa(x_i, x_j) + delta_ij jitter_xx + k_i^T C k_j        (var_f on the diagonal, before its clamp)
+ *   mean_R[r]    = Y[:, r]^T u,   Y (M x R), Y[:, r] = sum_{i in r} w_i k_i
+ *   cov_R[r, r'] = s G[r, r'] + delta_rr' (jitter_xx [+ noise]) sum_{i in r} w_i^2 + (Y^T C Y)[r, r']
+ *   G[r, r']     = sum_{i in r} sum_{j in r'} w_i w_j kappa(x_i, x_j)
+ * Rows xs (n, d) are sorted by region: region r is rows [seg[r], seg[r+1]) (seg: R + 1 device offsets, non-decreasing from 0 to
+ * n); w (n) optional (NULL = ones).  Every row belongs to exactly one region: nested basins may repeat rows in xs, but then
+ * jitter_xx is counted only for identical indices, not for repeated points.
+ * Pair sums (the new hot path, csrc/gibbs_segsum.cu): G is never formed as an n x n matrix.  Only pairs i < j are evaluated (a
+ * same-row pair contributes exactly w_i^2), so the variances cost sum_r n_r^2 / 2 pairs and the full R x R matrix n^2 / 2.
+ *   npgp_gibbs_diag_segsum: x (n, D), ell (D, n) dim-major, D = 1..6;  npgp_gibbs_full_segsum: x (n, d), S (n, P) packed, d = 2, 3,
+ *   jitter as npgp_gibbs_full_fwd.  kappa is bitwise the entry npgp_gibbs_*_fwd(x, x) computes with scale NULL.
+ *   Gdiag[r] = scale * G[r, r] always (scale: device scalar, NULL = 1); G (R x R, leading dimension ldg >= R) only with full,
+ *   which evaluates r <= r' and mirrors.  Items (pairs of 256-row tiles) each write one partial to work, a finishing kernel adds
+ *   every entry's partials in a fixed order: bitwise reproducible for fixed (n, seg, part, nparts), and with full = 0 Gdiag is
+ *   bitwise that of full = 1 (nparts = 1).  part / nparts (0 <= part < nparts) split the item list: each part OVERWRITES the
+ *   outputs with its share, and the sum over parts (one all-reduce of R + R^2 doubles) is the single-part result up to the order
+ *   of that sum.  seg is validated on the device: a seg that is not non-decreasing from 0 to n gives NaN outputs, return 0.
+ *   workspace_bytes: size of `work` (256-byte aligned) for any valid seg of n rows and R regions, -1 for n < 0, n >= 2^31 or
+ *   R < 1.  Errors before any launch: NPGP_EINVAL for R < 1, n < 0, n >= 2^31, D / d out of range, NULL operands, part outside
+ *   [0, nparts), full with ldg < R; NPGP_EUNSUPPORTED for a misaligned work; NPGP_EWORKSPACE for a small one.
+ * Segmented column sums (the Y of one chunk, csrc/gibbs_segsum.cu): K (n x M, ldk >= M) holds the rows row0 .. row0 + n - 1 of
+ *   the sorted set:  out[r * ldo + j] += sum_{i in r, row0 <= i < row0 + n} w_i K[i - row0, j]  (w: the chunk's n weights, NULL =
+ *   ones).  Each (region, column) has one owner per launch, which adds its rows in index order (in 256-row slices, the slices
+ *   in order): deterministic, and chunks add in stream order.  work: npgp_segment_colwsum_workspace_bytes(n, M) bytes, 8-byte
+ *   aligned.  seg is not validated here (a bad one gives wrong sums, never an access outside K, w, seg or out's R rows).
+ * Plan call (csrc/svgp_step.cu): rows streamed through the plan in chunks of B_local: the row field (kept in work: the pair sums
+ *   need every row), K(x, Z) in FP64 into the plan's T buffer (neither predict nor sample uses it) and the chunk's Y columns;
+ *   then mean_R = Y^T u, C Y and Y^T C Y with npgp_dgemm (only the diagonal, by a row-dot kernel, without cov_R), the pair sums
+ *   with scale = s, and (jitter_xx [+ noise]) sum w_i^2 with noise = 1e-4 + softplus(raw_noise).  var_R (R) required; cov_R
+ *   (R x R, leading dimension ldc >= R) optional: NULL costs the variances' pairs only.  With both, var_R is bitwise
+ *   diag(cov_R), and cov_R is symmetric bitwise.  The marginals' clamp max(var, min_var) has no joint counterpart: a one-row
+ *   region with w = 1 reproduces var_f wherever that clamp is inactive.  part / nparts go to the pair sums; the mean, low-rank
+ *   and jitter / noise terms come from part 0 only (other parts write mean 0), so one all-reduce of the outputs gives the
+ *   single-call answer.  State rules as npgp_svgp_sample: NPGP_EINVAL unless npgp_svgp_predict_prepare ran since the last
+ *   fwd / step / set_extra_jitter; invalidates the saved forward; leaves P, C, u and their planes intact, so predict and
+ *   sample give bitwise the same results after it.  One stream, no allocation, capturable.  Bitwise reproducible for a fixed
+ *   plan, n, seg, part and nparts, except that from M = 512 on with few regions npgp_dgemm splits the low-rank products over
+ *   K with FP64 atomics (as the prepares do).
+ *   region_workspace_bytes: size of `work` (256-byte aligned), -1 on a bad cfg, n < 0, n >= 2^31 or R < 1; full: with cov_R. */
+long npgp_segsum_workspace_bytes(long n, int R, int full);
+int npgp_gibbs_diag_segsum(int D, long n, const double* x, const double* ell, const double* w, int R, const long* seg, int full,
+                           int part, int nparts, const double* scale, double* Gdiag, double* G, long ldg, void* work,
+                           long work_bytes, npgp_stream_t stream);
+int npgp_gibbs_full_segsum(int d, long n, const double* x, const double* S, double jitter, const double* w, int R,
+                           const long* seg, int full, int part, int nparts, const double* scale, double* Gdiag, double* G,
+                           long ldg, void* work, long work_bytes, npgp_stream_t stream);
+long npgp_segment_colwsum_workspace_bytes(int n, int M);
+int npgp_segment_colwsum(int n, int M, const double* K, long ldk, const double* w, long row0, int R, const long* seg,
+                         double* out, long ldo, void* work, long work_bytes, npgp_stream_t stream);
+long npgp_svgp_region_workspace_bytes(const npgp_svgp_config* cfg, long n, int R, int full);
+int npgp_svgp_region_moments(npgp_svgp_plan* plan, long n, const double* xs, const double* w, int R, const long* seg,
+                             const double* theta, int noise, int part, int nparts, double* mean_R, double* var_R,
+                             double* cov_R, long ldc, void* work, long work_bytes, npgp_stream_t stream);
 /* device pointers into the workspace (inspection): 0 mu (B), 1 T (B,M), 2 P (M,M), 3 C (M,M), 4 u (M), 5 g_mu (B), 6 g_v (B),
  * 7 acc4, 8 info (ints: Kzz, then the prior-kernel factorisations) */
 const void* npgp_svgp_buffer(npgp_svgp_plan* plan, int which);

@@ -106,6 +106,13 @@ _SIGS = {
     "npgp_svgp_sample_prepare": ([_p, _p, _i, C.c_ulonglong, _p, _l, _p], _i),
     "npgp_svgp_sample": ([_p, _l, _p, _l, _p, _i, _p, _l, _p, _l, _p], _i),
     "npgp_sample_normals": ([_i, _i, _i, C.c_ulonglong, _p, _p], _i),
+    "npgp_segsum_workspace_bytes": ([_l, _i, _i], _l),
+    "npgp_gibbs_diag_segsum": ([_i, _l, _p, _p, _p, _i, _p, _i, _i, _i, _p, _p, _p, _l, _p, _l, _p], _i),
+    "npgp_gibbs_full_segsum": ([_i, _l, _p, _p, _d, _p, _i, _p, _i, _i, _i, _p, _p, _p, _l, _p, _l, _p], _i),
+    "npgp_segment_colwsum_workspace_bytes": ([_i, _i], _l),
+    "npgp_segment_colwsum": ([_i, _i, _p, _l, _p, _l, _i, _p, _p, _l, _p, _l, _p], _i),
+    "npgp_svgp_region_workspace_bytes": ([_p, _l, _i, _i], _l),
+    "npgp_svgp_region_moments": ([_p, _l, _p, _p, _i, _p, _p, _i, _i, _i, _p, _p, _p, _l, _p, _l, _p], _i),
     "npgp_svgp_buffer": ([_p, _i], _p),
     "npgp_sgpr_predict_workspace_bytes": ([_i], _l),
     "npgp_sgpr_predict_finish": ([_i, _p, _l, _i, _i, _p, _l, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _l, _p], _i),

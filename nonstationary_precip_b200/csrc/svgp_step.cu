@@ -25,6 +25,7 @@
 #include "common.cuh"
 #include "philox.cuh"
 #include "sample.cuh"
+#include "segsum.cuh"
 #include "svgp_glue.cuh"
 #include "../../include/npgp.h"
 
@@ -304,6 +305,49 @@ __global__ void __launch_bounds__(256) svgp_sample_finish_kernel(int n, int S, c
     ssd[tx] = sqrt(r);
   }
   sample_store_rows(n, S, F, ldf, seed, row0, out, ldo, tile, smean, ssd);
+}
+
+// Regional moments, after the row pass and the pair sums (scal = [s, noise, ...]).  One thread per region r:
+//   lead (part 0): mean[r] = mt[r]; the diagonal gets (jitter_xx [+ noise]) sum_{i in r} w_i^2 on top of s G (+ the low-rank
+//   term: in cov already, else qd[r]); var[r] = that diagonal.  Other parts: mean 0, var = their share of s G.
+//   A bad seg (flag of the pair sums) makes every output NaN.  w2: sum w_i^2 per region, NULL = unit weights (n_r).
+__global__ void __launch_bounds__(256) svgp_region_finish_kernel(int R, const int* __restrict__ bad, int lead,
+                                                                 const double* __restrict__ mt, const double* __restrict__ qd,
+                                                                 const double* __restrict__ w2, const long* __restrict__ seg,
+                                                                 const double* __restrict__ scal, double jitter_xx, int noise,
+                                                                 double* __restrict__ mean, double* __restrict__ var,
+                                                                 double* __restrict__ cov, long ldc) {
+  const int r = blockIdx.x * 256 + threadIdx.x;
+  if (r >= R) return;
+  if (*bad) {
+    const double nan = __longlong_as_double(0x7ff8000000000000LL);
+    mean[r] = nan;
+    var[r] = nan;
+    if (cov)
+      for (int c = 0; c < R; ++c) cov[(long)r * ldc + c] = nan;
+    return;
+  }
+  double v = cov ? cov[(long)r * ldc + r] : var[r];
+  if (lead) {
+    const double jit = noise ? jitter_xx + scal[1] : jitter_xx;
+    const double sw2 = w2 ? w2[r] : (double)(seg[r + 1] - seg[r]);
+    if (!cov) v += qd[r];
+    v = fma(jit, sw2, v);
+    if (cov) cov[(long)r * ldc + r] = v;
+  }
+  mean[r] = lead ? mt[r] : 0.0;
+  var[r] = v;
+}
+
+// qd[r] = sum_j A[r, j] B[r, j]: one warp per row, fixed order (the diagonal of Y^T C Y without the R x R product)
+__global__ void __launch_bounds__(256) svgp_rowdot_kernel(int R, int M, const double* __restrict__ A, const double* __restrict__ B,
+                                                          double* __restrict__ out) {
+  const int r = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (r >= R) return;
+  double a = 0.0;
+  for (int j = lane; j < M; j += 32) a = fma(A[(long)r * M + j], B[(long)r * M + j], a);
+  a = warp_sum(a);
+  if (lane == 0) out[r] = a;
 }
 }  // namespace npgp
 
@@ -1079,4 +1123,98 @@ extern "C" const void* npgp_svgp_buffer(npgp_svgp_plan* p, int which) {
     case 8: return p->info;
     default: return nullptr;
   }
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// posterior moments of weighted regional sums t_r = sum_{i in r} w_i f_i (rows sorted by region, r = [seg[r], seg[r+1])):
+//     mean_R = Y^T u,  cov_R = s G + diag((jitter_xx [+ noise]) sum_{i in r} w_i^2) + Y^T C Y,   Y[:, r] = sum_{i in r} w_i k_i
+// G = the pair sums of the unscaled Gibbs kernel (csrc/gibbs_segsum.cu).  Everything beyond the plan lives in `work`: the
+// field at all n rows, Y^T and (C Y)^T (R x M each), three R-vectors, the column-sum slices and the pair-sum workspace.
+// ---------------------------------------------------------------------------------------------------------------------
+struct RegionBufs {
+  double *field, *Yt, *CYt, *mt, *qd, *w2, *colw;
+  void* seg;
+  long colw_bytes, seg_bytes;
+};
+
+static long region_layout(const npgp_svgp_plan& p, long n, int R, int full, void* work, RegionBufs* b) {
+  const int M = p.c.M;
+  Carver w{static_cast<char*>(work), 0};
+  b->field = w.take<double>(n * p.P6);
+  b->Yt = w.take<double>((long)R * M), b->CYt = w.take<double>((long)R * M);
+  b->mt = w.take<double>(R), b->qd = w.take<double>(R), b->w2 = w.take<double>(R);
+  b->colw_bytes = npgp_segment_colwsum_workspace_bytes(p.c.B_local, M);
+  b->colw = w.take<double>(b->colw_bytes / 8);
+  b->seg_bytes = npgp_segsum_workspace_bytes(n, R, full);
+  b->seg = w.take<char>(b->seg_bytes);
+  return w.off + 256;
+}
+
+extern "C" long npgp_svgp_region_workspace_bytes(const npgp_svgp_config* cfg, long n, int R, int full) {
+  if (!cfg || n < 0 || n >= (1L << 31) || R < 1) return -1;
+  npgp_svgp_plan tmp;
+  tmp.c = *cfg;
+  long bytes;
+  if (svgp_layout(&tmp, nullptr, &bytes)) return -1;
+  RegionBufs b;
+  return region_layout(tmp, n, R, full != 0, nullptr, &b);
+}
+
+/* Posterior mean and variance (optionally covariance) of R weighted regional sums, with the factors of the last prepare. */
+extern "C" int npgp_svgp_region_moments(npgp_svgp_plan* p, long n, const double* xs, const double* w, int R, const long* seg,
+                                        const double* theta, int noise, int part, int nparts, double* mean_R, double* var_R,
+                                        double* cov_R, long ldc, void* work, long work_bytes, cudaStream_t st) {
+  if (!p || !p->prepared || n < 0 || n >= (1L << 31) || R < 1 || nparts < 1 || part < 0 || part >= nparts) return NPGP_EINVAL;
+  if (!seg || !theta || !mean_R || !var_R || !work || (cov_R && ldc < R) || (n > 0 && !xs)) return NPGP_EINVAL;
+  if (reinterpret_cast<uintptr_t>(work) & 255) return NPGP_EUNSUPPORTED;
+  const int full = cov_R != nullptr;
+  RegionBufs b;
+  if (work_bytes < region_layout(*p, n, R, full, work, &b)) return NPGP_EWORKSPACE;
+  const npgp_svgp_config& c = p->c;
+  const int M = c.M, d = c.d, B = c.B_local, lead = part == 0;
+  const double* Z = theta + p->off_Z;
+  p->fwd_done = false;  // the row field and T are overwritten
+  // ---- row pass: the field at every row (the pair sums need all of them), K(x, Z) in FP64 into T, Y^T += segment sums
+  NPGP_CUDA(cudaMemsetAsync(b.Yt, 0, sizeof(double) * R * M, st));
+  NPGP_CUDA(cudaMemsetAsync(b.w2, 0, sizeof(double) * R, st));
+  for (long lo = 0; lo < n; lo += B) {
+    const int nc = (int)(n - lo < B ? n - lo : B);
+    const double* x = xs + lo * d;
+    NPGP_TRY(svgp_row_field(p, nc, x, theta, st));
+    if (c.variant == 1)
+      NPGP_CUDA(cudaMemcpyAsync(b.field + lo * p->P6, p->fx, sizeof(double) * nc * p->P6, cudaMemcpyDeviceToDevice, st));
+    else  // (d, nc) chunk -> columns [lo, lo + nc) of the (d, n) field
+      NPGP_CUDA(cudaMemcpy2DAsync(b.field + lo, sizeof(double) * n, p->ell_x, sizeof(double) * nc, sizeof(double) * nc, d,
+                                  cudaMemcpyDeviceToDevice, st));
+    if (!lead) continue;  // other parts add the pair sums only
+    if (c.variant == 1)
+      NPGP_TRY(npgp_gibbs_full_fwd(d, nc, M, x, p->fx, Z, p->fz, c.kernel_jitter, p->scal, p->T, M, nullptr, nullptr, st));
+    else
+      NPGP_TRY(npgp_gibbs_diag_fwd(d, nc, M, x, p->ell_x, Z, p->fz, p->scal, p->T, M, nullptr, nullptr, st));
+    NPGP_TRY(npgp_segment_colwsum(nc, M, p->T, M, w ? w + lo : nullptr, lo, R, seg, b.Yt, M, b.colw, b.colw_bytes, st));
+    if (w) NPGP_TRY(npgp_segment_colwsum(nc, 1, w + lo, 1, w + lo, lo, R, seg, b.w2, 1, b.colw, b.colw_bytes, st));
+  }
+  // ---- pair sums: s G into var_R (diagonal) and cov_R
+  if (c.variant == 1)
+    NPGP_TRY(npgp_gibbs_full_segsum(d, n, xs, b.field, c.kernel_jitter, w, R, seg, full, part, nparts, p->scal, var_R, cov_R, ldc,
+                                    b.seg, b.seg_bytes, st));
+  else
+    NPGP_TRY(npgp_gibbs_diag_segsum(d, n, xs, b.field, w, R, seg, full, part, nparts, p->scal, var_R, cov_R, ldc, b.seg,
+                                    b.seg_bytes, st));
+  // ---- part 0: the mean Y^T u and the low-rank term Y^T C Y (C symmetric: (C Y)^T = Y^T C)
+  if (lead) {
+    NPGP_TRY(npgp_gemv_n(R, M, b.Yt, M, p->u, b.mt, st));
+    NPGP_TRY(npgp_dgemm(0, 0, R, M, M, 1.0, b.Yt, M, p->C, M, 0.0, b.CYt, M, 0, 0, 0, st));
+    if (full) {  // lower tiles added onto s G, then mirrored: cov_R stays symmetric bitwise
+      NPGP_TRY(npgp_dgemm(0, 1, R, R, M, 1.0, b.CYt, M, b.Yt, M, 1.0, cov_R, ldc, 0, 0, 1, st));
+      NPGP_TRY(npgp_symmetrize(R, cov_R, ldc, 0, st));
+    } else {
+      svgp_rowdot_kernel<<<ceil_div(R, 8), 256, 0, st>>>(R, M, b.CYt, b.Yt, b.qd);
+      NPGP_LAUNCH_CHECK();
+    }
+  }
+  svgp_region_finish_kernel<<<ceil_div(R, 256), 256, 0, st>>>(R, segsum_bad_flag(b.seg), lead, b.mt, b.qd, w ? b.w2 : nullptr,
+                                                                seg, p->scal, c.jitter_xx, noise, mean_R, var_R, cov_R, ldc);
+  NPGP_LAUNCH_CHECK();
+  return NPGP_OK;
 }

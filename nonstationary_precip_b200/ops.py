@@ -487,6 +487,57 @@ def colwsum(K, w=None, out=None):
     return out
 
 
+def _segsum_work(n, R, full, device):
+    nbytes = lib().npgp_segsum_workspace_bytes(n, R, int(full))
+    if nbytes < 0:
+        raise ValueError("no pair-sum workspace for n = %d rows, R = %d regions" % (n, R))
+    work = torch.empty(nbytes + 256, dtype=torch.uint8, device=device)
+    return work, work.data_ptr() + (-work.data_ptr()) % 256, nbytes
+
+
+def gibbs_diag_segsum(x, ell, seg, w=None, full=False, part=0, nparts=1, scale=None):
+    """Pair sums G[r, r'] = scale * sum_{i in r, j in r'} w_i w_j kappa(x_i, x_j) of the diagonal Gibbs kernel over the regions
+    rows [seg[r], seg[r+1]) (int64, R + 1 offsets).  x (n,D), ell (D,n).  Returns (Gdiag (R), G (R,R) or None)."""
+    x, ell, w, scale, seg = map(_c, (x, ell, w, scale, seg))
+    n, D = x.shape
+    R = seg.numel() - 1
+    f64 = dict(dtype=torch.float64, device=x.device)
+    Gdiag = torch.empty(R, **f64)
+    G = torch.empty(R, R, **f64) if full else None
+    _, wp, nbytes = work = _segsum_work(n, R, full, x.device)
+    check(lib().npgp_gibbs_diag_segsum(D, n, ptr(x), ptr(ell), ptr(w), R, ptr(seg), int(full), part, nparts, ptr(scale),
+                                       ptr(Gdiag), ptr(G), R, wp, nbytes, stream()), "npgp_gibbs_diag_segsum")
+    return Gdiag, G
+
+
+def gibbs_full_segsum(x, S1p, seg, w=None, jitter=1e-5, full=False, part=0, nparts=1, scale=None):
+    """The same for the full-matrix Gibbs kernel: S1p (n, d(d+1)/2) packed, jitter as gibbs_full_fwd."""
+    x, S1p, w, scale, seg = map(_c, (x, S1p, w, scale, seg))
+    n, d = x.shape
+    R = seg.numel() - 1
+    f64 = dict(dtype=torch.float64, device=x.device)
+    Gdiag = torch.empty(R, **f64)
+    G = torch.empty(R, R, **f64) if full else None
+    _, wp, nbytes = work = _segsum_work(n, R, full, x.device)
+    check(lib().npgp_gibbs_full_segsum(d, n, ptr(x), ptr(S1p), float(jitter), ptr(w), R, ptr(seg), int(full), part, nparts,
+                                       ptr(scale), ptr(Gdiag), ptr(G), R, wp, nbytes, stream()), "npgp_gibbs_full_segsum")
+    return Gdiag, G
+
+
+def segment_colwsum(K, seg, w=None, row0=0, out=None):
+    """out[r, j] (+)= sum_{i in r} w_i K[i - row0, j] for the rows row0 .. row0 + n - 1 of the sorted set (seg: R + 1 offsets)."""
+    n, M = K.shape
+    seg, w = _c(seg), _c(w)
+    R = seg.numel() - 1
+    if out is None:
+        out = torch.zeros(R, M, dtype=torch.float64, device=K.device)
+    nbytes = lib().npgp_segment_colwsum_workspace_bytes(n, M)
+    work = torch.empty(max(nbytes, 8) // 8, dtype=torch.float64, device=K.device)
+    check(lib().npgp_segment_colwsum(n, M, ptr(K), K.stride(0), ptr(w), row0, R, ptr(seg), ptr(out), out.stride(0), ptr(work),
+                                     nbytes, stream()), "npgp_segment_colwsum")
+    return out
+
+
 def gemv_n(A, v, out=None):
     """A @ v (one warp per row)."""
     n, M = A.shape

@@ -48,6 +48,23 @@ class Predictive(NamedTuple):
     sums: Optional[torch.Tensor]
 
 
+class RegionPosterior(NamedTuple):
+    """Posterior of weighted regional sums t_r = sum_{i in r} w_i f_i from SVGPGibbs.region_posterior: mean (R), var (R) and,
+    with cov=True, the covariance (R, R) (var is then its diagonal, bitwise).  Area means: w_i = area_i / sum_{j in r} area_j."""
+    mean: torch.Tensor
+    var: torch.Tensor
+    cov: Optional[torch.Tensor]
+
+
+def region_segments(labels: torch.Tensor, num_regions: int):
+    """Rows sorted by region: (order, seg) with labels[order] non-decreasing (stable, on the tensor's device, no host sync) and
+    seg (num_regions + 1, int64) the offsets of the regions in that order, region r = rows [seg[r], seg[r+1]).  Labels outside
+    [0, num_regions) leave seg[0] != 0 or seg[-1] != n, which the C call turns into NaN outputs."""
+    srt, order = torch.sort(labels.reshape(-1), stable=True)
+    bounds = torch.arange(num_regions + 1, dtype=srt.dtype, device=srt.device)
+    return order, torch.searchsorted(srt, bounds).to(torch.int64)
+
+
 class _Section:
     """Bracket around a named part of the step.  model.profile (a dict): CUDA-event pairs (eager runs only).
     model.timeline (an int64 device buffer): GPU-timer stamps written by tiny kernels, which ARE capturable, so the real
@@ -828,3 +845,37 @@ class SVGPGibbs:
         check(lib().npgp_svgp_sample(ent["handle"], n, ptr(xs), int(row_offset), ptr(self.theta), int(bool(noise)), ptr(out),
                                      n, wp, nbytes, stream()), "npgp_svgp_sample")
         return out
+
+    @torch.no_grad()
+    def region_posterior(self, xs, labels, num_regions: int, weights=None, *, noise: bool = False, cov: bool = True,
+                         part: int = 0, nparts: int = 1, chunk: int = 65536) -> RegionPosterior:
+        """Exact posterior mean and variance (cov=True: covariance) of t_r = sum_{i: labels_i = r} w_i f_i (noise=True: of y)
+        for r < num_regions, through npgp_svgp_predict_prepare + npgp_svgp_region_moments on the plan of predictive().  The
+        rows are sorted by label on the device (stable) and the offsets found by searchsorted, so nothing waits for the GPU;
+        labels outside [0, num_regions) give NaN.  weights: (n) or None (ones); an area mean takes w_i = area_i / sum of the
+        areas of its region.  part / nparts: this caller's share of the pair sums (part 0 also adds the mean, the low-rank and
+        the jitter / noise terms), so summing the outputs of all parts gives the single-call answer.  The variances alone cost
+        sum_r n_r^2 / 2 kernel pairs, the covariance n^2 / 2.  Needs M % 128 == 0 (the plan's path)."""
+        if self.M % 128:
+            raise ValueError("the C region moments need M % 128 == 0 (got %d)" % self.M)
+        from ._lib import check, lib, ptr, stream
+        import ctypes as C
+        ent = self._plan(chunk, 1, chunk)
+        n, R = xs.shape[0], int(num_regions)
+        order, seg = region_segments(labels, R)
+        xs_s = xs[order].contiguous()
+        w_s = weights.reshape(-1)[order].contiguous() if weights is not None else None
+        nbytes = lib().npgp_svgp_region_workspace_bytes(C.byref(ent["cfg"]), n, R, int(bool(cov)))
+        if nbytes < 0:
+            raise ValueError("no region workspace for n = %d rows, R = %d regions" % (n, R))
+        work = torch.empty(nbytes + 256, dtype=torch.uint8, device=self.dev)
+        wp = work.data_ptr() + (-work.data_ptr()) % 256
+        f64 = dict(dtype=torch.float64, device=self.dev)
+        mean, var = torch.empty(R, **f64), torch.empty(R, **f64)
+        cv = torch.empty(R, R, **f64) if cov else None
+        check(lib().npgp_svgp_predict_prepare(ent["handle"], ptr(self.theta), ptr(self.status), stream()),
+              "npgp_svgp_predict_prepare")
+        check(lib().npgp_svgp_region_moments(ent["handle"], n, ptr(xs_s), ptr(w_s), R, ptr(seg), ptr(self.theta),
+                                             int(bool(noise)), int(part), int(nparts), ptr(mean), ptr(var), ptr(cv), R, wp,
+                                             nbytes, stream()), "npgp_svgp_region_moments")
+        return RegionPosterior(mean, var, cv)
