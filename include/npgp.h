@@ -203,7 +203,9 @@ int npgp_rbfper_bwd(int n1, int n2, const double* t1, const double* t2, const do
  * GPyTorch) and Phi = Kzx Kxz of the SGPR objective.  Every operand entry is the integer rint(x 2^(54-e)) written as 7
  * signed base-256 digits, e a power-of-two exponent per row or per matrix; the 28 digit products with p + q <= 6 are
  * accumulated exactly in int32 by tcgen05.mma kind::i8 (S8 x S8) and recombined in the epilogue.
- * Results equal the FP64 product to its own rounding bound and are bit-exact on integer-valued data.
+ * Results equal the FP64 product to its own rounding bound and are bit-exact on integer-valued data.  Exception: a row
+ * (or column) whose largest magnitude is below 2^-961 has its exponent clamped at -960, so its entries carry an absolute
+ * error of up to 2^-1015 rather than a relative one.
  *
  * General operands (contract of npgp_rowquad / npgp_wsyrk): C symmetric, M % 64 == 0 (SYRK: M % 128 == 0), M <= 16384,
  * T 16-byte aligned with even ldt.  work: the *_workspace_bytes(n, M) bytes of device memory (digit planes, exponents,

@@ -711,19 +711,19 @@ o8_syrk_kernel(int M, int nks_total, int spc, int slots_per_cta, const int8_t* _
   if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512));
 }
 
-// one entry of a row-layout digit matrix (A-type planes) as a double, without the power-of-two scale
-__device__ __forceinline__ double o8_entry(const int8_t* __restrict__ digits, int nks, int r, int k) {
+// the seven signed digits of one entry of a row-layout digit matrix (A-type planes)
+__device__ __forceinline__ void o8_entry_digits(const int8_t* __restrict__ digits, int nks, int r, int k, int (&d)[O8_NS]) {
   const int8_t* b = digits + o8_a_offset(r, k & ~15, nks) + (k & 15);
-  long long y = 0;
 #pragma unroll
-  for (int p = 0; p < O8_NS; ++p) y = y * 256 + (long long)b[(long)p * nks * O8_A_PLANE];  // seven signed digits
-  return (double)y;
+  for (int p = 0; p < O8_NS; ++p) d[p] = b[(long)p * nks * O8_A_PLANE];
 }
 
 // Out (symmetric) (+)= alpha * w0 * (sum of the tile's segment partials - sum_{i in skip} x_i x_i^T).  One CTA per upper
 // 128 x 64 tile; the segments of the tile are found by re-running the CTAs' segment iterators (a handful of integer steps)
 // and added in CTA / index order (bitwise reproducible).  skip (optional): rows whose weight is 0 instead of w0 (rows of the
 // SVGP step whose predictive variance was clamped: their gradient is zero), rebuilt from the digit planes; normally empty.
+// The correction is the same 28 digit products as the main path, summed exactly in 64-bit integers over the list and
+// recombined as o8_recombine does: it does not depend on the order of skip_rows (which the caller fills through atomics).
 __global__ void __launch_bounds__(256) o8_syrk_finish_kernel(int M, int nks_total, int spc, int n_cta, int slots_per_cta,
                                                              const double* __restrict__ part, double alpha,
                                                              const double* __restrict__ w0, const double* __restrict__ uniform_count,
@@ -786,13 +786,26 @@ __global__ void __launch_bounds__(256) o8_syrk_finish_kernel(int M, int nks_tota
     double s = acc[i];
     if (n_skip > 0) {
       const int ex = o8_exponent_of_scale(*x_scale);
-      const double sc2 = o8_pow2(2 * (ex - O8_FRAC));
-      double corr = 0.0;
+      long long g[O8_NS] = {0, 0, 0, 0, 0, 0, 0};  // |g_t| <= 7 * 2^14 per listed row
       for (int t = 0; t < n_skip; ++t) {
         const int ii = skip_rows[t];
-        corr = fma(o8_entry(digits, M / O8_KS, ii, r), o8_entry(digits, M / O8_KS, ii, c), corr);
+        int a[O8_NS], b[O8_NS];
+        o8_entry_digits(digits, M / O8_KS, ii, r, a);
+        o8_entry_digits(digits, M / O8_KS, ii, c, b);
+#pragma unroll
+        for (int p = 0; p < O8_NS; ++p)
+#pragma unroll
+          for (int q = 0; q < O8_NS - p; ++q) g[p + q] += a[p] * b[q];
       }
-      s -= corr * sc2;
+      // hi needs more than 64 bits for lists longer than 2^22 rows
+      __int128 hi = g[0];
+      long long lo = g[4];
+#pragma unroll
+      for (int t = 1; t < 4; ++t) hi = hi * 256 + g[t];
+#pragma unroll
+      for (int t = 5; t < O8_NS; ++t) lo = lo * 256 + g[t];
+      const double corr = fma((double)lo, 5.9604644775390625e-08 /* 2^-24 */, (double)hi);
+      s -= corr * o8_scale_or_nan(ex, -36) * o8_scale_or_nan(ex, 0);
     }
     s *= scale;
     if (accumulate) {

@@ -2,25 +2,17 @@
 digits, the row-quadratic product and the MN-major SYRK that consume them, the deterministic partial reductions.
 Checked against the FP64 tile kernels / FP64 products and, through them, the oracle (test_ops_gpu.py pins those)."""
 import math
+import os
+import sys
 
 import pytest
 import torch
 
+sys.path.insert(0, os.path.dirname(__file__))
+from oz8_ref import decode_planes, encode_a_planes, encode_b_planes  # noqa: E402
+
 pytestmark = pytest.mark.gpu
 torch.set_default_dtype(torch.float64)
-
-
-def decode_planes(digits, n, M):
-    """Inverse of the A-type row layout of csrc/oz8.cuh: int8 planes -> integer-valued double matrix (npad, M), without the
-    power-of-two scale.  Layout: [row block][digit][k-step][16-byte half][8-row group][row in group][16 bytes]."""
-    npad = (n + 127) // 128 * 128
-    nks = M // 32
-    d = digits[:npad * M * 7].view(torch.int8).view(npad // 128, 7, nks, 2, 16, 8, 16).to(torch.int64)
-    y = d[:, 0]
-    for p in range(1, 7):
-        y = y * 256 + d[:, p]  # seven signed digits
-    # y: [rb, ks, cj, m8, r8, k16] -> rows rb*128 + m8*8 + r8, cols ks*32 + cj*16 + k16
-    return y.permute(0, 3, 4, 1, 2, 5).reshape(npad, M).double()
 
 
 def gibbs_inputs(variant, n, M, d, seed):
@@ -188,22 +180,6 @@ def test_svgp_step_with_clamped_rows_matches_dmma_path(variant):
 
 
 # ---- digit-level diagnostics: hand-made planes, exact integer reference ----------------------------------------------
-def encode_a_planes(D):
-    """D: (7, npad, M) int8 digits -> uint8 buffer in the A-type row layout [rb][p][ks][cj][m8][r8][k16]."""
-    _, npad, M = D.shape
-    nks = M // 32
-    t = D.view(7, npad // 128, 16, 8, nks, 2, 16)      # [p, rb, m8, r8, ks, cj, k16]
-    return t.permute(1, 0, 4, 5, 2, 3, 6).contiguous().view(torch.uint8).reshape(-1)
-
-
-def encode_b_planes(D):
-    """D: (7, Mr, Kd) int8 digits of the B operand (row blocks of 64) -> [cb][ks][p][cj][m8][r8][k16]."""
-    _, Mr, Kd = D.shape
-    nks = Kd // 32
-    t = D.view(7, Mr // 64, 8, 8, nks, 2, 16)          # [p, cb, m8, r8, ks, cj, k16]
-    return t.permute(1, 4, 0, 5, 2, 3, 6).contiguous().view(torch.uint8).reshape(-1)
-
-
 @pytest.mark.parametrize("n,M", [(128, 64), (256, 128)])
 def test_every_digit_product_is_exact(n, M):
     """A carries only digit p, C only digit q: T must be exactly 2^(-12-8(p+q)) A_p C_q^T for the 28 kept products and 0 for
